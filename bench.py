@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the MERV fusion hot path (BASELINE.json metric: merv-full fusion videos/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A step = one pass of the whole path (pool -> projector -> score/softmax -> mix) over one batch of 64 synthetic
@@ -18,6 +18,10 @@ Sub-records of the same line (each with its own clock record):
                 compute-then-NCCL vs the GEMM whose epilogue stores every tile into all ranks' symmetric buffers
   configs       N = 1: configs[3] (SigLIP single encoder, B = 256) and configs[4] (generate: time-to-prefix, TTFT)
   kernels / roofline   per-kernel CUDA-event durations from an instrumented pass over the same K steps
+
+--dump-outputs DIR writes what the last timed step returned (rank 0): DIR/weights.npy, the mixing weights [batch, 4], and
+DIR/prefix_sample.npy, the prefix [batch, 1024, 4096] at DUMP_SAMPLE fixed, seeded flat positions (both float32).  Inputs and
+weights are seeded, so two builds run with the same arguments can be compared output for output.
 
 --impl reference times the reference's own CPU implementation of the path (the unmodified merv/util/nn_utils.py modules
 staged in oracle/_ref; oracle/torch_port.py where that file is absent) on the host cores, rank 0 only, without importing
@@ -52,6 +56,7 @@ BYTES_OUT = OUT_TOKENS * LLM_DIM * 2
 FLOPS_LINEAR = 2 * OUT_TOKENS * LLM_DIM * sum(DIMS)  # 30.065 GFLOP
 FLOPS_GELU = FLOPS_LINEAR + 4 * 2 * OUT_TOKENS * LLM_DIM * LLM_DIM  # 167.5 GFLOP
 GLOBAL_BATCH = 64  # BASELINE.json configs[2] / SURVEY.md §8d config 3
+DUMP_SAMPLE, DUMP_SEED = 1 << 22, 0  # --dump-outputs: 16 MB of float32 out of the 1 GB (as float32) prefix of 64 videos
 
 
 def ncu_traffic_bytes(*profile_txts: str):
@@ -160,6 +165,18 @@ def cpu_reference_run(mlp_type: str, sample_videos: int, steps: int, warmup: int
     return sample_videos * steps / dt, dt / steps * 1e3, cores, kind, what
 
 
+def dump_outputs(directory: str, out, w) -> None:
+    """The arrays a caller of the timed path receives, as float32 .npy: the mixing weights whole, the prefix at DUMP_SAMPLE flat
+    positions drawn from a generator seeded with DUMP_SEED (the same positions for every run of the same shape)."""
+    import numpy as np
+    import torch
+
+    os.makedirs(directory, exist_ok=True)
+    idx = torch.randint(0, out.numel(), (min(DUMP_SAMPLE, out.numel()),), generator=torch.Generator().manual_seed(DUMP_SEED))
+    np.save(os.path.join(directory, "prefix_sample.npy"), out.reshape(-1)[idx.to(out.device)].float().cpu().numpy())
+    np.save(os.path.join(directory, "weights.npy"), w.float().cpu().numpy())
+
+
 def workload_config(args, world: int, note: str = ""):
     return {
         "workload": f"merv-full fusion bf16 batch {args.batch} per GPU on {world}xB200 (3d-avg pool + {args.projector} projector + cross-attn mix)",
@@ -213,6 +230,8 @@ def main():
                     help="N = 1: also A/B the opt-in pooling inside the GEMM launch (MERV_POOL_ASSIST=1) in the sustained regime; off by default so "
                          "that the default run only ever executes the production path")
     ap.add_argument("--gather-timeout", type=float, default=240.0, help="watchdog (s) around the multi-GPU gather sub-records")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/*.npy (float32; a fixed, seeded sample of the prefix)")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", 0))
@@ -309,6 +328,8 @@ def main():
         with ops.KernelTimer(timing=False) as counter:  # counts the kernels launched inside the timed region (no events, no syncs)
             ms_step, clocks = timed(step, args.steps)
         launches = counter.launches
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, keep["out"], keep["w"])
         value = world * B * 1e3 / ms_step
         checksum = float(keep["out"].float().abs().mean().item())
 

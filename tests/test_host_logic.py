@@ -195,10 +195,7 @@ def test_first_and_token_concat_fusions():
         M.MervFusion(projs, None)
 
 
-# ---- patch_merv on the reference's own modules (only where the reference tree exists: this container) -------------
-REF_PRESENT = os.path.isfile("/root/reference/merv/util/nn_utils.py")
-
-
+# ---- patch_merv on the reference's own modules ---------------------------------------------------------------------
 class _FakeMerv(torch.nn.Module):
     """The attributes of the reference MERV that patch_merv touches (merv.py:152-223)."""
 
@@ -209,7 +206,6 @@ class _FakeMerv(torch.nn.Module):
         self.feature_fusion_type = fusion_type
 
 
-@pytest.mark.skipif(not REF_PRESENT, reason="reference tree not present on this box")
 @pytest.mark.parametrize("fusion_type", ["cross_attention_avg_lq", "concat_channel", "concat_channel_ln", "first", "concat"])
 def test_patch_merv_shares_parameters_and_reproduces_the_reference(fusion_type):
     import merv_b200 as M
@@ -296,7 +292,6 @@ def test_fused_training_gradients_match_reference_autograd():
     assert ff.attention.v_proj_weight.grad is None and ff.attention.out_proj.weight.grad is None
 
 
-@pytest.mark.skipif(not REF_PRESENT, reason="reference tree not present on this box")
 def test_attentive_pooler_init_sequence_and_adoption_match_the_reference():
     # same seed -> same initial parameters (module tree and init order mirror nn_utils.py:182-227); patch_merv adopts the reference module
     import merv_b200 as M
@@ -355,10 +350,8 @@ def test_attentive_pooler_backward_wiring_matches_reference_autograd(monkeypatch
     import copy
 
     import merv_b200 as M
-    from oracle.ref_loader import load_reference_nn_utils, reference_available
+    from oracle.ref_loader import load_reference_nn_utils
 
-    if not reference_available():
-        pytest.skip("needs the reference's nn_utils.py")
     kernel_emulation.emulate(monkeypatch)
     ref = load_reference_nn_utils()
     torch.manual_seed(11)
@@ -396,10 +389,8 @@ def test_conv3d_projector_backward_wiring_and_adoption_match_the_reference(monke
     import copy
 
     import merv_b200 as M
-    from oracle.ref_loader import load_reference_nn_utils, reference_available
+    from oracle.ref_loader import load_reference_nn_utils
 
-    if not reference_available():
-        pytest.skip("needs the reference's nn_utils.py")
     kernel_emulation.emulate(monkeypatch)
     ref = load_reference_nn_utils()
     torch.manual_seed(3)

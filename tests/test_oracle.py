@@ -166,6 +166,92 @@ def test_oracle_variants_match_reference_golden(name):
         assert np.abs(w - 1.0 / w.shape[1]).max() > 0.03, "degenerate (flat) softmax: the fixture would not catch a broken score path"
 
 
+def _restated_variant_module(v):
+    import torch
+
+    from oracle import reference_nn as R
+
+    kind = v["kind"]
+    if kind == "projector":
+        cls = {"LinearProjector": R.LinearProjector}.get(v["cls"])
+        if cls is not None:
+            return cls(v["vision_dim"], v["llm_dim"], pre_proj_layernorm=True)
+        return getattr(R, v["cls"])(v["vision_dim"], v["llm_dim"], "gelu-mlp" if v["cls"] != "FusedMLPProjector" else "fused-gelu-mlp",
+                                    pre_proj_layernorm=True)
+    if kind == "attntv":
+        return R.AttentivePooler(v["C"], v["llm_dim"], num_query_tokens=v["queries"], num_heads=v["heads"], output_frames=v["F"], mlp_type=v["mlp_type"])
+    if kind == "conv3d":
+        return R.Convolutional3DProjector(v["C"], v["llm_dim"], output_frames=v["T"], output_size=v["S"], mlp_type=v["mlp_type"])
+    if kind == "concat_channel_ln":  # merv.py:219-223
+        return torch.nn.Sequential(torch.nn.LayerNorm(v["E"] * v["K"]), R.LinearProjector(v["E"] * v["K"], v["K"]))
+    return R.CrossAttentionAdapterLearnableQuery(embed_dim=v["embed"], llm_dim=v["K"], token_length=v["T"], averagetoken=v["averagetoken"],
+                                                 num_encoder=v["E"], positional_embedding=v["pe"])
+
+
+@pytest.mark.parametrize("name", _variant_names())
+def test_reference_restatement_matches_reference_golden(name):
+    """oracle/reference_nn.py (what the module-level tests use as the reference modules) reproduces the outputs the UNMODIFIED
+    reference modules produced on the same seeded inputs and weights, every variant through its own state-dict keys."""
+    import torch
+
+    from tests.golden_util import load_variant
+
+    v, inputs, params, gold = load_variant(name)
+    m = _restated_variant_module(v).eval()
+    m.load_state_dict({k: torch.from_numpy(np.ascontiguousarray(a)) for k, a in params.items()})
+    xs = [torch.from_numpy(np.ascontiguousarray(x)) for x in inputs]
+    with torch.no_grad():
+        if v["kind"] in ("projector", "attntv", "conv3d"):
+            out, w = m(xs[0]), None
+        elif v["kind"] == "concat_channel_ln":  # merv.py:603-606
+            out, w = m(torch.concat(xs, -1)), None
+        else:
+            out, w = m(xs)
+    assert tuple(out.shape) == gold["out"].shape
+    assert O.rel_err(out.numpy(), gold["out"]) < FP32_TOL
+    if w is not None:
+        assert np.abs(w.numpy() - gold["weights"]).max() < 2e-5
+
+
+@pytest.mark.parametrize("name", list(C.CASES))
+def test_reference_restatement_matches_reference_golden_cases(name):
+    """The same for the whole fusion path of every Case (pooling resamplers + the case's mixer), against the stored samples."""
+    import torch
+
+    from oracle import reference_nn as R
+
+    case = C.CASES[name]
+    g, feats, pp, fp = regenerate(case)
+    tt = lambda d: {k: torch.from_numpy(np.ascontiguousarray(a)) for k, a in d.items()}  # noqa: E731
+    ys = []
+    for x, p, c, t in zip(feats, pp, case.dims, case.out_frames):
+        P = R.AveragePoolingProjector if case.resampler == "avg" else R.AveragePooling3DProjector
+        proj = P(c, case.llm_dim, output_frames=t, output_size=case.out_size, mlp_type=case.mlp_type)
+        proj.projector.load_state_dict(tt(p))
+        with torch.no_grad():
+            ys.append(proj(torch.from_numpy(x)))
+    if case.fusion == "scalar":
+        ff = R.ScalarAdapter(case.num_encoders)
+    elif case.fusion == "concat_channel":
+        ff = R.LinearProjector(case.num_encoders * case.llm_dim, case.llm_dim)
+    else:
+        ff = R.CrossAttentionAdapterLearnableQuery(embed_dim=case.embed_dim, llm_dim=case.llm_dim, token_length=case.token_length, averagetoken=True,
+                                                   num_encoder=case.num_encoders)
+    ff.load_state_dict(tt(fp))
+    with torch.no_grad():
+        if case.fusion == "concat_channel":
+            out, w = ff(torch.concat(ys, -1)), None
+        else:
+            out, w = ff(ys)
+    idx = g["sample_idx"]
+    assert np.abs(out.numpy().reshape(-1)[idx] - g["out_samples"]).max() / float(g["out_abs_max"]) < FP32_TOL
+    for e, y in enumerate(ys):
+        ref = g["y_samples"][e]
+        assert np.abs(y.numpy().reshape(-1)[idx % y.numel()] - ref).max() / max(np.abs(ref).max(), 1e-6) < FP32_TOL
+    if w is not None:
+        assert np.abs(w.numpy() - g["weights"]).max() < 2e-5
+
+
 def test_variant_fixtures_are_sensitive_to_the_variant():
     # the positional embedding / the flattened key / the LayerNorm must move the reference's output well beyond the parity tolerance
     from tests.golden_util import load_variant
@@ -192,12 +278,7 @@ def test_reference_arm_port_weights_equal_the_reference_modules():
     import torch
 
     from oracle import reference_model as RM
-    from oracle.ref_loader import reference_available
 
-    if not reference_available():
-        import pytest
-
-        pytest.skip("needs the reference's nn_utils.py")
     dims, llm, frames, S = [64, 48], 96, [4, 4], 2
     for mlp_type in ("linear", "gelu-mlp"):
         fwd_ref, (projs, ff) = RM.build_reference(dims, llm, frames, S, mlp_type, 16, q_scale=8.0)
