@@ -294,6 +294,23 @@ int merv_mix_backward(const void* const* V, const void* dOut, const float* weigh
                       const float* u, const void* Q, const void* Wq, const void* Wk, const void* in_proj_bias,
                       void* const* dV, void* dQ, void* dWq, void* dWk, void* dbias, float* workspace,
                       size_t workspace_floats, int B, int E, int T, int K, int embed, int dtype, void* stream);
+/* merv_mix_backward for every configuration the forward (merv_scores_from_tokens_ex + merv_softmax_mix) supports; with
+ * ds = softmax backward of (dw + dweights_out) as above:
+ *   tokens[e] in {T, 1}: a single-token encoder (repeated to T tokens, nn_utils.py:502) gets dV_e [B, 1, K] = the sum over t of
+ *       the T-token gradient rows, i.e. w_e sum_t dOut[b,t] + ds_e ubar, and dw_e = <sum_t dOut[b,t], V_e[b,0]>;
+ *   u_token_stride == 0 (averagetoken=True, u [K]):   dV_e = w_e dOut + (ds_e / T) u,  du = sum_{b,e} ds_e (mean_t V_e + pe[e]), ubar = u;
+ *       pe [E, K] (ldpe, `dtype`) or NULL: positional_embedding=True (nn_utils.py:510-511); then dpe[e] = (sum_b ds_e[b]) u, dpe [E, K];
+ *   u_token_stride == K (averagetoken=False, nn_utils.py:514-518, u [T*K]): dV_e = w_e dOut[b,t] + ds_e u[t],
+ *       du[t] = sum_{b,e} ds_e V_e[b,t] (length T*K, Wk / dWk are [embed, T*K]), ubar = sum_t u[t]; pe must be NULL.
+ * Then dq, dWk, dWq, db_q, dQ from du as in merv_mix_backward.  Fixed-order reductions (bit-reproducible).  With every tokens[e] == T,
+ * u_token_stride == 0 and pe == NULL it is merv_mix_backward (same kernels, bit-identical).  workspace: merv_mix_backward_ex_workspace
+ * floats (B * K fewer suffice when every encoder has T tokens). */
+size_t merv_mix_backward_ex_workspace(int B, int E, int T, int K, int embed, int64_t u_token_stride);
+int merv_mix_backward_ex(const void* const* V, const int32_t* tokens, const void* dOut, const float* weights,
+                         const float* dweights_out, const float* u, int64_t u_token_stride, const void* pe, int64_t ldpe,
+                         const void* Q, const void* Wq, const void* Wk, const void* in_proj_bias, void* const* dV, void* dQ,
+                         void* dWq, void* dWk, void* dbias, void* dpe, float* workspace, size_t workspace_floats, int B, int E,
+                         int T, int K, int embed, int dtype, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * Backward of the FUSED path (linear projectors linked to the adapter, forward = merv_fused_linear_mix): the training step of

@@ -7,9 +7,16 @@
 //        dw_e   = <dOut, V_e>                     ds = softmax'(w) dw
 //        dV_e   = w_e dOut + (ds_e / T) u         du = sum_{b,e} ds_e mean_t V_e
 //        u = Wk^T q / sqrt(E), q = Wq Q^T + b_q:  dq = Wk du / sqrt(E), dWk = q du^T / sqrt(E), dWq = dq Q, db_q = dq, dQ = Wq^T dq
+//   the other configurations of the adapter (merv_mix_backward_ex), same ds:
+//     positional_embedding  w = softmax_e(u . (mean_t V_e + pe_e)):  dV_e as above,  du = sum_{b,e} ds_e (mean_t V_e + pe_e),
+//                           dpe_e = (sum_b ds_e) u                                        (du_pe_kernel; no extra pass over V)
+//     averagetoken=False    w = softmax_e(sum_t u_t . V_e[t]), u [T*K]:  dV_e[t] = w_e dOut[t] + ds_e u_t,
+//                           du_t = sum_{b,e} ds_e V_e[b,t]  (length T*K, in the dV pass: mix_bwd_dv_flat_kernel)
+//     single-token encoder  (repeated to T tokens) dV_e[b,0] = sum_t of the rows above = w_e gsum[b] + ds_e ubar,
+//                           gsum[b] = sum_t dOut[b,t], ubar = u or sum_t u_t;  dw_e = <gsum[b], V_e[b,0]>, mean_t V_e = V_e[b,0]
 //   v_proj_weight / out_proj / b_k / b_v receive no (zero) gradient, exactly as in the reference where the attention
 //   output is discarded and b_k cancels in the softmax.
-// All reductions are fixed-order (deterministic).
+// All reductions are fixed-order (deterministic, no atomics).
 #include "common.cuh"
 
 namespace merv {
@@ -71,21 +78,70 @@ __global__ void __launch_bounds__(256) colsum_final_kernel(const float* __restri
 struct BwdPtrs {
   const void* V[MERV_MAX_ENCODERS];
   void* dV[MERV_MAX_ENCODERS];
+  int tokens[MERV_MAX_ENCODERS];  // T or 1 (a single-token encoder, repeated to T tokens in the forward)
 };
 
 // grid (column blocks of 8 vectors = 128 bytes, E, B), 256 threads = 8 vectors x 32 token groups; a thread walks every 32nd token with four
 // independent pairs of 16-byte loads in flight, the 32 groups are then reduced through shared memory in a fixed order.  (The first version
 // gave one thread a whole column of T tokens: 256 CTAs x 2 loads in flight = 1.4 TB/s, 0.49 ms of the 2.2 ms training step at 16 videos.)
+// A single-token encoder reads dOut only: its column sums gsum[b,:] = sum_t dOut[b,t,:] (same fixed order) give dw = <gsum, V_e[b,0]>,
+// vbar = V_e[b,0], and are kept for its dV (written by the CTAs of encoder gsum_e, the first single-token one).
 constexpr int kMixRedCols = 8;  // 16-byte vectors per CTA
 template <typename T>
 __global__ void __launch_bounds__(256) mix_bwd_reduce_kernel(const __grid_constant__ BwdPtrs p, const T* __restrict__ dOut, float* __restrict__ dw_partial,
-                                                             float* __restrict__ vbar, int E, int Ttok, int K) {
+                                                             float* __restrict__ vbar, float* __restrict__ gsum, int gsum_e, int E, int Ttok, int K) {
   constexpr int VEC = Vec16<T>::kN;
   __shared__ float part[32][kMixRedCols * VEC + 1];
   __shared__ float red[32];
   const int kb = blockIdx.x, e = blockIdx.y, b = blockIdx.z;
   const int cv = threadIdx.x & (kMixRedCols - 1), rg = threadIdx.x / kMixRedCols;
   const int k0 = (kb * kMixRedCols + cv) * VEC;
+  if (p.tokens[e] != Ttok) {
+    float gs[VEC];
+#pragma unroll
+    for (int c = 0; c < VEC; ++c) gs[c] = 0.f;
+    if (k0 < K) {
+      const T* g = dOut + (long long)b * Ttok * K + k0;
+      int t = rg;
+      for (; t + 96 < Ttok; t += 128) {
+        uint4 rd[4];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) rd[i] = ldg_nc_v4(g + (long long)(t + 32 * i) * K);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          float d[VEC];
+          Vec16<T>::unpack(rd[i], d);
+#pragma unroll
+          for (int c = 0; c < VEC; ++c) gs[c] += d[c];
+        }
+      }
+      for (; t < Ttok; t += 32) {
+        float d[VEC];
+        Vec16<T>::unpack(ldg_nc_v4(g + (long long)t * K), d);
+#pragma unroll
+        for (int c = 0; c < VEC; ++c) gs[c] += d[c];
+      }
+    }
+#pragma unroll
+    for (int c = 0; c < VEC; ++c) part[rg][cv * VEC + c] = gs[c];
+    __syncthreads();
+    float sdot = 0.f;
+    if (threadIdx.x < kMixRedCols * VEC) {
+      const int k = kb * kMixRedCols * VEC + threadIdx.x;
+      if (k < K) {
+        float sum = 0.f;
+#pragma unroll
+        for (int gidx = 0; gidx < 32; ++gidx) sum += part[gidx][threadIdx.x];
+        const float v = to_float(static_cast<const T*>(p.V[e])[(long long)b * K + k]);
+        vbar[((long long)b * E + e) * K + k] = v;
+        if (e == gsum_e) gsum[(long long)b * K + k] = sum;
+        sdot = sum * v;
+      }
+    }
+    sdot = bwd_block_sum<256>(sdot, red);
+    if (threadIdx.x == 0) dw_partial[((long long)b * E + e) * gridDim.x + kb] = sdot;
+    return;
+  }
   float vs[VEC], dot = 0.f;
 #pragma unroll
   for (int c = 0; c < VEC; ++c) vs[c] = 0.f;
@@ -153,10 +209,10 @@ __global__ void __launch_bounds__(32) mix_bwd_scores_kernel(const float* __restr
   if (lane < E) ds[(long long)b * E + lane] = w * (dw - inner);
 }
 
-// ---- stage 3: dV_e[b,t,:] = w[b,e] dOut[b,t,:] + (ds[b,e] / T) u -----------------------------------------------
+// ---- stage 3: dV_e[b,t,:] = w[b,e] dOut[b,t,:] + (ds[b,e] / T) u  for the encoders in full_mask (the T-token ones) --------------
 template <typename T, int E>
 __global__ void __launch_bounds__(256) mix_bwd_dv_kernel(const __grid_constant__ BwdPtrs p, const T* __restrict__ dOut, const float* __restrict__ weights,
-                                                         const float* __restrict__ ds, const float* __restrict__ u, int Ttok, int K) {
+                                                         const float* __restrict__ ds, const float* __restrict__ u, int Ttok, int K, unsigned full_mask) {
   constexpr int VEC = Vec16<T>::kN;
   const int b = blockIdx.y;
   float w[E], s[E];
@@ -179,11 +235,78 @@ __global__ void __launch_bounds__(256) mix_bwd_dv_kernel(const __grid_constant__
     }
 #pragma unroll
     for (int e = 0; e < E; ++e) {
+      if (!((full_mask >> e) & 1u)) continue;
       float o[VEC];
 #pragma unroll
       for (int c = 0; c < VEC; ++c) o[c] = fmaf(w[e], d[c], s[e] * uu[c]);
       stg_na_v4(static_cast<T*>(p.dV[e]) + (long long)b * Ttok * K + i * VEC, Vec16<T>::pack(o));
     }
+  }
+}
+
+// ---- stage 3, averagetoken=False (u [T, K], one row per token, no token mean in the score), with du in the same pass ------------
+//   dV_e[b,t,:] = w[b,e] dOut[b,t,:] + ds[b,e] u[t,:]   (T-token encoders, full_mask)
+//   du[t,:]     = sum_b sum_e ds[b,e] V_e[b,t,:]         (a single-token encoder contributes its one row V_e[b,0,:] to every t)
+// du needs ds, hence the second read of V; a thread owns one 16-byte column vector of one token for ALL videos, so du is summed in a fixed
+// order (videos, then encoders) in registers and written once: no atomics, no [B, T*K] partials.
+template <typename T, int E>
+__global__ void __launch_bounds__(256) mix_bwd_dv_flat_kernel(const __grid_constant__ BwdPtrs p, const T* __restrict__ dOut, const float* __restrict__ weights,
+                                                              const float* __restrict__ ds, const float* __restrict__ u, float* __restrict__ du, int B,
+                                                              int Ttok, int K, unsigned full_mask) {
+  constexpr int VEC = Vec16<T>::kN;
+  const int kvec = K / VEC;
+  const long long nvec = (long long)Ttok * kvec;
+  const long long vstride = (long long)Ttok * K;
+  for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < nvec; i += (long long)gridDim.x * 256) {
+    const int kc = int(i % kvec) * VEC;
+    float uu[VEC], acc[VEC];
+#pragma unroll
+    for (int c = 0; c < VEC; c += 4) {
+      const float4 u4 = __ldg(reinterpret_cast<const float4*>(u + i * VEC + c));
+      uu[c] = u4.x; uu[c + 1] = u4.y; uu[c + 2] = u4.z; uu[c + 3] = u4.w;
+    }
+#pragma unroll
+    for (int c = 0; c < VEC; ++c) acc[c] = 0.f;
+    for (int b = 0; b < B; ++b) {
+      float d[VEC];
+      Vec16<T>::unpack(ldg_nc_v4(dOut + b * vstride + i * VEC), d);
+#pragma unroll
+      for (int e = 0; e < E; ++e) {
+        const float w = __ldg(weights + (long long)b * E + e), s = __ldg(ds + (long long)b * E + e);
+        const bool full = (full_mask >> e) & 1u;
+        const T* v = static_cast<const T*>(p.V[e]) + (full ? b * vstride + i * VEC : (long long)b * K + kc);
+        float a[VEC];
+        Vec16<T>::unpack(full ? ldg_nc_v4(v) : ldg_v4(v), a);
+#pragma unroll
+        for (int c = 0; c < VEC; ++c) acc[c] = fmaf(s, a[c], acc[c]);
+        if (full) {
+          float o[VEC];
+#pragma unroll
+          for (int c = 0; c < VEC; ++c) o[c] = fmaf(w, d[c], s * uu[c]);
+          stg_na_v4(static_cast<T*>(p.dV[e]) + b * vstride + i * VEC, Vec16<T>::pack(o));
+        }
+      }
+    }
+#pragma unroll
+    for (int c = 0; c < VEC; ++c) du[i * VEC + c] = acc[c];  // du sits at a workspace offset that need not be 16-byte aligned
+  }
+}
+
+// ---- stage 3 of a single-token encoder: dV_e[b,0,:] = sum_t (row t of the T-token gradient) = w[b,e] gsum[b,:] + ds[b,e] ubar,
+//      ubar = u (averagetoken: T rows of (ds / T) u) or sum_t u[t,:] (averagetoken=False, u_rows = T).  grid (ceil(K / 256), B) --------
+template <typename T>
+__global__ void __launch_bounds__(256) mix_bwd_dv_single_kernel(const __grid_constant__ BwdPtrs p, const float* __restrict__ weights, const float* __restrict__ ds,
+                                                                const float* __restrict__ u, int u_rows, const float* __restrict__ gsum, int E, int K,
+                                                                unsigned full_mask) {
+  const int k = blockIdx.x * 256 + threadIdx.x, b = blockIdx.y;
+  if (k >= K) return;
+  float ub = 0.f;
+  for (int r = 0; r < u_rows; ++r) ub += u[(long long)r * K + k];
+  const float g = gsum[(long long)b * K + k];
+  for (int e = 0; e < E; ++e) {
+    if ((full_mask >> e) & 1u) continue;
+    const float w = weights[(long long)b * E + e], s = ds[(long long)b * E + e];
+    static_cast<T*>(p.dV[e])[(long long)b * K + k] = from_float<T>(fmaf(w, g, s * ub));
   }
 }
 
@@ -194,6 +317,24 @@ __global__ void __launch_bounds__(256) du_kernel(const float* __restrict__ ds, c
   if (k >= K) return;
   float acc = 0.f;
   for (int i = 0; i < BE; ++i) acc = fmaf(ds[i], vbar[(long long)i * K + k], acc);
+  du[k] = acc;
+}
+// positional_embedding=True: the key is mean_t V_e + pe[e], so  du[k] = sum_{b,e} ds[b,e] (vbar[b,e,k] + pe[e,k])  and
+// dpe[e,k] = (sum_b ds[b,e]) u[k]; the column sums sig_e are recomputed per thread (B * E floats from L1, fixed order)
+template <typename T>
+__global__ void __launch_bounds__(256) du_pe_kernel(const float* __restrict__ ds, const float* __restrict__ vbar, const T* __restrict__ pe, long long ldpe,
+                                                    const float* __restrict__ u, float* __restrict__ du, T* __restrict__ dpe, int B, int E, int K) {
+  const int k = blockIdx.x * 256 + threadIdx.x;
+  if (k >= K) return;
+  float acc = 0.f;
+  for (int i = 0; i < B * E; ++i) acc = fmaf(ds[i], vbar[(long long)i * K + k], acc);
+  const float uk = u[k];
+  for (int e = 0; e < E; ++e) {
+    float sig = 0.f;
+    for (int b = 0; b < B; ++b) sig += ds[(long long)b * E + e];
+    acc = fmaf(sig, to_float(pe[(long long)e * ldpe + k]), acc);
+    dpe[(long long)e * K + k] = from_float<T>(sig * uk);
+  }
   du[k] = acc;
 }
 // out[d] = scale * sum_k W[d,k] x[k] (+ bias[d]) : one warp per row
@@ -308,7 +449,7 @@ __global__ void __launch_bounds__(256) gelu_kernel(const T* __restrict__ z, cons
 
 template <typename T>
 static int launch_mix_dv(const BwdPtrs& p, const void* dOut, const float* weights, const float* ds, const float* u, int B, int E, int Ttok, int K,
-                         cudaStream_t s) {
+                         unsigned full_mask, cudaStream_t s) {
   constexpr int VEC = Vec16<T>::kN;
   const long long nvec = (long long)Ttok * (K / VEC);
   long long gx = (nvec + 255) / 256;
@@ -317,10 +458,29 @@ static int launch_mix_dv(const BwdPtrs& p, const void* dOut, const float* weight
   dim3 grid((unsigned)gx, B);
   const T* g = static_cast<const T*>(dOut);
   switch (E) {
-#define MERV_DV_CASE(n) case n: mix_bwd_dv_kernel<T, n><<<grid, 256, 0, s>>>(p, g, weights, ds, u, Ttok, K); break;
+#define MERV_DV_CASE(n) case n: mix_bwd_dv_kernel<T, n><<<grid, 256, 0, s>>>(p, g, weights, ds, u, Ttok, K, full_mask); break;
     MERV_DV_CASE(1) MERV_DV_CASE(2) MERV_DV_CASE(3) MERV_DV_CASE(4) MERV_DV_CASE(5) MERV_DV_CASE(6) MERV_DV_CASE(7) MERV_DV_CASE(8)
 #undef MERV_DV_CASE
     default: return fail(MERV_E_ARG, "merv_mix_backward: E=%d", E);
+  }
+  MERV_CUDA_OK(cudaGetLastError());
+  return MERV_OK;
+}
+
+template <typename T>
+static int launch_mix_dv_flat(const BwdPtrs& p, const void* dOut, const float* weights, const float* ds, const float* u, float* du, int B, int E,
+                              int Ttok, int K, unsigned full_mask, cudaStream_t s) {
+  constexpr int VEC = Vec16<T>::kN;
+  const long long nvec = (long long)Ttok * (K / VEC);
+  long long gx = (nvec + 255) / 256;
+  const long long cap = (long long)sm_count() * 16;  // every thread walks all B videos
+  if (gx > cap) gx = cap;
+  const T* g = static_cast<const T*>(dOut);
+  switch (E) {
+#define MERV_DV_CASE(n) case n: mix_bwd_dv_flat_kernel<T, n><<<(unsigned)gx, 256, 0, s>>>(p, g, weights, ds, u, du, B, Ttok, K, full_mask); break;
+    MERV_DV_CASE(1) MERV_DV_CASE(2) MERV_DV_CASE(3) MERV_DV_CASE(4) MERV_DV_CASE(5) MERV_DV_CASE(6) MERV_DV_CASE(7) MERV_DV_CASE(8)
+#undef MERV_DV_CASE
+    default: return fail(MERV_E_ARG, "merv_mix_backward_ex: E=%d", E);
   }
   MERV_CUDA_OK(cudaGetLastError());
   return MERV_OK;
@@ -763,11 +923,106 @@ extern "C" int merv_colsum(const void* x, void* out, float* workspace, int M, in
 }
 
 constexpr int kMixDqSplit = 16;  // row splits of the two-stage dQ = Wq^T dq (3072 x 3072: 96 CTAs in one stage could not fill the GPU)
+// floats of the workspace without the single-token column sums: dw partials | vbar | ds | du (ku floats) | q | dq | dq partials
+static size_t mix_bwd_base_floats(int B, int E, int K, size_t ku, int embed) {
+  const size_t kblocks = (size_t)(K + kMixRedCols * 4 - 1) / (kMixRedCols * 4);  // upper bound (fp32 vectors are the narrower ones)
+  return (size_t)B * E * kblocks + (size_t)B * E * K + (size_t)B * E + ku + 2 * (size_t)embed + (size_t)kMixDqSplit * embed;
+}
+
 extern "C" size_t merv_mix_backward_workspace(int B, int E, int T, int K, int embed) {
   (void)T;
   if (B <= 0 || E <= 0 || K <= 0) return 0;
-  const size_t kblocks = (size_t)(K + kMixRedCols * 4 - 1) / (kMixRedCols * 4);  // upper bound (fp32 vectors are the narrower ones)
-  return (size_t)B * E * kblocks + (size_t)B * E * K + (size_t)B * E + (size_t)K + 2 * (size_t)embed + (size_t)kMixDqSplit * embed;
+  return mix_bwd_base_floats(B, E, K, (size_t)K, embed);
+}
+
+extern "C" size_t merv_mix_backward_ex_workspace(int B, int E, int T, int K, int embed, int64_t u_token_stride) {
+  if (B <= 0 || E <= 0 || T <= 0 || K <= 0) return 0;
+  const size_t ku = u_token_stride != 0 ? (size_t)T * K : (size_t)K;
+  return mix_bwd_base_floats(B, E, K, ku, embed) + (size_t)B * K;  // + gsum [B, K] of the single-token encoders
+}
+
+// Every case of CrossAttentionAdapterLearnableQuery.forward (nn_utils.py:487-521).  V_e [B, T_e, K] with T_e = tokens[e] in {T, 1},
+// dOut [B, T, K], weights fp32 [B, E] (forward output), dweights_out (optional) fp32 [B, E]: gradient w.r.t. the returned weights.
+//   u_token_stride == 0 : averagetoken=True,  u fp32 [K],    s_e = u . (mean_t V_e + pe[e])     (pe [E, K] (ldpe) or NULL)
+//   u_token_stride == K : averagetoken=False, u fp32 [T*K],  s_e = sum_t u[t,:] . V_e[b,t,:]    (pe must be NULL; Wk is [embed, T*K])
+// Outputs: dV_e [B, T_e, K], dQ [embed], dWq [embed, embed], dWk [embed, T*K or K], dbias [3 * embed] and, with pe, dpe [E, K] (all `dtype`).
+// The T-token-only, stride-0, pe-less call is merv_mix_backward: the same kernels, bit-identical gradients.
+extern "C" int merv_mix_backward_ex(const void* const* V, const int32_t* tokens, const void* dOut, const float* weights, const float* dweights_out,
+                                    const float* u, int64_t u_token_stride, const void* pe, int64_t ldpe, const void* Q, const void* Wq, const void* Wk,
+                                    const void* in_proj_bias, void* const* dV, void* dQ, void* dWq, void* dWk, void* dbias, void* dpe, float* workspace,
+                                    size_t workspace_floats, int B, int E, int T, int K, int embed, int dtype, void* stream) {
+  MERV_REQUIRE(dtype == MERV_F32 || dtype == MERV_BF16, MERV_E_DTYPE, "merv_mix_backward_ex: unknown dtype %d", dtype);
+  MERV_REQUIRE(V && tokens && dOut && weights && u && Q && Wq && Wk && dV && dQ && dWq && dWk && dbias && workspace, MERV_E_ARG,
+               "merv_mix_backward_ex: NULL pointer");
+  MERV_REQUIRE(E >= 1 && E <= MERV_MAX_ENCODERS, MERV_E_ARG, "merv_mix_backward_ex: E=%d", E);
+  MERV_REQUIRE(B > 0 && T > 0 && K > 0 && embed > 0, MERV_E_SHAPE, "merv_mix_backward_ex: B=%d T=%d K=%d embed=%d", B, T, K, embed);
+  const int vec = dtype == MERV_BF16 ? 8 : 4;
+  MERV_REQUIRE(K % vec == 0, MERV_E_SHAPE, "merv_mix_backward_ex: K=%d must be a multiple of %d", K, vec);
+  const bool flat = u_token_stride != 0;
+  MERV_REQUIRE(!flat || u_token_stride == K, MERV_E_SHAPE, "merv_mix_backward_ex: u_token_stride=%lld (0 or K=%d)", (long long)u_token_stride, K);
+  MERV_REQUIRE(!flat || (long long)T * K <= 0x7fffffffLL, MERV_E_SHAPE, "merv_mix_backward_ex: T*K overflows");
+  MERV_REQUIRE(!(flat && pe), MERV_E_ARG, "merv_mix_backward_ex: pe is only read with averagetoken=True (u_token_stride == 0)");
+  MERV_REQUIRE((pe == nullptr) == (dpe == nullptr), MERV_E_ARG, "merv_mix_backward_ex: pe and dpe go together");
+  MERV_REQUIRE(pe == nullptr || ldpe >= K, MERV_E_SHAPE, "merv_mix_backward_ex: ldpe=%lld < K=%d", (long long)ldpe, K);
+  MERV_REQUIRE(aligned16(u), MERV_E_ALIGN, "merv_mix_backward_ex: u must be 16-byte aligned");
+  if (int rc = require_sm100()) return rc;
+  BwdPtrs p = {};
+  unsigned full_mask = 0;
+  int gsum_e = -1;
+  for (int e = 0; e < E; ++e) {
+    MERV_REQUIRE(tokens[e] == T || tokens[e] == 1, MERV_E_SHAPE, "merv_mix_backward_ex: encoder %d has %d tokens, expected %d or 1", e, tokens[e], T);
+    MERV_REQUIRE(V[e] && dV[e] && aligned16(V[e]) && aligned16(dV[e]), MERV_E_ALIGN, "merv_mix_backward_ex: encoder %d: NULL or misaligned tensor", e);
+    p.V[e] = V[e];
+    p.dV[e] = dV[e];
+    p.tokens[e] = tokens[e];
+    if (tokens[e] == T) full_mask |= 1u << e;
+    else if (gsum_e < 0) gsum_e = e;
+  }
+  const int Ku = flat ? T * K : K;  // length of u, du and the rows of Wk / dWk
+  const size_t base = mix_bwd_base_floats(B, E, K, (size_t)Ku, embed);
+  MERV_REQUIRE(workspace_floats >= base + (gsum_e >= 0 ? (size_t)B * K : 0), MERV_E_ARG, "merv_mix_backward_ex: workspace too small");
+  const int kblocks = (K / vec + kMixRedCols - 1) / kMixRedCols;
+  float* dw_partial = workspace;
+  float* vbar = dw_partial + (size_t)B * E * ((K + kMixRedCols * 4 - 1) / (kMixRedCols * 4));
+  float* ds = vbar + (size_t)B * E * K;
+  float* du = ds + (size_t)B * E;
+  float* q = du + Ku;
+  float* dq = q + embed;
+  float* dq_partial = dq + embed;  // [kMixDqSplit, embed]
+  float* gsum = workspace + base;  // [B, K], single-token encoders only
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const float rs = 1.0f / sqrtf(float(embed));
+  const long long nWk = (long long)embed * Ku, nWq = (long long)embed * embed;
+#define MERV_MIX_BWD_BODY(T_)                                                                                                                      \
+  mix_bwd_reduce_kernel<T_><<<dim3(kblocks, E, B), 256, 0, s>>>(p, (const T_*)dOut, dw_partial, vbar, gsum, gsum_e, E, T, K);                     \
+  mix_bwd_scores_kernel<<<B, 32, 0, s>>>(dw_partial, weights, dweights_out, ds, E, kblocks);                                                       \
+  if (flat) {                                                                                                                                      \
+    if (int rc = launch_mix_dv_flat<T_>(p, dOut, weights, ds, u, du, B, E, T, K, full_mask, s)) return rc;                                         \
+  } else {                                                                                                                                         \
+    if (full_mask != 0) {                                                                                                                          \
+      if (int rc = launch_mix_dv<T_>(p, dOut, weights, ds, u, B, E, T, K, full_mask, s)) return rc;                                                \
+    }                                                                                                                                              \
+    if (pe != nullptr)                                                                                                                             \
+      du_pe_kernel<T_><<<(K + 255) / 256, 256, 0, s>>>(ds, vbar, (const T_*)pe, ldpe, u, du, (T_*)dpe, B, E, K);                                   \
+    else                                                                                                                                           \
+      du_kernel<<<(K + 255) / 256, 256, 0, s>>>(ds, vbar, du, B * E, K);                                                                           \
+  }                                                                                                                                                \
+  if (gsum_e >= 0)                                                                                                                                 \
+    mix_bwd_dv_single_kernel<T_><<<dim3((K + 255) / 256, B), 256, 0, s>>>(p, weights, ds, u, flat ? T : 1, gsum, E, K, full_mask);                 \
+  launch_gemv_n<T_, T_>((const T_*)Wq, (const T_*)Q, (const T_*)in_proj_bias, q, embed, embed, 1.0f, s);                                          \
+  launch_gemv_n<T_, float>((const T_*)Wk, du, nullptr, dq, embed, Ku, rs, s);                                                                      \
+  outer_kernel<T_, float><<<(unsigned)((nWk + 255) / 256), 256, 0, s>>>(q, du, (T_*)dWk, embed, Ku, rs);                                          \
+  outer_kernel<T_, T_><<<(unsigned)((nWq + 255) / 256), 256, 0, s>>>(dq, (const T_*)Q, (T_*)dWq, embed, embed, 1.0f);                             \
+  gemv_tf_partial_kernel<T_><<<dim3((embed + 31) / 32, kMixDqSplit), 256, 0, s>>>((const T_*)Wq, dq, dq_partial, embed, embed);                    \
+  fused_bwd_final_kernel<T_><<<(3 * embed + 255) / 256, 256, 0, s>>>(dq_partial, kMixDqSplit, dq, (T_*)dQ, (T_*)dbias, embed);
+  if (dtype == MERV_BF16) {
+    MERV_MIX_BWD_BODY(__nv_bfloat16)
+  } else {
+    MERV_MIX_BWD_BODY(float)
+  }
+#undef MERV_MIX_BWD_BODY
+  MERV_CUDA_OK(cudaGetLastError());
+  return MERV_OK;
 }
 
 // V_e [B, T, K] (all encoders must have T tokens), dOut [B, T, K], weights fp32 [B, E] (forward output), u fp32 [K];
@@ -784,51 +1039,10 @@ extern "C" int merv_mix_backward(const void* const* V, const void* dOut, const f
   const int vec = dtype == MERV_BF16 ? 8 : 4;
   MERV_REQUIRE(K % vec == 0, MERV_E_SHAPE, "merv_mix_backward: K=%d must be a multiple of %d", K, vec);
   MERV_REQUIRE(workspace_floats >= merv_mix_backward_workspace(B, E, T, K, embed), MERV_E_ARG, "merv_mix_backward: workspace too small");
-  if (int rc = require_sm100()) return rc;
-  BwdPtrs p = {};
-  for (int e = 0; e < E; ++e) {
-    MERV_REQUIRE(V[e] && dV[e] && aligned16(V[e]) && aligned16(dV[e]), MERV_E_ALIGN, "merv_mix_backward: encoder %d: NULL or misaligned tensor", e);
-    p.V[e] = V[e];
-    p.dV[e] = dV[e];
-  }
-  const int kblocks = (K / vec + kMixRedCols - 1) / kMixRedCols;
-  float* dw_partial = workspace;
-  float* vbar = dw_partial + (size_t)B * E * ((K + kMixRedCols * 4 - 1) / (kMixRedCols * 4));
-  float* ds = vbar + (size_t)B * E * K;
-  float* du = ds + (size_t)B * E;
-  float* q = du + K;
-  float* dq = q + embed;
-  float* dq_partial = dq + embed;  // [kMixDqSplit, embed]
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const float rs = 1.0f / sqrtf(float(embed));
-  const long long nWk = (long long)embed * K, nWq = (long long)embed * embed;
-  if (dtype == MERV_BF16) {
-    using T_ = __nv_bfloat16;
-    mix_bwd_reduce_kernel<T_><<<dim3(kblocks, E, B), 256, 0, s>>>(p, (const T_*)dOut, dw_partial, vbar, E, T, K);
-    mix_bwd_scores_kernel<<<B, 32, 0, s>>>(dw_partial, weights, dweights_out, ds, E, kblocks);
-    if (int rc = launch_mix_dv<T_>(p, dOut, weights, ds, u, B, E, T, K, s)) return rc;
-    du_kernel<<<(K + 255) / 256, 256, 0, s>>>(ds, vbar, du, B * E, K);
-    launch_gemv_n<T_, T_>((const T_*)Wq, (const T_*)Q, (const T_*)in_proj_bias, q, embed, embed, 1.0f, s);
-    launch_gemv_n<T_, float>((const T_*)Wk, du, nullptr, dq, embed, K, rs, s);
-    outer_kernel<T_, float><<<(unsigned)((nWk + 255) / 256), 256, 0, s>>>(q, du, (T_*)dWk, embed, K, rs);
-    outer_kernel<T_, T_><<<(unsigned)((nWq + 255) / 256), 256, 0, s>>>(dq, (const T_*)Q, (T_*)dWq, embed, embed, 1.0f);
-    gemv_tf_partial_kernel<T_><<<dim3((embed + 31) / 32, kMixDqSplit), 256, 0, s>>>((const T_*)Wq, dq, dq_partial, embed, embed);
-    fused_bwd_final_kernel<T_><<<(3 * embed + 255) / 256, 256, 0, s>>>(dq_partial, kMixDqSplit, dq, (T_*)dQ, (T_*)dbias, embed);
-  } else {
-    using T_ = float;
-    mix_bwd_reduce_kernel<T_><<<dim3(kblocks, E, B), 256, 0, s>>>(p, (const T_*)dOut, dw_partial, vbar, E, T, K);
-    mix_bwd_scores_kernel<<<B, 32, 0, s>>>(dw_partial, weights, dweights_out, ds, E, kblocks);
-    if (int rc = launch_mix_dv<T_>(p, dOut, weights, ds, u, B, E, T, K, s)) return rc;
-    du_kernel<<<(K + 255) / 256, 256, 0, s>>>(ds, vbar, du, B * E, K);
-    launch_gemv_n<T_, T_>((const T_*)Wq, (const T_*)Q, (const T_*)in_proj_bias, q, embed, embed, 1.0f, s);
-    launch_gemv_n<T_, float>((const T_*)Wk, du, nullptr, dq, embed, K, rs, s);
-    outer_kernel<T_, float><<<(unsigned)((nWk + 255) / 256), 256, 0, s>>>(q, du, (T_*)dWk, embed, K, rs);
-    outer_kernel<T_, T_><<<(unsigned)((nWq + 255) / 256), 256, 0, s>>>(dq, (const T_*)Q, (T_*)dWq, embed, embed, 1.0f);
-    gemv_tf_partial_kernel<T_><<<dim3((embed + 31) / 32, kMixDqSplit), 256, 0, s>>>((const T_*)Wq, dq, dq_partial, embed, embed);
-    fused_bwd_final_kernel<T_><<<(3 * embed + 255) / 256, 256, 0, s>>>(dq_partial, kMixDqSplit, dq, (T_*)dQ, (T_*)dbias, embed);
-  }
-  MERV_CUDA_OK(cudaGetLastError());
-  return MERV_OK;
+  int32_t tokens[MERV_MAX_ENCODERS];
+  for (int e = 0; e < E; ++e) tokens[e] = T;
+  return merv_mix_backward_ex(V, tokens, dOut, weights, dweights_out, u, 0, nullptr, 0, Q, Wq, Wk, in_proj_bias, dV, dQ, dWq, dWk, dbias, nullptr,
+                              workspace, workspace_floats, B, E, T, K, embed, dtype, stream);
 }
 
 // out = gelu(z) (dy == NULL) or out = dy * gelu'(z); n elements, contiguous, n % (16 / sizeof) == 0

@@ -226,26 +226,37 @@ class _ConvTapsFn(torch.autograd.Function):
 
 
 class _MixFn(torch.autograd.Function):
-    """CrossAttentionAdapterLearnableQuery.forward (nn_utils.py:487-521) with its hand-written backward."""
+    """CrossAttentionAdapterLearnableQuery.forward (nn_utils.py:487-521) with its hand-written backward, in every configuration:
+    averagetoken=True / False, single-token (repeated) encoders, and positional_embedding=True, where ``pe`` is an input (None
+    otherwise: with averagetoken=False the reference never reads it, so it gets no gradient)."""
 
     @staticmethod
-    def forward(ctx, adapter, dtype, Q, Wq, Wk, bias, *V):
+    def forward(ctx, adapter, dtype, Q, Wq, Wk, bias, pe, *V):
         c = adapter._cast_cache
         Vc = [v if v.dtype == dtype else v.to(dtype) for v in V]
-        u = adapter.query_vector(dtype)
-        scores = ops.scores_from_tokens(Vc, u, adapter.token_length)
+        u = adapter.query_vector(dtype)  # [K], or [T*K] with averagetoken=False (the key is the flattened token block)
+        per_token_u = not adapter.averagetoken
+        scores = ops.scores_from_tokens(Vc, u, adapter.token_length, per_token_u=per_token_u, consts=adapter._pe_consts(dtype),
+                                        mean=adapter.averagetoken)
         out, weights = ops.softmax_mix(Vc, adapter.token_length, scores=scores)
-        ctx.save_for_backward(weights, u, c.get(Q, dtype), c.get(Wq, dtype), c.get(Wk, dtype), c.get(bias, dtype), *Vc)
-        ctx.meta = (dtype, [p.dtype for p in (Q, Wq, Wk, bias)], [v.dtype for v in V])
+        params = (Q, Wq, Wk, bias) + (() if pe is None else (pe,))
+        ctx.save_for_backward(weights, u, *[c.get(p, dtype) for p in params], *Vc)
+        ctx.meta = (dtype, per_token_u, [p.dtype for p in params], [v.dtype for v in V])
         return out, weights.to(dtype)
 
     @staticmethod
     def backward(ctx, dout, dweights):
-        weights, u, Qc, Wqc, Wkc, bc, *Vc = ctx.saved_tensors
-        dtype, pdt, vdt = ctx.meta
+        dtype, per_token_u, pdt, vdt = ctx.meta
+        weights, u, Qc, Wqc, Wkc, bc, *rest = ctx.saved_tensors
+        pec, Vc = (rest[0], rest[1:]) if len(pdt) == 5 else (None, rest)
         dw = None if dweights is None else dweights.float().contiguous()
-        dVs, dQ, dWq, dWk, dbias = ops.mix_backward(Vc, dout.to(dtype), weights, dw, u, Qc, Wqc, Wkc, bc)
-        grads = [g.to(t) for g, t in zip((dQ, dWq, dWk, dbias), pdt)]
+        if per_token_u or pec is not None or any(v.shape[1] != dout.shape[1] for v in Vc):
+            dVs, dQ, dWq, dWk, dbias, dpe = ops.mix_backward_ex(Vc, dout.to(dtype), weights, dw, u, Qc, Wqc, Wkc, bc, per_token_u=per_token_u, pe=pec)
+        else:  # the configuration MERV constructs (merv.py:214-216): the same kernels, bit-identical to mix_backward_ex
+            (dVs, dQ, dWq, dWk, dbias), dpe = ops.mix_backward(Vc, dout.to(dtype), weights, dw, u, Qc, Wqc, Wkc, bc), None
+        grads = [g.to(t) for g, t in zip((dQ, dWq, dWk, dbias, dpe), pdt)]
+        if dpe is None:
+            grads.append(None)
         return (None, None, *grads, *[g.to(t) for g, t in zip(dVs, vdt)])
 
 
@@ -1065,13 +1076,9 @@ class CrossAttentionAdapterLearnableQuery(nn.Module):
             raise NotImplementedError("out= / batch_index= / gather= are supported on the linked bf16 path only")
         V = [v.materialize() if isinstance(v, DeferredProjection) else v for v in V]
         if _needs_grad(self, *V):
-            if any(v.shape[1] != self.token_length for v in V):
-                raise NotImplementedError("the backward does not cover single-token (broadcast) encoders")
-            if not self.averagetoken or self.positional_embedding:
-                raise NotImplementedError("the backward covers averagetoken=True without positional embedding only "
-                                          "(the configuration MERV constructs, merv.py:214-216)")
             att = self.attention
-            return _MixFn.apply(self, _compute_dtype(V[0]), self.Q, att.q_proj_weight, att.k_proj_weight, att.in_proj_bias, *V)
+            pe = self.pe if self.positional_embedding and self.averagetoken else None
+            return _MixFn.apply(self, _compute_dtype(V[0]), self.Q, att.q_proj_weight, att.k_proj_weight, att.in_proj_bias, pe, *V)
         return self._forward_tokens(V)
 
     def _forward_tokens(self, V: Sequence[torch.Tensor], rowdots=None) -> Tuple[torch.Tensor, torch.Tensor]:

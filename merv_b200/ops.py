@@ -59,6 +59,7 @@ KERNELS_PER_CALL = {
     "merv_transpose": 1, "merv_colsum": 2, "merv_mix_backward": 10, "merv_gelu": 1,
     "merv_cross_attention": 1, "merv_cross_attention_backward": 1, "merv_add_rows": 1, "merv_video_colsum": 1, "merv_pair_dot": 1, "merv_transpose_rowscale": 1, "merv_fused_backward": 10, "merv_wgrad_video": 3,
     "merv_scores_from_tokens_ex": 2, "merv_score_consts": 1, "merv_layernorm": 1, "merv_layernorm_backward": 1, "merv_concat_linear": 1,
+    "merv_mix_backward_ex": 10,  # as merv_mix_backward; one more with single-token encoders, one fewer with averagetoken=False
 }
 
 
@@ -841,3 +842,40 @@ def mix_backward(Vs: Sequence[torch.Tensor], dout: torch.Tensor, weights: torch.
               ptr_array([d.data_ptr() for d in dVs]), dQ.data_ptr(), dWq.data_ptr(), dWk.data_ptr(), dbias.data_ptr(), ws.data_ptr(), n,
               B, E, T, K, embed, dtype_code(dt), _stream())
     return dVs, dQ, dWq, dWk, dbias
+
+
+def mix_backward_ex(Vs: Sequence[torch.Tensor], dout: torch.Tensor, weights: torch.Tensor, dweights: Optional[torch.Tensor], u: torch.Tensor,
+                    Q: torch.Tensor, Wq: torch.Tensor, Wk: torch.Tensor, in_proj_bias: torch.Tensor, per_token_u: bool = False,
+                    pe: Optional[torch.Tensor] = None):
+    """Gradients of the adapter in every configuration of its forward: V_e [B, T_e, K] with T_e in {T, 1} (dout is [B, T, K]),
+    ``per_token_u`` for averagetoken=False (u and the rows of Wk are [T*K]), ``pe`` [E, K] for positional_embedding=True.
+    Returns (dV list with each encoder's own T_e, dQ [1, embed], dWq, dWk, d in_proj_bias, dpe or None) in the compute dtype."""
+    lib = _lib.load()
+    dev = _require_cuda(*Vs, dout, weights, dweights, u, Q, Wq, Wk, in_proj_bias, pe)
+    B, T, K = dout.shape
+    E, embed = len(Vs), Wk.shape[0]
+    dt = Vs[0].dtype
+    Ku = T * K if per_token_u else K
+    Vs = [v.contiguous() for v in Vs]
+    dout = dout.contiguous()
+    assert all(v.shape in ((B, T, K), (B, 1, K)) and v.dtype == dt for v in Vs) and dout.dtype == dt
+    assert u.dtype == torch.float32 and u.is_contiguous() and u.numel() == Ku and Wk.shape[1] == Ku
+    assert weights.dtype == torch.float32 and weights.is_contiguous() and (dweights is None or (dweights.dtype == torch.float32 and dweights.is_contiguous()))
+    assert pe is None or (not per_token_u and pe.shape == (E, K) and pe.dtype == dt)
+    if pe is not None and pe.stride(1) != 1:
+        pe = pe.contiguous()
+    with torch.cuda.device(dev):
+        dVs = [torch.empty_like(v) for v in Vs]
+        dQ = torch.empty((1, embed), dtype=dt, device=dev)
+        dWq = torch.empty((embed, embed), dtype=dt, device=dev)
+        dWk = torch.empty((embed, Ku), dtype=dt, device=dev)
+        dbias = torch.empty(3 * embed, dtype=dt, device=dev)
+        dpe = None if pe is None else torch.empty((E, K), dtype=dt, device=dev)
+        n = lib.merv_mix_backward_ex_workspace(B, E, T, K, embed, K if per_token_u else 0)
+        ws = torch.empty(n, dtype=torch.float32, device=dev)
+        _call('merv_mix_backward_ex', lib.merv_mix_backward_ex, ptr_array([v.data_ptr() for v in Vs]), i32_array([v.shape[1] for v in Vs]),
+              dout.data_ptr(), weights.data_ptr(), _p(dweights), u.data_ptr(), K if per_token_u else 0, _p(pe), 0 if pe is None else pe.stride(0),
+              Q.contiguous().data_ptr(), Wq.contiguous().data_ptr(), Wk.contiguous().data_ptr(), in_proj_bias.data_ptr(),
+              ptr_array([d.data_ptr() for d in dVs]), dQ.data_ptr(), dWq.data_ptr(), dWk.data_ptr(), dbias.data_ptr(), _p(dpe), ws.data_ptr(), n,
+              B, E, T, K, embed, dtype_code(dt), _stream())
+    return dVs, dQ, dWq, dWk, dbias, dpe
