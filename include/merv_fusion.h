@@ -311,6 +311,16 @@ int merv_mix_backward_ex(const void* const* V, const int32_t* tokens, const void
                          const void* Q, const void* Wq, const void* Wk, const void* in_proj_bias, void* const* dV, void* dQ,
                          void* dWq, void* dWk, void* dbias, void* dpe, float* workspace, size_t workspace_floats, int B, int E,
                          int T, int K, int embed, int dtype, void* stream);
+/* Gradients of ScalarAdapter.forward (feature_fusion == "scalar", nn_utils.py:524-537): w = softmax(scalar) [E] for every video,
+ * out = sum_e w_e V_e, returned weights w[None].  With dweights_out [E] the gradient of the returned weights:
+ *     dV_e = w_e dOut,   g_e = sum_b <dOut[b], V_e[b]> + dweights_out[e],   dscalar = w (.) (g - <w, g>)
+ * V_e, dOut, dV_e [B, T, K] contiguous in `dtype` (the reference stacks the encoders, so all share one shape), weights fp32 [E],
+ * dweights_out fp32 [E] or NULL, dscalar fp32 [E] out.  One pass reads dOut and every V_e once and writes every dV_e once; the dots
+ * are reduced in a fixed order (bit-reproducible).  B == 0 reads no tensor: dscalar from dweights_out alone.
+ * workspace: merv_scalar_mix_backward_workspace(B, E, K) floats. */
+size_t merv_scalar_mix_backward_workspace(int B, int E, int K);
+int merv_scalar_mix_backward(const void* const* V, const void* dOut, const float* weights, const float* dweights_out, void* const* dV,
+                             float* dscalar, float* workspace, size_t workspace_floats, int B, int E, int T, int K, int dtype, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * Backward of the FUSED path (linear projectors linked to the adapter, forward = merv_fused_linear_mix): the training step of
@@ -374,6 +384,16 @@ int merv_wgrad_video(const void* dY, int64_t lddy, const void* X, int64_t ldx, c
                      int C, void* stream);
 size_t merv_fused_backward_workspace(const merv_fused_bwd_desc* desc);
 int merv_fused_backward(const merv_fused_bwd_desc* desc, int dtype, void* stream);
+/* The same fused training step in front of the ScalarAdapter (one w [E] for every video, no query vector).  Per encoder,
+ * merv_wgrad_video(dOut, P_e, scale = &w[e], scale_stride = 0, W_e) gives dW_e = w_e dOut^T P_e and dw_partial[e] = the partials of
+ * <W_e, dOut[b]^T P_e[b]>; merv_video_colsum(dOut) gives gsum [B, K].  This finishes the step, all sums in a fixed order:
+ *     gs = sum_b gsum[b],   db_e = w_e gs,   g_e = sum(dw_partial[e]) + b_e . gs + dweights_out[e],   dscalar = w (.) (g - <w, g>)
+ * weights fp32 [E], dweights_out fp32 [E] or NULL, dw_partial[e] fp32 [B, merv_pair_dot_chunks()], bias[e] / db[e] [K] (`dtype`) or
+ * NULL entries, dscalar fp32 [E] out.  workspace: merv_scalar_fused_backward_workspace(E, K) floats. */
+size_t merv_scalar_fused_backward_workspace(int E, int K);
+int merv_scalar_fused_backward(const float* weights, const float* dweights_out, const float* gsum, const float* const* dw_partial,
+                               const void* const* bias, void* const* db, float* dscalar, float* workspace, size_t workspace_floats, int B,
+                               int E, int K, int dtype, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * Attentive pooler ("attntv" resampler: AttentivePooler.forward, merv/util/nn_utils.py:229-238; constructed at

@@ -131,6 +131,12 @@ _SIGNATURES = {
     "merv_mix_backward_ex": (c_int, [_PP, POINTER(c_int32), c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p,
                                      c_void_p, c_void_p, _PP, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int, c_int,
                                      c_int, c_int, c_int, c_int, c_void_p]),
+    "merv_scalar_mix_backward_workspace": (c_size_t, [c_int, c_int, c_int]),
+    "merv_scalar_mix_backward": (c_int, [_PP, c_void_p, c_void_p, c_void_p, _PP, c_void_p, c_void_p, c_size_t, c_int, c_int, c_int, c_int, c_int,
+                                         c_void_p]),
+    "merv_scalar_fused_backward_workspace": (c_size_t, [c_int, c_int]),
+    "merv_scalar_fused_backward": (c_int, [c_void_p, c_void_p, c_void_p, _PP, _PP, _PP, c_void_p, c_void_p, c_size_t, c_int, c_int, c_int, c_int,
+                                           c_void_p]),
     "merv_softmax_mix": (c_int, [_PP, POINTER(c_int32), c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "merv_fused_linear_mix": (c_int, [_PP, POINTER(c_int64), _PP, POINTER(c_int64), POINTER(c_int32), c_int, c_void_p, c_void_p,
                                       c_void_p, c_int64, c_int64, c_int, c_int, c_int, c_int, c_void_p]),

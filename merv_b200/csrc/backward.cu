@@ -16,6 +16,9 @@
 //                           gsum[b] = sum_t dOut[b,t], ubar = u or sum_t u_t;  dw_e = <gsum[b], V_e[b,0]>, mean_t V_e = V_e[b,0]
 //   v_proj_weight / out_proj / b_k / b_v receive no (zero) gradient, exactly as in the reference where the attention
 //   output is discarded and b_k cancels in the softmax.
+//   ScalarAdapter (nn_utils.py:524-537, w = softmax(scalar) for every video, out = sum_e w_e V_e):
+//        dV_e = w_e dOut,  g_e = sum_b <dOut[b], V_e[b]> + dweights_out[e],  dscalar = w (.) (g - <w, g>)   (merv_scalar_mix_backward;
+//        in front of linked linear projectors merv_scalar_fused_backward finishes the fused step)
 // All reductions are fixed-order (deterministic, no atomics).
 #include "common.cuh"
 
@@ -486,6 +489,163 @@ static int launch_mix_dv_flat(const BwdPtrs& p, const void* dOut, const float* w
   return MERV_OK;
 }
 
+// ============================================================================================================
+// ScalarAdapter (feature_fusion == "scalar", nn_utils.py:524-537):  w = softmax(scalar) [E], the same for every video,
+// out = sum_e w_e V_e, returned weights w[None].  With dweights_out [E] the gradient of the returned weights:
+//     dV_e    = w_e dOut                                   (independent of the scalar gradient: one pass suffices)
+//     g_e     = sum_b <dOut[b], V_e[b]> + dweights_out[e]
+//     dscalar = w (.) (g - <w, g>)
+// ============================================================================================================
+
+// ---- one pass: grid (column blocks of 8 vectors = 128 bytes, B), 256 threads = 8 vectors x 32 token groups as in mix_bwd_reduce_kernel,
+//      but a CTA owns its column block for ALL encoders: every dOut vector is read once (not once per encoder), every V_e vector once and
+//      every dV_e vector written once, (1 + 2E) B T K elements in all.  Two tokens per iteration keep 2 (1 + E) independent 16-byte loads
+//      in flight per thread.  The dots are reduced in a fixed order (warp butterfly, then the 8 warps in order) into partial[b, e, kb].
+template <typename T, int E>
+__global__ void __launch_bounds__(256) scalar_mix_bwd_kernel(const __grid_constant__ BwdPtrs p, const T* __restrict__ dOut, const float* __restrict__ weights,
+                                                             float* __restrict__ partial, int Ttok, int K) {
+  constexpr int VEC = Vec16<T>::kN;
+  __shared__ float red[E][8];
+  const int kb = blockIdx.x, b = blockIdx.y;
+  const int cv = threadIdx.x & (kMixRedCols - 1), rg = threadIdx.x / kMixRedCols;
+  const int k0 = (kb * kMixRedCols + cv) * VEC;
+  float w[E], dot[E];
+#pragma unroll
+  for (int e = 0; e < E; ++e) {
+    w[e] = weights[e];
+    dot[e] = 0.f;
+  }
+  if (k0 < K) {
+    const long long base = (long long)b * Ttok * K + k0;
+    const T* g = dOut + base;
+    const T* vb[E];
+    T* db[E];
+#pragma unroll
+    for (int e = 0; e < E; ++e) {
+      vb[e] = static_cast<const T*>(p.V[e]) + base;
+      db[e] = static_cast<T*>(p.dV[e]) + base;
+    }
+    int t = rg;
+    for (; t + 32 < Ttok; t += 64) {
+      uint4 rd[2], rv[2][E];
+#pragma unroll
+      for (int i = 0; i < 2; ++i) {
+        const long long off = (long long)(t + 32 * i) * K;
+        rd[i] = ldg_nc_v4(g + off);
+#pragma unroll
+        for (int e = 0; e < E; ++e) rv[i][e] = ldg_nc_v4(vb[e] + off);
+      }
+#pragma unroll
+      for (int i = 0; i < 2; ++i) {
+        const long long off = (long long)(t + 32 * i) * K;
+        float d[VEC];
+        Vec16<T>::unpack(rd[i], d);
+#pragma unroll
+        for (int e = 0; e < E; ++e) {
+          float a[VEC], o[VEC];
+          Vec16<T>::unpack(rv[i][e], a);
+#pragma unroll
+          for (int c = 0; c < VEC; ++c) {
+            dot[e] = fmaf(a[c], d[c], dot[e]);
+            o[c] = w[e] * d[c];
+          }
+          stg_na_v4(db[e] + off, Vec16<T>::pack(o));
+        }
+      }
+    }
+#pragma unroll 1
+    for (; t < Ttok; t += 32) {
+      const long long off = (long long)t * K;
+      float d[VEC];
+      Vec16<T>::unpack(ldg_nc_v4(g + off), d);
+#pragma unroll
+      for (int e = 0; e < E; ++e) {
+        float a[VEC], o[VEC];
+        Vec16<T>::unpack(ldg_nc_v4(vb[e] + off), a);
+#pragma unroll
+        for (int c = 0; c < VEC; ++c) {
+          dot[e] = fmaf(a[c], d[c], dot[e]);
+          o[c] = w[e] * d[c];
+        }
+        stg_na_v4(db[e] + off, Vec16<T>::pack(o));
+      }
+    }
+  }
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int e = 0; e < E; ++e) {
+    const float v = warp_sum(dot[e]);
+    if (lane == 0) red[e][warp] = v;
+  }
+  __syncthreads();
+  if (threadIdx.x < E) {
+    float s = 0.f;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) s += red[threadIdx.x][i];
+    partial[((long long)b * E + threadIdx.x) * gridDim.x + kb] = s;
+  }
+}
+
+// ---- the end of both scalar backward paths (256 threads, all of them call it): per-thread sums acc[e] -> block sums (warp butterfly, then
+//      the 8 warps in order) -> g_e = block sum + dweights_out[e] -> dscalar = w (.) (g - <w, g>) ------------------------------------------
+__device__ __forceinline__ void scalar_grad_from_block(const float (&acc)[MERV_MAX_ENCODERS], const float* __restrict__ weights,
+                                                       const float* __restrict__ dweights_out, float* __restrict__ dscalar, int E) {
+  __shared__ float red[MERV_MAX_ENCODERS][8];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int e = 0; e < MERV_MAX_ENCODERS; ++e) {
+    if (e >= E) break;
+    const float v = warp_sum(acc[e]);
+    if (lane == 0) red[e][warp] = v;
+  }
+  __syncthreads();
+  if (warp == 0) {
+    float g = 0.f, w = 0.f;
+    if (lane < E) {
+#pragma unroll
+      for (int i = 0; i < 8; ++i) g += red[lane][i];
+      if (dweights_out != nullptr) g += dweights_out[lane];
+      w = weights[lane];
+    }
+    const float inner = warp_sum(w * g);
+    if (lane < E) dscalar[lane] = w * (g - inner);
+  }
+}
+
+// ---- fold of the one-pass partials, one CTA: thread i sums the (video, column block) pairs i, i + 256, ... (videos outer) of every encoder.
+//      (A single warp would wait on B * kblocks / 32 dependent loads per encoder, 128 at 64 videos of merv-full.) --------------------------
+__global__ void __launch_bounds__(256) scalar_mix_fold_kernel(const float* __restrict__ partial, const float* __restrict__ weights,
+                                                              const float* __restrict__ dweights_out, float* __restrict__ dscalar, int B, int E,
+                                                              int kblocks) {
+  float acc[MERV_MAX_ENCODERS];
+#pragma unroll
+  for (int e = 0; e < MERV_MAX_ENCODERS; ++e) acc[e] = 0.f;
+  const long long n = (long long)B * kblocks;
+  for (long long i = threadIdx.x; i < n; i += 256) {
+    const long long b = i / kblocks, kb = i - b * kblocks;
+#pragma unroll
+    for (int e = 0; e < MERV_MAX_ENCODERS; ++e)
+      if (e < E) acc[e] += partial[(b * E + e) * kblocks + kb];
+  }
+  scalar_grad_from_block(acc, weights, dweights_out, dscalar, E);
+}
+
+template <typename T>
+static int launch_scalar_mix_bwd(const BwdPtrs& p, const void* dOut, const float* weights, float* partial, int B, int E, int Ttok, int K,
+                                 int kblocks, cudaStream_t s) {
+  dim3 grid(kblocks, B);
+  const T* g = static_cast<const T*>(dOut);
+  switch (E) {
+#define MERV_SCALAR_CASE(n) case n: scalar_mix_bwd_kernel<T, n><<<grid, 256, 0, s>>>(p, g, weights, partial, Ttok, K); break;
+    MERV_SCALAR_CASE(1) MERV_SCALAR_CASE(2) MERV_SCALAR_CASE(3) MERV_SCALAR_CASE(4) MERV_SCALAR_CASE(5) MERV_SCALAR_CASE(6) MERV_SCALAR_CASE(7)
+    MERV_SCALAR_CASE(8)
+#undef MERV_SCALAR_CASE
+    default: return fail(MERV_E_ARG, "merv_scalar_mix_backward: E=%d", E);
+  }
+  MERV_CUDA_OK(cudaGetLastError());
+  return MERV_OK;
+}
+
 
 // ============================================================================================================
 // Backward of the FUSED path (linear projectors linked to the adapter; merv_fused_linear_mix forward).
@@ -853,6 +1013,52 @@ __global__ void __launch_bounds__(256) fused_bwd_final_kernel(const float* __res
   if (i < 3 * embed) dbias[i] = from_float<T>(i < embed ? dq[i] : 0.f);  // b_k cancels in the softmax, b_v is dead
 }
 
+// ---- fused scalar step (linear projectors linked to the ScalarAdapter; forward = merv_fused_linear_mix with the same w for every video).
+//      merv_wgrad_video with scale_stride 0 gives dW_e = w_e dOut^T P_e and the partials of <W_e, dOut[b]^T P_e[b]> = <dOut[b], Y_e[b] - b_e>;
+//      with gs = sum_b gsum[b] (the column sums of dOut over every token):
+//          db_e = w_e gs,   g_e = sum of those partials + b_e . gs + dweights_out[e],   dscalar = w (.) (g - <w, g>)
+struct ScalarFusedPtrs {
+  const float* dw_partial[MERV_MAX_ENCODERS];  // [B, kPairDotChunks]
+  const void* bias[MERV_MAX_ENCODERS];         // [K] or NULL
+  void* db[MERV_MAX_ENCODERS];                 // [K] or NULL
+};
+
+// stage 1, grid ceil(K / 256): gs for 256 columns (videos in order), db_e, and the per-CTA sums of b_e . gs -> bpart[e, block]
+template <typename T>
+__global__ void __launch_bounds__(256) scalar_fused_bias_kernel(const __grid_constant__ ScalarFusedPtrs p, const float* __restrict__ gsum,
+                                                                const float* __restrict__ weights, float* __restrict__ bpart, int B, int E, int K) {
+  __shared__ float red[32];
+  const int k = blockIdx.x * 256 + threadIdx.x;
+  float gs = 0.f;
+  if (k < K)
+    for (int b = 0; b < B; ++b) gs += gsum[(long long)b * K + k];
+  for (int e = 0; e < E; ++e) {
+    float v = 0.f;
+    if (k < K) {
+      if (p.db[e] != nullptr) static_cast<T*>(p.db[e])[k] = from_float<T>(weights[e] * gs);
+      if (p.bias[e] != nullptr) v = to_float(static_cast<const T*>(p.bias[e])[k]) * gs;
+    }
+    v = bwd_block_sum<256>(v, red);
+    if (threadIdx.x == 0) bpart[(long long)e * gridDim.x + blockIdx.x] = v;
+  }
+}
+
+// stage 2, one CTA: g_e = the wgrad_video partials of encoder e (videos in order) + its bpart row + dweights_out[e], then dscalar
+__global__ void __launch_bounds__(256) scalar_fused_final_kernel(const __grid_constant__ ScalarFusedPtrs p, const float* __restrict__ bpart, int nbpart,
+                                                                 const float* __restrict__ weights, const float* __restrict__ dweights_out,
+                                                                 float* __restrict__ dscalar, int B, int E) {
+  float acc[MERV_MAX_ENCODERS];
+  const int n = B * kPairDotChunks;
+#pragma unroll
+  for (int e = 0; e < MERV_MAX_ENCODERS; ++e) {
+    acc[e] = 0.f;
+    if (e >= E) continue;
+    for (int i = threadIdx.x; i < n; i += 256) acc[e] += p.dw_partial[e][i];
+    for (int i = threadIdx.x; i < nbpart; i += 256) acc[e] += bpart[(long long)e * nbpart + i];
+  }
+  scalar_grad_from_block(acc, weights, dweights_out, dscalar, E);
+}
+
 }  // namespace merv
 
 using namespace merv;
@@ -1043,6 +1249,87 @@ extern "C" int merv_mix_backward(const void* const* V, const void* dOut, const f
   for (int e = 0; e < E; ++e) tokens[e] = T;
   return merv_mix_backward_ex(V, tokens, dOut, weights, dweights_out, u, 0, nullptr, 0, Q, Wq, Wk, in_proj_bias, dV, dQ, dWq, dWk, dbias, nullptr,
                               workspace, workspace_floats, B, E, T, K, embed, dtype, stream);
+}
+
+// ---- ScalarAdapter backward (see the block comment above scalar_mix_bwd_kernel) -------------------------------------------------------
+// floats of the [B, E, kblocks] partials; kblocks is bounded with the narrower fp32 vectors, as in mix_bwd_base_floats
+extern "C" size_t merv_scalar_mix_backward_workspace(int B, int E, int K) {
+  if (B <= 0 || E <= 0 || K <= 0) return 0;
+  return (size_t)B * E * ((K + kMixRedCols * 4 - 1) / (kMixRedCols * 4));
+}
+
+// V_e, dOut, dV_e [B, T, K] contiguous (`dtype`), weights = softmax(scalar) fp32 [E], dweights_out fp32 [E] or NULL, dscalar fp32 [E].
+// B == 0 (a rank without videos) reads no tensor and gives dscalar from dweights_out alone.
+extern "C" int merv_scalar_mix_backward(const void* const* V, const void* dOut, const float* weights, const float* dweights_out, void* const* dV,
+                                        float* dscalar, float* workspace, size_t workspace_floats, int B, int E, int T, int K, int dtype,
+                                        void* stream) {
+  MERV_REQUIRE(dtype == MERV_F32 || dtype == MERV_BF16, MERV_E_DTYPE, "merv_scalar_mix_backward: unknown dtype %d", dtype);
+  MERV_REQUIRE(V && dV && weights && dscalar, MERV_E_ARG, "merv_scalar_mix_backward: NULL pointer");
+  MERV_REQUIRE(E >= 1 && E <= MERV_MAX_ENCODERS, MERV_E_ARG, "merv_scalar_mix_backward: E=%d not in [1,%d]", E, MERV_MAX_ENCODERS);
+  MERV_REQUIRE(B >= 0 && T > 0 && K > 0, MERV_E_SHAPE, "merv_scalar_mix_backward: B=%d T=%d K=%d", B, T, K);
+  const int vec = dtype == MERV_BF16 ? 8 : 4;
+  MERV_REQUIRE(K % vec == 0, MERV_E_SHAPE, "merv_scalar_mix_backward: K=%d must be a multiple of %d", K, vec);
+  BwdPtrs p = {};
+  if (B > 0) {
+    MERV_REQUIRE(dOut && workspace, MERV_E_ARG, "merv_scalar_mix_backward: NULL pointer");
+    MERV_REQUIRE(aligned16(dOut), MERV_E_ALIGN, "merv_scalar_mix_backward: dOut must be 16-byte aligned");
+    for (int e = 0; e < E; ++e) {
+      MERV_REQUIRE(V[e] && dV[e], MERV_E_ARG, "merv_scalar_mix_backward: encoder %d: NULL pointer", e);
+      MERV_REQUIRE(aligned16(V[e]) && aligned16(dV[e]), MERV_E_ALIGN, "merv_scalar_mix_backward: encoder %d: tensor not 16-byte aligned", e);
+      p.V[e] = V[e];
+      p.dV[e] = dV[e];
+      p.tokens[e] = T;
+    }
+    MERV_REQUIRE(workspace_floats >= merv_scalar_mix_backward_workspace(B, E, K), MERV_E_ARG, "merv_scalar_mix_backward: workspace too small");
+  }
+  MERV_REQUIRE(B <= 65535, MERV_E_SHAPE, "merv_scalar_mix_backward: B=%d too large", B);
+  if (int rc = require_sm100()) return rc;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int kblocks = (K / vec + kMixRedCols - 1) / kMixRedCols;
+  if (B > 0) {
+    const int rc = dtype == MERV_BF16 ? launch_scalar_mix_bwd<__nv_bfloat16>(p, dOut, weights, workspace, B, E, T, K, kblocks, s)
+                                      : launch_scalar_mix_bwd<float>(p, dOut, weights, workspace, B, E, T, K, kblocks, s);
+    if (rc) return rc;
+  }
+  scalar_mix_fold_kernel<<<1, 256, 0, s>>>(workspace, weights, dweights_out, dscalar, B, E, kblocks);
+  MERV_CUDA_OK(cudaGetLastError());
+  return MERV_OK;
+}
+
+extern "C" size_t merv_scalar_fused_backward_workspace(int E, int K) {
+  if (E <= 0 || K <= 0) return 0;
+  return (size_t)E * ((K + 255) / 256);
+}
+
+// The fused scalar step after its merv_wgrad_video / merv_video_colsum calls: weights = softmax(scalar) fp32 [E], dweights_out fp32 [E] or
+// NULL, gsum fp32 [B, K] (merv_video_colsum(dOut)), dw_partial[e] fp32 [B, merv_pair_dot_chunks()] (merv_wgrad_video of encoder e with
+// scale_stride 0), bias[e] / db[e] [K] (`dtype`) or NULL, dscalar fp32 [E].
+extern "C" int merv_scalar_fused_backward(const float* weights, const float* dweights_out, const float* gsum, const float* const* dw_partial,
+                                          const void* const* bias, void* const* db, float* dscalar, float* workspace, size_t workspace_floats, int B,
+                                          int E, int K, int dtype, void* stream) {
+  MERV_REQUIRE(dtype == MERV_F32 || dtype == MERV_BF16, MERV_E_DTYPE, "merv_scalar_fused_backward: unknown dtype %d", dtype);
+  MERV_REQUIRE(weights && dw_partial && bias && db && dscalar && workspace, MERV_E_ARG, "merv_scalar_fused_backward: NULL pointer");
+  MERV_REQUIRE(E >= 1 && E <= MERV_MAX_ENCODERS, MERV_E_ARG, "merv_scalar_fused_backward: E=%d not in [1,%d]", E, MERV_MAX_ENCODERS);
+  MERV_REQUIRE(B >= 0 && K > 0 && (long long)B * kPairDotChunks <= 0x7fffffffLL, MERV_E_SHAPE, "merv_scalar_fused_backward: B=%d K=%d", B, K);
+  MERV_REQUIRE(B == 0 || gsum, MERV_E_ARG, "merv_scalar_fused_backward: NULL gsum");
+  MERV_REQUIRE(workspace_floats >= merv_scalar_fused_backward_workspace(E, K), MERV_E_ARG, "merv_scalar_fused_backward: workspace too small");
+  ScalarFusedPtrs p = {};
+  for (int e = 0; e < E; ++e) {
+    MERV_REQUIRE(B == 0 || dw_partial[e], MERV_E_ARG, "merv_scalar_fused_backward: encoder %d: NULL dw_partial", e);
+    p.dw_partial[e] = dw_partial[e];
+    p.bias[e] = bias[e];
+    p.db[e] = db[e];
+  }
+  if (int rc = require_sm100()) return rc;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int nb = (K + 255) / 256;
+  if (dtype == MERV_BF16)
+    scalar_fused_bias_kernel<__nv_bfloat16><<<nb, 256, 0, s>>>(p, gsum, weights, workspace, B, E, K);
+  else
+    scalar_fused_bias_kernel<float><<<nb, 256, 0, s>>>(p, gsum, weights, workspace, B, E, K);
+  scalar_fused_final_kernel<<<1, 256, 0, s>>>(p, workspace, nb, weights, dweights_out, dscalar, B, E);
+  MERV_CUDA_OK(cudaGetLastError());
+  return MERV_OK;
 }
 
 // out = gelu(z) (dy == NULL) or out = dy * gelu'(z); n elements, contiguous, n % (16 / sizeof) == 0

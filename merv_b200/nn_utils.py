@@ -30,8 +30,8 @@ Two execution modes:
   adapter runs the whole path as pool -> [hidden layers] -> scores -> ONE tcgen05 GEMM whose epilogue applies the
   mixing weights, so the per-encoder projections never touch HBM.  Valid whenever the LAST projector layer is
   affine (true for every projector type of the reference).  In grad mode the linear projectors take the same fused
-  forward with a backward that keeps only the pooled tokens (``_FusedLinearFn``) unless FSDP manages a parameter involved;
-  everything else trains through the module-by-module autograd Functions.
+  forward with a backward that keeps only the pooled tokens (``_FusedLinearFn``, or ``_FusedScalarLinearFn`` in front of the
+  scalar mixer) unless FSDP manages a parameter involved; everything else trains through the module-by-module autograd Functions.
 """
 
 from __future__ import annotations
@@ -260,6 +260,38 @@ class _MixFn(torch.autograd.Function):
         return (None, None, *grads, *[g.to(t) for g, t in zip(dVs, vdt)])
 
 
+class _ScalarMixFn(torch.autograd.Function):
+    """ScalarAdapter.forward (nn_utils.py:524-537) with its hand-written backward: w = softmax(scalar) [E] for every video,
+    out = sum_e w_e V_e, returns (out, w[None]).  dV_e = w_e dOut and dscalar = w (.) (g - <w, g>) with
+    g_e = sum_b <dOut[b], V_e[b]> + dW_out[e], in one pass over dOut and the V_e (merv_scalar_mix_backward).  Every V_e is [B, T, K]:
+    the reference stacks them.  The scalar gradient comes back in the parameter's dtype (fp32 master weights under autocast)."""
+
+    @staticmethod
+    def forward(ctx, scalar, dtype, *V):
+        Vc = [v if v.dtype == dtype else v.to(dtype) for v in V]
+        B, T, K = Vc[0].shape
+        E = len(Vc)
+        w, _ = ops.softmax_weights(scalar.detach().float().reshape(1, E))
+        if B > 0:
+            out, _ = ops.softmax_mix(Vc, T, weights=w.expand(B, E).contiguous())
+        else:  # a rank that owns no videos (merv_b200/parallel.py): no mix to launch, the weights still carry a gradient
+            out = torch.empty((0, T, K), dtype=dtype, device=Vc[0].device)
+        ctx.save_for_backward(w, *Vc)
+        ctx.meta = (scalar.dtype, [v.dtype for v in V])
+        return out, w.to(dtype)
+
+    @staticmethod
+    def backward(ctx, dout, dweights):
+        w, *Vc = ctx.saved_tensors
+        sdt, vdt = ctx.meta
+        dt = Vc[0].dtype
+        if dout is None:  # only the mixing weights were used downstream
+            dout = torch.zeros_like(Vc[0])
+        dw = None if dweights is None else dweights.float().reshape(-1).contiguous()
+        dVs, dscalar = ops.scalar_mix_backward(Vc, dout.to(dt), w.reshape(-1), dw)
+        return (dscalar.to(sdt), None, *[g.to(t) for g, t in zip(dVs, vdt)])
+
+
 class _AttentivePoolFn(torch.autograd.Function):
     """AttentivePooler.forward up to (not including) its projector (nn_utils.py:229-237 with CrossAttentionBlock.forward :447-451 and
     CrossAttention.forward :393-412), bf16, with a hand-written backward; the patch features get no gradient (frozen backbones).
@@ -439,6 +471,60 @@ class _FusedLinearFn(torch.autograd.Function):
             dWs.append(ops.gemm_ex(g, Ps.view(B * T, -1), a_t=True, w_t=True))  # dOut^T (w_e (.) P_e) : contraction over the tokens -> [K, C_e]
         _, dbs, dQ, dWq, dWk, dbias = ops.fused_backward(weights, dwo, u, gsum, dw_partials, pbars, Ws, biases, Qc, Wqc, Wkc, bc, dWs)
         grads = [dQ.reshape(1, -1), dWq, dWk, dbias]
+        for e in range(E):
+            grads += [dWs[e], dbs[e]]
+        grads = [gr.to(pd) if gr is not None else None for gr, pd in zip(grads, ctx.param_dtypes)]
+        return (None, None, None, *grads)
+
+
+class _FusedScalarLinearFn(torch.autograd.Function):
+    """Training step of 3d-avg / avg pool + linear projectors + ScalarAdapter through the fused forward (pool -> softmax(scalar) ->
+    merv_fused_linear_mix), with a backward that never materialises the per-encoder projections Y_e or their gradients dV_e.
+
+    backward: per encoder ONE tcgen05 pass over dOut and the pooled tokens P_e (merv_wgrad_video, the same w_e for every video):
+              dW_e = w_e dOut^T P_e and the partials of <dOut[b], Y_e[b] - b_e>;  gsum = colsum_t(dOut);  then merv_scalar_fused_backward:
+              db_e = w_e sum_b gsum[b],  g_e = partials + b_e . sum_b gsum[b] + dW_out[e],  dscalar = w (.) (g - <w, g>).
+    Needs T % 64 == 0 (ScalarAdapter._can_fuse_training); no gradient flows into the patch features (frozen backbones)."""
+
+    @staticmethod
+    def forward(ctx, adapter, projs, xs, scalar, *proj_params):
+        dtype = torch.bfloat16
+        E, B = len(projs), xs[0].shape[0]
+        lasts = [p.layers()[0][0] for p in projs]
+        Ws = [p._cast_cache.get(lin.weight, dtype) for lin, p in zip(lasts, projs)]
+        biases = [p._cast_cache.get(lin.bias, dtype) for lin, p in zip(lasts, projs)]
+        pooled, _ = ops.pool3d(xs, [p.output_frames for p in projs], projs[0].output_size)
+        T, K = pooled[0].shape[1], lasts[0].out_features
+        scores = scalar.detach().float().reshape(1, E).expand(B, E).contiguous()
+        weights, bias_mix = ops.softmax_weights(scores, biases, K)
+        out = ops.fused_linear_mix(pooled, Ws, weights, bias_mix, T)
+        ctx.dims = (B, E, T, K)
+        ctx.param_dtypes = [t.dtype for t in (scalar, *proj_params)]
+        ctx.save_for_backward(weights[0], *pooled, *Ws, *biases)
+        return out.view(B, T, K), weights[:1].to(dtype)
+
+    @staticmethod
+    def backward(ctx, dout, dweights):
+        B, E, T, K = ctx.dims
+        w, *saved = ctx.saved_tensors
+        pooled, Ws, biases = saved[:E], saved[E:2 * E], saved[2 * E:3 * E]
+        dt = Ws[0].dtype
+        if dout is None:  # only the mixing weights were used downstream
+            dout = torch.zeros((B, T, K), dtype=dt, device=w.device)
+        g = dout.reshape(B * T, K)
+        if g.dtype != dt:
+            g = g.to(dt)
+        if g.stride(1) != 1 or g.stride(0) != K:
+            g = g.contiguous()
+        gsum = ops.video_colsum(g.view(B, T, K))
+        dWs, dw_partials = [], []
+        for e in range(E):  # scale stride 0: w_e for every video
+            dW, dwp = ops.wgrad_video(g, pooled[e].reshape(B * T, -1), w[e].expand(B), Ws[e], B)
+            dWs.append(dW)
+            dw_partials.append(dwp)
+        dwo = None if dweights is None else dweights.float().reshape(-1).contiguous()
+        dscalar, dbs = ops.scalar_fused_backward(w, dwo, gsum, dw_partials, biases)
+        grads = [dscalar]
         for e in range(E):
             grads += [dWs[e], dbs[e]]
         grads = [gr.to(pd) if gr is not None else None for gr, pd in zip(grads, ctx.param_dtypes)]
@@ -966,7 +1052,35 @@ class AttentivePooler(TokenResampler):
 
 
 # Adapters here
-class CrossAttentionAdapterLearnableQuery(nn.Module):
+class _LinkedMixer(nn.Module):
+    """When linked projectors hand their input over to a mixer (DeferredProjection) instead of projecting it themselves.  Shared by the
+    mixers that run a fused path: CrossAttentionAdapterLearnableQuery and ScalarAdapter."""
+
+    # True / False force the training step onto / off the fused path (_FusedLinearFn, _FusedScalarLinearFn); None (default) decides per
+    # call: fused unless a parameter involved is managed by FSDP.  The fused path reads every projector's parameters inside the mixer's
+    # forward, and per-projector FSDP units (merv.py:473-485) have resharded them by then; wrap MervFusion as one unit (INTEGRATION.md)
+    # and set True to use it under FSDP.
+    fused_training: Optional[bool] = None
+
+    def _defer_in_grad_mode(self, projector: nn.Module) -> bool:
+        """Whether a linked projector should hand its input over (DeferredProjection) although autograd is recording."""
+        if self.fused_training is not None:
+            return bool(self.fused_training)
+        return not any(_is_sharded_param(p) for m in (self, projector) for p in m.parameters())
+
+    def _may_defer(self, projector: nn.Module) -> bool:
+        """Whether a linked projector hands its input over to this mixer instead of projecting it itself.  The fused pipeline
+        reads the projector's weights inside THIS module's forward, so parameters managed by a different FSDP unit (already
+        resharded by then) rule it out — with or without autograd — unless ``fused_training=True`` states that projectors and
+        mixer share one unit."""
+        if torch.is_grad_enabled():
+            return self._defer_in_grad_mode(projector)
+        if self.fused_training:
+            return True
+        return not any(_is_sharded_param(p) for m in (self, projector) for p in m.parameters())
+
+
+class CrossAttentionAdapterLearnableQuery(_LinkedMixer):
     def __init__(
         self, embed_dim=3072, llm_dim=4098, token_length=8, averagetoken=False, num_encoder=4, positional_embedding=False
     ) -> None:
@@ -992,11 +1106,7 @@ class CrossAttentionAdapterLearnableQuery(nn.Module):
         self._cast_cache = _CastCache()
         self._u_cache = {}
         self._vc_cache = {}
-        # True / False force the training step onto / off the fused path (_FusedLinearFn); None (default) decides per call: fused unless
-        # a parameter involved is managed by FSDP.  The fused path reads every projector's parameters inside THIS module's forward, and
-        # per-projector FSDP units (merv.py:473-485) have resharded them by then; wrap MervFusion as one unit (INTEGRATION.md) and
-        # set True to use it under FSDP.
-        self.fused_training: Optional[bool] = None
+        self.fused_training: Optional[bool] = None  # see _LinkedMixer
 
     def _reset_parameters(self):
         xavier_uniform_(self.Q)
@@ -1103,23 +1213,6 @@ class CrossAttentionAdapterLearnableQuery(nn.Module):
         if len({v.projector.output_size for v in V}) != 1:
             return False
         return all(len(v.projector.layers()) >= 1 for v in V)
-
-    def _defer_in_grad_mode(self, projector: nn.Module) -> bool:
-        """Whether a linked projector should hand its input over (DeferredProjection) although autograd is recording."""
-        if self.fused_training is not None:
-            return bool(self.fused_training)
-        return not any(_is_sharded_param(p) for m in (self, projector) for p in m.parameters())
-
-    def _may_defer(self, projector: nn.Module) -> bool:
-        """Whether a linked projector hands its input over to this adapter instead of projecting it itself.  The fused pipeline
-        reads the projector's weights inside THIS module's forward, so parameters managed by a different FSDP unit (already
-        resharded by then) rule it out — with or without autograd — unless ``fused_training=True`` states that projectors and
-        adapter share one unit."""
-        if torch.is_grad_enabled():
-            return hasattr(self, "_defer_in_grad_mode") and self._defer_in_grad_mode(projector)
-        if self.fused_training:
-            return True
-        return not any(_is_sharded_param(p) for m in (self, projector) for p in m.parameters())
 
     def _can_fuse_training(self, V: Sequence[DeferredProjection]) -> bool:
         """The fused backward (_FusedLinearFn) covers what MERV constructs (merv.py:152-163,214-216): single-Linear projectors with
@@ -1242,20 +1335,26 @@ class CrossAttentionAdapterLearnableQuery(nn.Module):
         self.__dict__.pop("_last_plan", None)
 
 
-class ScalarAdapter(nn.Module):
+class ScalarAdapter(_LinkedMixer):
     """One learnable scalar per encoder, softmax-normalised, the same mix for every video (nn_utils.py:524-537;
-    feature_fusion == "scalar", merv.py:224-225).  Like the reference it always holds 4 scalars."""
+    feature_fusion == "scalar", merv.py:224-225).  Like the reference it always holds 4 scalars.
+
+    Training: linked 3d-avg / avg pools with single-Linear projectors (bf16, T % 64 == 0) take the fused forward with a backward that keeps
+    only the pooled tokens (_FusedScalarLinearFn); everything else trains module by module through _ScalarMixFn.  Whether linked
+    projectors hand their input over at all is _LinkedMixer's policy (``fused_training``)."""
 
     def __init__(self, num_encoder=4) -> None:
         super().__init__()
         self.scalar = torch.nn.Parameter(torch.randn(4))
+        self.fused_training: Optional[bool] = None  # see _LinkedMixer
 
     def forward(self, projected_patch_embeddings):
         V = projected_patch_embeddings
         E = len(V)
         assert E == self.scalar.numel(), f"ScalarAdapter holds {self.scalar.numel()} scalars, got {E} encoders (nn_utils.py:527,535)"
-        if _needs_grad(self, *[v for v in V if isinstance(v, torch.Tensor)]):
-            raise NotImplementedError("the backward of ScalarAdapter is not implemented (SURVEY.md §8 f-4)")
+        proj_params = [t for v in V if isinstance(v, DeferredProjection) for t in v.projector.parameters()]
+        if _needs_grad(self, *[v for v in V if isinstance(v, torch.Tensor)], *proj_params):
+            return self._forward_train(V)
         linked = all(isinstance(v, DeferredProjection) for v in V)
         first = V[0].features if linked else V[0]
         B = first.shape[0]
@@ -1277,6 +1376,34 @@ class ScalarAdapter(nn.Module):
         V = [v if v.dtype == dtype else v.to(dtype) for v in V]
         out, weights = ops.softmax_mix(V, V[0].shape[1], scores=scores)
         return out, weights[:1].to(dtype)
+
+    def _can_fuse_training(self, V) -> bool:
+        """The fused backward (_FusedScalarLinearFn) covers single-Linear projectors with bias on one pooled grid, bf16 compute, token
+        counts that are a multiple of 64 (a k-block of merv_wgrad_video never spans two videos), frozen features, at least one video."""
+        if not all(isinstance(v, DeferredProjection) for v in V) or any(v.dtype != torch.bfloat16 for v in V):
+            return False
+        if len({(v.projector.output_size, v.shape[1]) for v in V}) != 1 or V[0].shape[1] % 64 or V[0].shape[0] == 0:
+            return False
+        for v in V:
+            layers = v.projector.layers()
+            if len(layers) != 1 or layers[0][0].bias is None or v.features.requires_grad:
+                return False
+        return True
+
+    def _forward_train(self, V) -> Tuple[torch.Tensor, torch.Tensor]:
+        if self._can_fuse_training(V):
+            dtype = torch.bfloat16
+            projs = [v.projector for v in V]
+            xs = [v.features.detach() for v in V]
+            xs = [x if x.dtype == dtype else x.to(dtype) for x in xs]
+            xs = [x if _tma_readable(x) else x.contiguous() for x in xs]
+            params = [t for p in projs for t in (p.layers()[0][0].weight, p.layers()[0][0].bias)]
+            return _FusedScalarLinearFn.apply(self, projs, xs, self.scalar, *params)
+        V = [v.materialize() if isinstance(v, DeferredProjection) else v for v in V]
+        if len({tuple(v.shape) for v in V}) != 1:
+            raise ValueError("training the ScalarAdapter needs every encoder at one [B, T, K] shape (the reference stacks them, "
+                             f"nn_utils.py:535), got {[tuple(v.shape) for v in V]}")
+        return _ScalarMixFn.apply(self.scalar, _compute_dtype(V[0]), *V)
 
 
 class ConcatChannelFusion(LinearProjector):
@@ -1374,10 +1501,10 @@ class MervFusion(nn.Module):
         super().__init__()
         self.projectors = nn.ModuleList(projectors)
         self.feature_fusion = feature_fusion
-        if fused_training is not None:  # force the training step onto / off the fused forward + _FusedLinearFn backward (None: automatic)
-            assert not fused_training or (fused and isinstance(feature_fusion, CrossAttentionAdapterLearnableQuery)), \
-                "fused_training needs the linked learnable-query mixer"
-            if isinstance(feature_fusion, CrossAttentionAdapterLearnableQuery):
+        if fused_training is not None:  # force the training step onto / off the fused forward + backward (None: automatic)
+            assert not fused_training or (fused and isinstance(feature_fusion, _LinkedMixer)), \
+                "fused_training needs a linked learnable-query or scalar mixer"
+            if isinstance(feature_fusion, _LinkedMixer):
                 feature_fusion.fused_training = fused_training
         # the parameter-free fusions of merv.py:598-601: "first" (encoder 0 only) and "concat" (token-wise concatenation)
         self.fusion_type = fusion_type
@@ -1531,7 +1658,7 @@ class MervFusion(nn.Module):
         linkable = fused and tokens_resampled and all(isinstance(p, AveragePooling3DProjector) for p in projs) and \
             isinstance(ff, (CrossAttentionAdapterLearnableQuery, ScalarAdapter))
         m = cls(projs, ff, fused=linkable, fusion_type=feature_fusion if ff is None else None,
-                fused_training=fused_training if linkable and isinstance(ff, CrossAttentionAdapterLearnableQuery) else None)
+                fused_training=fused_training if linkable else None)
         m.arch_specifier, m.feature_fusion_type, m.tokens_resampled = arch_specifier, feature_fusion, tokens_resampled
         m.visual_feature_length, m.text_embedding_dim = visual_feature_length, text_embedding_dim
         return m
@@ -1810,6 +1937,6 @@ def patch_merv(vidlm: nn.Module, fused: bool = True, fused_training: Optional[bo
     _extend_fsdp_policy(vidlm, fused_training if fused else None)
     if fused:
         link_fused(new_projs, new_ff)
-        if fused_training is not None and isinstance(new_ff, CrossAttentionAdapterLearnableQuery):
+        if fused_training is not None and isinstance(new_ff, _LinkedMixer):
             new_ff.fused_training = fused_training  # None: per call, fused unless FSDP manages a parameter involved
     return vidlm

@@ -60,6 +60,7 @@ KERNELS_PER_CALL = {
     "merv_cross_attention": 1, "merv_cross_attention_backward": 1, "merv_add_rows": 1, "merv_video_colsum": 1, "merv_pair_dot": 1, "merv_transpose_rowscale": 1, "merv_fused_backward": 10, "merv_wgrad_video": 3,
     "merv_scores_from_tokens_ex": 2, "merv_score_consts": 1, "merv_layernorm": 1, "merv_layernorm_backward": 1, "merv_concat_linear": 1,
     "merv_mix_backward_ex": 10,  # as merv_mix_backward; one more with single-token encoders, one fewer with averagetoken=False
+    "merv_scalar_mix_backward": 2, "merv_scalar_fused_backward": 2,
 }
 
 
@@ -879,3 +880,52 @@ def mix_backward_ex(Vs: Sequence[torch.Tensor], dout: torch.Tensor, weights: tor
               ptr_array([d.data_ptr() for d in dVs]), dQ.data_ptr(), dWq.data_ptr(), dWk.data_ptr(), dbias.data_ptr(), _p(dpe), ws.data_ptr(), n,
               B, E, T, K, embed, dtype_code(dt), _stream())
     return dVs, dQ, dWq, dWk, dbias, dpe
+
+
+def scalar_mix_backward(Vs: Sequence[torch.Tensor], dout: torch.Tensor, weights: torch.Tensor, dweights: Optional[torch.Tensor] = None):
+    """Gradients of ScalarAdapter.forward (include/merv_fusion.h: merv_scalar_mix_backward): V_e and dout [B, T, K] of one shape and dtype,
+    ``weights`` = softmax(scalar) fp32 [E], ``dweights`` fp32 [E] or None (gradient w.r.t. the returned weights).
+    Returns (dV list in the dtype of V, dscalar fp32 [E])."""
+    lib = _lib.load()
+    dev = _require_cuda(*Vs, dout, weights, dweights)
+    B, T, K = dout.shape
+    E, dt = len(Vs), dout.dtype
+    Vs = [v.contiguous() for v in Vs]
+    dout = dout.contiguous()
+    assert all(v.shape == (B, T, K) and v.dtype == dt for v in Vs), "every encoder must have the [B, T, K] shape and dtype of dout"
+    assert weights.dtype == torch.float32 and weights.is_contiguous() and weights.numel() == E
+    assert dweights is None or (dweights.dtype == torch.float32 and dweights.is_contiguous() and dweights.numel() == E)
+    with torch.cuda.device(dev):
+        dVs = [torch.empty_like(v) for v in Vs]
+        dscalar = torch.empty(E, dtype=torch.float32, device=dev)
+        n = lib.merv_scalar_mix_backward_workspace(B, E, K)
+        ws = torch.empty(max(n, 1), dtype=torch.float32, device=dev)
+        _call('merv_scalar_mix_backward', lib.merv_scalar_mix_backward, ptr_array([v.data_ptr() for v in Vs]), dout.data_ptr(), weights.data_ptr(),
+              _p(dweights), ptr_array([d.data_ptr() for d in dVs]), dscalar.data_ptr(), ws.data_ptr(), n, B, E, T, K, dtype_code(dt), _stream())
+    return dVs, dscalar
+
+
+def scalar_fused_backward(weights: torch.Tensor, dweights: Optional[torch.Tensor], gsum: torch.Tensor, dw_partials: Sequence[torch.Tensor],
+                          biases: Sequence[Optional[torch.Tensor]]):
+    """The end of the fused scalar training step (include/merv_fusion.h: merv_scalar_fused_backward): ``weights`` = softmax(scalar) fp32 [E],
+    ``dweights`` fp32 [E] or None, ``gsum`` = video_colsum(dout) [B, K], ``dw_partials[e]`` from wgrad_video of encoder e, ``biases[e]`` [K].
+    Returns (dscalar fp32 [E], [db_e] in the dtype of the biases)."""
+    lib = _lib.load()
+    dev = _require_cuda(weights, dweights, gsum, *dw_partials, *biases)
+    B, K = gsum.shape
+    E = weights.numel()
+    present = [b for b in biases if b is not None]
+    dt = present[0].dtype if present else torch.float32
+    assert weights.dtype == torch.float32 and weights.is_contiguous() and gsum.dtype == torch.float32 and gsum.is_contiguous()
+    assert dweights is None or (dweights.dtype == torch.float32 and dweights.is_contiguous() and dweights.numel() == E)
+    assert len(dw_partials) == E and all(p.is_contiguous() and p.shape == (B, lib.merv_pair_dot_chunks()) for p in dw_partials)
+    assert len(biases) == E and all(b.dtype == dt and b.is_contiguous() and b.numel() == K for b in present)
+    with torch.cuda.device(dev):
+        dscalar = torch.empty(E, dtype=torch.float32, device=dev)
+        dbs = [None if b is None else torch.empty(K, dtype=dt, device=dev) for b in biases]
+        n = lib.merv_scalar_fused_backward_workspace(E, K)
+        ws = torch.empty(max(n, 1), dtype=torch.float32, device=dev)
+        _call('merv_scalar_fused_backward', lib.merv_scalar_fused_backward, weights.data_ptr(), _p(dweights), gsum.data_ptr(),
+              ptr_array([p.data_ptr() for p in dw_partials]), ptr_array([_p(b) for b in biases]), ptr_array([_p(d) for d in dbs]), dscalar.data_ptr(),
+              ws.data_ptr(), n, B, E, K, dtype_code(dt), _stream())
+    return dscalar, dbs
