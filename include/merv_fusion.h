@@ -411,10 +411,23 @@ int merv_cross_attention(const void* q, int64_t ldq, int64_t q_batch_stride, con
 /* Backward of merv_cross_attention on the tensor cores (bf16; n_q <= 64, n_kv <= 256, head_dim % 32 == 0 and <= 128): S and P are
  * recomputed, dP = dO V^T, dS = scale P (.) (dP - rowsum(P (.) dP)), dV = P^T dO, dK = dS^T Q, dQ = dS K — five tcgen05 contractions per
  * (frame, head).  dout [batches, n_q, C] (lddo), dq [batches, n_q, C] (lddq): dQ of EVERY frame (with shared queries, q_batch_stride == 0,
- * the caller sums the frames), dkv [batches * n_kv, 2C] (lddkv) = [dK | dV] in the layout of kv. */
+ * the caller sums the frames), dkv [batches * n_kv, 2C] (lddkv) = [dK | dV] in the layout of kv.  Rows 16-byte aligned.
+ * Same as merv_cross_attention_backward_ex(..., MERV_BF16, NULL, 0, stream): other shapes are rejected. */
 int merv_cross_attention_backward(const void* q, int64_t ldq, int64_t q_batch_stride, const void* kv, int64_t ldkv, const void* dout,
                                   int64_t lddo, void* dq, int64_t lddq, void* dkv, int64_t lddkv, int batches, int n_q, int n_kv,
                                   int heads, int head_dim, float scale, void* stream);
+/* The backward of merv_cross_attention on its whole domain: fp32 or bf16 (`dtype`), any n_q and n_kv, head_dim <= 128 and a multiple of
+ * 8 (bf16) / 4 (fp32), shared or per-entry queries, rows 16-byte aligned; same operands and outputs as above.  bf16 inside the tcgen05
+ * tile (n_q <= 64, n_kv <= 256, head_dim % 32 == 0) runs the tensor-core kernel, bit-identical to merv_cross_attention_backward;
+ * everything else (and every shape under MERV_ATTN_IMPL=simt) runs a CUDA-core kernel: softmax statistics and D = rowsum(P (.) dP)
+ * recomputed in a first sweep over the keys, then a keys-outer sweep; P and every sum in fp32, outputs rounded once; fixed-order
+ * reductions, no atomics, so results are bit-reproducible and a frame's gradients do not depend on the other frames of the call.
+ * workspace: merv_cross_attention_backward_ex_workspace(...) floats (0 when the tcgen05 kernel runs; workspace may then be NULL). */
+size_t merv_cross_attention_backward_ex_workspace(int batches, int n_q, int n_kv, int heads, int head_dim, int dtype);
+int merv_cross_attention_backward_ex(const void* q, int64_t ldq, int64_t q_batch_stride, const void* kv, int64_t ldkv, const void* dout,
+                                     int64_t lddo, void* dq, int64_t lddq, void* dkv, int64_t lddkv, int batches, int n_q, int n_kv,
+                                     int heads, int head_dim, float scale, int dtype, float* workspace, size_t workspace_floats,
+                                     void* stream);
 int merv_add_rows(const void* a, int64_t lda, const void* b, int64_t ldb, void* out, int64_t ldo, int64_t M, int C, int period, int dtype,
                   void* stream);
 

@@ -109,6 +109,9 @@ _SIGNATURES = {
                                      c_void_p]),
     "merv_cross_attention_backward": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64,
                                               c_int, c_int, c_int, c_int, c_int, c_float, c_void_p]),
+    "merv_cross_attention_backward_ex_workspace": (c_size_t, [c_int, c_int, c_int, c_int, c_int, c_int]),
+    "merv_cross_attention_backward_ex": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p,
+                                                 c_int64, c_int, c_int, c_int, c_int, c_int, c_float, c_int, c_void_p, c_size_t, c_void_p]),
     "merv_add_rows": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int64, c_int, c_int, c_int, c_void_p]),
     "merv_video_colsum": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int64, c_int64, c_float, c_int, c_void_p]),
     "merv_pair_dot_chunks": (c_int, []),

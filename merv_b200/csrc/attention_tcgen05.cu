@@ -586,9 +586,17 @@ int launch_attention_bwd_tcgen05(const void* q, long long ldq, long long q_batch
   return MERV_OK;
 }
 
-bool attention_tcgen05_supported(int n_q, int n_kv, int heads, int hd, long long ldq, long long q_batch_stride, long long ldkv, long long ldo) {
+static bool attention_simt_forced() {
   const char* e = getenv("MERV_ATTN_IMPL");
-  if (e != nullptr && strcmp(e, "simt") == 0) return false;
+  return e != nullptr && strcmp(e, "simt") == 0;
+}
+
+bool attention_bwd_tcgen05_supported(int n_q, int n_kv, int hd) {
+  return !attention_simt_forced() && n_q <= AB_ROWS && n_kv <= AT_KEYS && hd % 32 == 0 && hd <= AT_MAX_HD;
+}
+
+bool attention_tcgen05_supported(int n_q, int n_kv, int heads, int hd, long long ldq, long long q_batch_stride, long long ldkv, long long ldo) {
+  if (attention_simt_forced()) return false;
   (void)heads;
   return n_q <= AT_M && n_kv <= AT_KEYS && hd % 32 == 0 && hd <= AT_MAX_HD && ldq % 8 == 0 && ldkv % 8 == 0 && ldo % 8 == 0 && q_batch_stride % 8 == 0;
 }

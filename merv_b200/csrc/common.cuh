@@ -71,6 +71,9 @@ int launch_scores_softmax_weights(const float* const* partial, const int32_t* co
 bool attention_tcgen05_supported(int n_q, int n_kv, int heads, int hd, long long ldq, long long q_batch_stride, long long ldkv, long long ldo);
 int launch_attention_tcgen05(const void* q, long long ldq, long long q_batch_stride, const void* kv, long long ldkv, void* out, long long ldo,
                              int batches, int n_q, int n_kv, int heads, int hd, float scale, cudaStream_t stream);
+// the tcgen05 backward's tile: bf16, n_q <= 64, n_kv <= 256, head_dim % 32 == 0 and <= 128 (false under MERV_ATTN_IMPL=simt).  Row
+// alignment is not part of it: both backward kernels require 16-byte aligned rows.
+bool attention_bwd_tcgen05_supported(int n_q, int n_kv, int hd);
 int launch_attention_bwd_tcgen05(const void* q, long long ldq, long long q_batch_stride, const void* kv, long long ldkv, const void* dout, long long lddo,
                                  void* dq, long long lddq, void* dkv, long long lddkv, int batches, int n_q, int n_kv, int heads, int hd, float scale,
                                  cudaStream_t stream);

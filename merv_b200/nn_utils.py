@@ -10,7 +10,7 @@ error behaviour as the reference (paths below are relative to the reference root
     get_mlp_projector                    merv/util/nn_utils.py:111-121
     TokenResampler                       merv/util/nn_utils.py:124-133
     AveragePoolingProjector              merv/util/nn_utils.py:136-174    (2-D "avg")
-    AttentivePooler (+ CrossAttention, MLP, CrossAttentionBlock containers)   merv/util/nn_utils.py:177-246,380-452  ("attntv", inference)
+    AttentivePooler (+ CrossAttention, MLP, CrossAttentionBlock containers)   merv/util/nn_utils.py:177-246,380-452  ("attntv", fp32 / bf16 training)
     AveragePooling3DProjector            merv/util/nn_utils.py:306-338
     Convolutional3DProjector             merv/util/nn_utils.py:341-377    ("3dconv": 27 displaced poolings + one GEMM on the pooled grid)
     CrossAttentionAdapterLearnableQuery  merv/util/nn_utils.py:455-521    (averagetoken either way, positional embedding)
@@ -107,6 +107,23 @@ def _needs_grad(module: nn.Module, *tensors) -> bool:
     )
 
 
+def _linear_wgrad(g: torch.Tensor, x: torch.Tensor) -> torch.Tensor:
+    """dW = g^T x of a Linear (g [M, N], x [M, K] -> [N, K]), a contraction over the tokens.  bf16: the tensor cores read both operands
+    MN-major in place; fp32 (the parity path, SIMT GEMM, K-major) transposes them first."""
+    if g.dtype == torch.bfloat16:
+        return ops.gemm_ex(g, x, a_t=True, w_t=True)
+    dW, _ = ops.linear_bias_act(ops.transpose(g, pad=True), ops.transpose(x, pad=True), None, ACT_NONE)  # [N, M] x [K, M]^T
+    return dW
+
+
+def _linear_dgrad(g: torch.Tensor, w: torch.Tensor) -> torch.Tensor:
+    """dX = g W of a Linear (g [M, N], W [N, K] -> [M, K]); bf16 reads W MN-major in place, fp32 transposes it."""
+    if g.dtype == torch.bfloat16:
+        return ops.gemm_ex(g, w, w_t=True)
+    dx, _ = ops.linear_bias_act(g, ops.transpose(w), None, ACT_NONE)  # [M, N] x [K, N]^T
+    return dx
+
+
 class _ProjectorFn(torch.autograd.Function):
     """[LayerNorm ->] Linear / gelu-mlp / fused-gelu-mlp projector (nn_utils.py:22-108) with a hand-written backward.
 
@@ -168,19 +185,11 @@ class _ProjectorFn(torch.autograd.Function):
         for i in reversed(range(n)):
             if zs[i] is not None:
                 g = ops.gelu(zs[i].reshape(g.shape), g)  # dZ_i
-            x2 = xs[i].reshape(-1, xs[i].shape[-1])
-            tc = g.dtype == torch.bfloat16  # tensor cores read dZ, X and W MN-major in place; the fp32 parity path (SIMT, K-major) transposes
-            if tc:
-                dW = ops.gemm_ex(g, x2, a_t=True, w_t=True)  # dW_i = dZ_i^T X_i: contraction over the tokens
-            else:
-                dW, _ = ops.linear_bias_act(ops.transpose(g, pad=True), ops.transpose(x2, pad=True), None, ACT_NONE)  # [N, M] x [K, M]^T -> [N, K]
+            dW = _linear_wgrad(g, xs[i].reshape(-1, xs[i].shape[-1]))  # dW_i = dZ_i^T X_i
             grads[off + 2 * i] = dW.to(ctx.param_dtypes[off + 2 * i])
             grads[off + 2 * i + 1] = ops.colsum(g).to(ctx.param_dtypes[off + 2 * i + 1])
             if i > 0 or need_dx or has_ln:
-                if tc:
-                    g = ops.gemm_ex(g, ws[i], w_t=True)  # dX_i = dZ_i W_i
-                else:
-                    g, _ = ops.linear_bias_act(g, ops.transpose(ws[i]), None, ACT_NONE)  # [M, N] x [K, N]^T -> [M, K]
+                g = _linear_dgrad(g, ws[i])  # dX_i = dZ_i W_i
         dx = g if need_dx else None
         if has_ln:
             x_in, gamma = saved[-2], saved[-1]
@@ -215,10 +224,7 @@ class _ConvTapsFn(torch.autograd.Function):
             g = g.to(A2.dtype)
         if g.stride(1) != 1:
             g = g.contiguous()
-        if g.dtype == torch.bfloat16:
-            dW2 = ops.gemm_ex(g, A2, a_t=True, w_t=True)
-        else:
-            dW2, _ = ops.linear_bias_act(ops.transpose(g, pad=True), ops.transpose(A2, pad=True), None, ACT_NONE)
+        dW2 = _linear_wgrad(g, A2)
         K, C = ctx.wshape[0], ctx.wshape[1]
         dW = dW2.reshape(K, 3, 3, 3, C).permute(0, 4, 1, 2, 3).to(ctx.wdtype)  # back to Conv3d's [K, C, kf, kh, kw]
         db = None if ctx.bdtype is None else ops.colsum(g).to(ctx.bdtype)
@@ -294,17 +300,19 @@ class _ScalarMixFn(torch.autograd.Function):
 
 class _AttentivePoolFn(torch.autograd.Function):
     """AttentivePooler.forward up to (not including) its projector (nn_utils.py:229-237 with CrossAttentionBlock.forward :447-451 and
-    CrossAttention.forward :393-412), bf16, with a hand-written backward; the patch features get no gradient (frozen backbones).
+    CrossAttention.forward :393-412) in the compute dtype (fp32 or bf16), with a hand-written backward; the patch features get no
+    gradient (frozen backbones).
 
-    forward : xn = LN1(x);  kv = xn Wkv^T + bkv;  qp = qt Wq^T + bq;  a = attention(qp, kv) (tcgen05);  y = a Wp^T + bp;  q1 = y + qt;
+    forward : xn = LN1(x);  kv = xn Wkv^T + bkv;  qp = qt Wq^T + bq;  a = attention(qp, kv);  y = a Wp^T + bp;  q1 = y + qt;
               hn = LN2(q1);  z1 = hn W1^T + b1;  g1 = gelu(z1);  h2 = g1 W2^T + b2;  q2 = q1 + h2
-    backward: every Linear through the MN-major tcgen05 GEMM (dW = dY^T X, dX = dY W, no transposed copies), the attention through
-              merv_cross_attention_backward (five tcgen05 contractions per frame and head), LayerNorm / GELU / reductions through their
-              HBM-bound kernels.  The learned queries are shared by all frames: their gradient sums the frames."""
+    backward: every Linear as dW = dY^T X and dX = dY W (_linear_wgrad / _linear_dgrad: the MN-major tcgen05 GEMM in bf16, the SIMT GEMM
+              on transposed copies in fp32), the attention through merv_cross_attention_backward_ex (five tcgen05 contractions per frame
+              and head for bf16 frames inside its tile, the CUDA-core kernel for every other shape and for fp32), LayerNorm / GELU /
+              reductions through their HBM-bound kernels.  The learned queries are shared by all frames: their gradient sums the frames."""
 
     @staticmethod
-    def forward(ctx, x, cache, heads, scale, eps1, eps2, qt3, g1w, g1b, Wkv, bkv, Wq, bq, Wp, bp, g2w, g2b, W1, b1, W2, b2):
-        dt = torch.bfloat16
+    def forward(ctx, x, dtype, cache, heads, scale, eps1, eps2, qt3, g1w, g1b, Wkv, bkv, Wq, bq, Wp, bp, g2w, g2b, W1, b1, W2, b2):
+        dt = dtype
         c = cache
         B, F, N, C_ = x.shape
         n = qt3.shape[1]
@@ -332,33 +340,33 @@ class _AttentivePoolFn(torch.autograd.Function):
     def backward(ctx, dq2):
         heads, scale, eps1, eps2, (B, F, N, C_, n), pdt = ctx.meta
         xf, xn, kv, qp, a2, q1, hn, z1, g1, qt, g1wc, Wkvc, Wqc, Wpc, g2wc, W1c, W2c = ctx.saved_tensors
-        dt = torch.bfloat16
+        dt = xf.dtype
         g = dq2.reshape(-1, C_)
         g = (g if g.dtype == dt else g.to(dt)).contiguous()
         BF = B * F
         # q2 = q1 + fc2(gelu(fc1(LN2(q1))))
-        dW2 = ops.gemm_ex(g, g1, a_t=True, w_t=True)
+        dW2 = _linear_wgrad(g, g1)
         db2 = ops.colsum(g)
-        dz1 = ops.gelu(z1, ops.gemm_ex(g, W2c, w_t=True))
-        dW1 = ops.gemm_ex(dz1, hn, a_t=True, w_t=True)
+        dz1 = ops.gelu(z1, _linear_dgrad(g, W2c))
+        dW1 = _linear_wgrad(dz1, hn)
         db1 = ops.colsum(dz1)
-        dq1_ln, dg2w, dg2b = ops.layernorm_backward([q1], ops.gemm_ex(dz1, W1c, w_t=True), g2wc, eps2)
+        dq1_ln, dg2w, dg2b = ops.layernorm_backward([q1], _linear_dgrad(dz1, W1c), g2wc, eps2)
         dq1 = ops.add_rows(g, dq1_ln)
         # q1 = proj(attention) + query tokens (the same tokens for every frame)
         dqt = ops.video_colsum(dq1.view(1, BF, n * C_)).view(n, C_)  # fp32
-        dWp = ops.gemm_ex(dq1, a2, a_t=True, w_t=True)
+        dWp = _linear_wgrad(dq1, a2)
         dbp = ops.colsum(dq1)
-        da = ops.gemm_ex(dq1, Wpc, w_t=True)
+        da = _linear_dgrad(dq1, Wpc)
         dq_frames, dkv = ops.cross_attention_backward(qp, kv, da.view(BF, n, C_), BF, heads, scale)
         dqp = ops.video_colsum(dq_frames.view(1, BF, n * C_)).view(n, C_).to(dt)
-        dWq = ops.gemm_ex(dqp, qt, a_t=True, w_t=True)
+        dWq = _linear_wgrad(dqp, qt)
         dbq = ops.colsum(dqp)
-        dqt = dqt + ops.gemm_ex(dqp, Wqc, w_t=True).float()
-        dWkv = ops.gemm_ex(dkv, xn, a_t=True, w_t=True)
+        dqt = dqt + _linear_dgrad(dqp, Wqc).float()
+        dWkv = _linear_wgrad(dkv, xn)
         dbkv = ops.colsum(dkv)
-        _, dg1w, dg1b = ops.layernorm_backward([xf], ops.gemm_ex(dkv, Wkvc, w_t=True), g1wc, eps1, need_dx=False)
+        _, dg1w, dg1b = ops.layernorm_backward([xf], _linear_dgrad(dkv, Wkvc), g1wc, eps1, need_dx=False)
         grads = [dqt.view(1, n, C_), dg1w, dg1b, dWkv, dbkv, dWq, dbq, dWp, dbp, dg2w, dg2b, dW1, db1, dW2, db2]
-        return (None, None, None, None, None, None, *[gr.to(t) for gr, t in zip(grads, pdt)])
+        return (None, None, None, None, None, None, None, *[gr.to(t) for gr, t in zip(grads, pdt)])
 
 
 def _version(p: torch.Tensor) -> int:
@@ -950,8 +958,9 @@ class AttentivePooler(TokenResampler):
     Same constructor signature, module tree (hence state-dict keys: ``query_tokens``, ``cross_attn.{norm1,xattn.{q,kv,proj},norm2,
     mlp.{fc1,fc2}}``, ``projector.*``) and initialisation sequence as the reference.  forward: LayerNorm (merv_layernorm), the kv / proj /
     MLP / projector Linears on the tcgen05 GEMM (GELU in the epilogue), merv_cross_attention (both contractions as tcgen05.mma in bf16),
-    merv_add_rows for the two residuals.  Training (bf16 compute): _AttentivePoolFn, a hand-written backward whose attention part runs
-    five tcgen05 contractions per frame and head (merv_cross_attention_backward)."""
+    merv_add_rows for the two residuals.  Training, in fp32 or bf16 compute, wherever the forward runs: _AttentivePoolFn, a hand-written
+    backward whose attention part is merv_cross_attention_backward_ex (five tcgen05 contractions per frame and head for bf16 frames of
+    at most 64 queries and 256 keys with head_dim % 32 == 0, the CUDA-core kernel otherwise)."""
 
     def __init__(self, fused_vision_dim: int, llm_dim: int, num_query_tokens: int, num_heads: int = 8, output_frames: int = 8,
                  mlp_type: str = "gelu-mlp") -> None:
@@ -1014,15 +1023,12 @@ class AttentivePooler(TokenResampler):
         if _needs_grad(self, x):
             if x.requires_grad:
                 raise NotImplementedError("gradients w.r.t. the patch features are not implemented (frozen backbones, merv.py:316)")
-            if dtype != torch.bfloat16:
-                raise NotImplementedError("training the attentive pooler needs bf16 compute (torch.autocast): its attention backward runs on the "
-                                          "tensor cores only")
             lins = (att.kv, att.q, att.proj, blk.mlp.fc1, blk.mlp.fc2)
             if any(l.bias is None for l in lins) or any(ln.weight is None or ln.bias is None for ln in (blk.norm1, blk.norm2)):
                 raise NotImplementedError("bias-free layers / non-affine LayerNorms of the attentive pooler are not covered by the backward")
             xb = x.detach()
             xb = xb if xb.dtype == dtype else xb.to(dtype)
-            q2 = _AttentivePoolFn.apply(xb, c, att.num_heads, att.scale, blk.norm1.eps, blk.norm2.eps, self.query_tokens, blk.norm1.weight,
+            q2 = _AttentivePoolFn.apply(xb, dtype, c, att.num_heads, att.scale, blk.norm1.eps, blk.norm2.eps, self.query_tokens, blk.norm1.weight,
                                         blk.norm1.bias, att.kv.weight, att.kv.bias, att.q.weight, att.q.bias, att.proj.weight, att.proj.bias,
                                         blk.norm2.weight, blk.norm2.bias, blk.mlp.fc1.weight, blk.mlp.fc1.bias, blk.mlp.fc2.weight, blk.mlp.fc2.bias)
             out = self.projector(q2)

@@ -61,6 +61,7 @@ KERNELS_PER_CALL = {
     "merv_scores_from_tokens_ex": 2, "merv_score_consts": 1, "merv_layernorm": 1, "merv_layernorm_backward": 1, "merv_concat_linear": 1,
     "merv_mix_backward_ex": 10,  # as merv_mix_backward; one more with single-token encoders, one fewer with averagetoken=False
     "merv_scalar_mix_backward": 2, "merv_scalar_fused_backward": 2,
+    "merv_cross_attention_backward_ex": 1,
 }
 
 
@@ -655,12 +656,14 @@ def cross_attention(q: torch.Tensor, kv: torch.Tensor, batches: int, heads: int,
 
 def cross_attention_backward(q: torch.Tensor, kv: torch.Tensor, dout: torch.Tensor, batches: int, heads: int,
                              scale: Optional[float] = None) -> Tuple[torch.Tensor, torch.Tensor]:
-    """Gradients of `cross_attention` (bf16, tensor cores): returns (dq [batches, n_q, C] — one dQ per batch entry, to be summed by the
-    caller when the queries are shared — and dkv [batches * n_kv, 2C] = [dK | dV])."""
+    """Gradients of `cross_attention`, fp32 or bf16, on every shape it runs: returns (dq [batches, n_q, C] — one dQ per batch entry, to
+    be summed by the caller when the queries are shared — and dkv [batches * n_kv, 2C] = [dK | dV]) in the input dtype.  bf16 frames
+    inside the tcgen05 tile take the tensor-core kernel, everything else the CUDA-core one (merv_cross_attention_backward_ex)."""
     lib = _lib.load()
     dev = _require_cuda(q, kv, dout)
     C_ = q.shape[-1]
-    assert q.dtype == torch.bfloat16 and kv.dtype == torch.bfloat16 and dout.dtype == torch.bfloat16, "the attention backward is bf16 only"
+    dt = q.dtype
+    assert dt in (torch.float32, torch.bfloat16) and kv.dtype == dt and dout.dtype == dt
     assert kv.dim() == 2 and kv.shape[1] == 2 * C_ and kv.shape[0] % max(batches, 1) == 0 and C_ % heads == 0
     n_q, n_kv, hd = q.shape[-2], kv.shape[0] // max(batches, 1), C_ // heads
     assert dout.shape == (batches, n_q, C_)
@@ -668,12 +671,15 @@ def cross_attention_backward(q: torch.Tensor, kv: torch.Tensor, dout: torch.Tens
     kv = kv if kv.stride(1) == 1 else kv.contiguous()
     dout = dout.contiguous()
     qbs = 0 if q.dim() == 2 else q.stride(0)
+    code = dtype_code(dt)
     with torch.cuda.device(dev):
-        dq = torch.empty((batches, n_q, C_), dtype=torch.bfloat16, device=dev)
-        dkv = torch.empty((batches * n_kv, 2 * C_), dtype=torch.bfloat16, device=dev)
-        _call('merv_cross_attention_backward', lib.merv_cross_attention_backward, q.data_ptr(), q.stride(-2), qbs, kv.data_ptr(), kv.stride(0),
-              dout.data_ptr(), dout.stride(1), dq.data_ptr(), dq.stride(1), dkv.data_ptr(), dkv.stride(0), batches, n_q, n_kv, heads, hd,
-              float(hd ** -0.5 if scale is None else scale), _stream())
+        dq = torch.empty((batches, n_q, C_), dtype=dt, device=dev)
+        dkv = torch.empty((batches * n_kv, 2 * C_), dtype=dt, device=dev)
+        n = lib.merv_cross_attention_backward_ex_workspace(batches, n_q, n_kv, heads, hd, code)
+        ws = torch.empty(n, dtype=torch.float32, device=dev) if n else None
+        _call('merv_cross_attention_backward_ex', lib.merv_cross_attention_backward_ex, q.data_ptr(), q.stride(-2), qbs, kv.data_ptr(),
+              kv.stride(0), dout.data_ptr(), dout.stride(1), dq.data_ptr(), dq.stride(1), dkv.data_ptr(), dkv.stride(0), batches, n_q, n_kv,
+              heads, hd, float(hd ** -0.5 if scale is None else scale), code, _p(ws), n, _stream())
     return dq, dkv
 
 
