@@ -185,6 +185,12 @@ int merv_scores_softmax_weights(const float* const* partial, const int32_t* coun
  * output; otherwise `weights` is an input. */
 int merv_softmax_mix(const void* const* V, const int32_t* tokens, const float* scores, float* weights, void* out,
                      int B, int E, int T, int K, int dtype, void* stream);
+/* merv_softmax_mix writing video b's fused tokens at out + b * out_batch_stride, rows ldo apart: the prefix slot of the
+ * [B, bos + T + L_text, K] multimodal embedding buffer that MERV.forward otherwise builds with torch.cat (merv.py:633-640).  Writes
+ * nothing outside the [B, T, K] block.  ldo and out_batch_stride whole 16-byte vectors (MERV_E_ALIGN), ldo >= K and
+ * out_batch_stride >= T * ldo (MERV_E_SHAPE).  merv_softmax_mix is this call with ldo = K, out_batch_stride = T * K (bit-identical). */
+int merv_softmax_mix_ex(const void* const* V, const int32_t* tokens, const float* scores, float* weights, void* out, int64_t ldo,
+                        int64_t out_batch_stride, int B, int E, int T, int K, int dtype, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * Fused affine path (the shipped "3davg+linear" + "cross_attention_avg_lq" configuration):
@@ -311,6 +317,15 @@ int merv_mix_backward_ex(const void* const* V, const int32_t* tokens, const void
                          const void* Q, const void* Wq, const void* Wk, const void* in_proj_bias, void* const* dV, void* dQ,
                          void* dWq, void* dWk, void* dbias, void* dpe, float* workspace, size_t workspace_floats, int B, int E,
                          int T, int K, int embed, int dtype, void* stream);
+/* merv_mix_backward_ex reading dOut in place from a batch-strided slot: video b's rows start at dOut + b * dout_batch_stride, rows lddo
+ * apart (the gradient of the prefix slot of the multimodal embedding buffer), in every pass that reads it; dV stays contiguous.  dOut
+ * 16-byte aligned, lddo and dout_batch_stride whole 16-byte vectors (MERV_E_ALIGN), lddo >= K and dout_batch_stride >= T * lddo
+ * (MERV_E_SHAPE).  merv_mix_backward_ex is this call with lddo = K, dout_batch_stride = T * K (the same kernels, bit-identical). */
+int merv_mix_backward_strided(const void* const* V, const int32_t* tokens, const void* dOut, int64_t lddo, int64_t dout_batch_stride,
+                              const float* weights, const float* dweights_out, const float* u, int64_t u_token_stride, const void* pe, int64_t ldpe,
+                              const void* Q, const void* Wq, const void* Wk, const void* in_proj_bias, void* const* dV, void* dQ, void* dWq,
+                              void* dWk, void* dbias, void* dpe, float* workspace, size_t workspace_floats, int B, int E, int T, int K, int embed,
+                              int dtype, void* stream);
 /* Gradients of ScalarAdapter.forward (feature_fusion == "scalar", nn_utils.py:524-537): w = softmax(scalar) [E] for every video,
  * out = sum_e w_e V_e, returned weights w[None].  With dweights_out [E] the gradient of the returned weights:
  *     dV_e = w_e dOut,   g_e = sum_b <dOut[b], V_e[b]> + dweights_out[e],   dscalar = w (.) (g - <w, g>)
@@ -321,6 +336,11 @@ int merv_mix_backward_ex(const void* const* V, const int32_t* tokens, const void
 size_t merv_scalar_mix_backward_workspace(int B, int E, int K);
 int merv_scalar_mix_backward(const void* const* V, const void* dOut, const float* weights, const float* dweights_out, void* const* dV,
                              float* dscalar, float* workspace, size_t workspace_floats, int B, int E, int T, int K, int dtype, void* stream);
+/* merv_scalar_mix_backward with dOut read in place from a batch-strided slot (rows lddo apart, videos dout_batch_stride apart; checks as for
+ * merv_mix_backward_strided); V_e and dV_e stay contiguous.  merv_scalar_mix_backward is this call with lddo = K, dout_batch_stride = T * K. */
+int merv_scalar_mix_backward_strided(const void* const* V, const void* dOut, int64_t lddo, int64_t dout_batch_stride, const float* weights,
+                                     const float* dweights_out, void* const* dV, float* dscalar, float* workspace, size_t workspace_floats, int B,
+                                     int E, int T, int K, int dtype, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * Backward of the FUSED path (linear projectors linked to the adapter, forward = merv_fused_linear_mix): the training step of
@@ -382,6 +402,13 @@ size_t merv_wgrad_video_workspace(int videos, int N_out, int C);
 int merv_wgrad_video(const void* dY, int64_t lddy, const void* X, int64_t ldx, const float* scale, int64_t scale_stride, const void* W,
                      int64_t ldw, void* dW, int64_t lddw, float* dot_partial, float* workspace, int videos, int tokens_per_video, int N_out,
                      int C, void* stream);
+/* merv_wgrad_video with dY video b's rows at dY + b * dy_batch_stride (rows lddy apart): the gradient of the prefix slot of the multimodal
+ * embedding buffer read in place by a 3-D TMA map (N_out columns, token in video, video).  dY 16-byte aligned, lddy and dy_batch_stride
+ * multiples of 8 (MERV_E_ALIGN), dy_batch_stride >= tokens_per_video * lddy (MERV_E_SHAPE).  With dy_batch_stride = tokens_per_video * lddy
+ * it is merv_wgrad_video (the same kernel, bit-identical); other strides run a separate instantiation doing the same reductions. */
+int merv_wgrad_video_ex(const void* dY, int64_t lddy, int64_t dy_batch_stride, const void* X, int64_t ldx, const float* scale, int64_t scale_stride,
+                        const void* W, int64_t ldw, void* dW, int64_t lddw, float* dot_partial, float* workspace, int videos, int tokens_per_video,
+                        int N_out, int C, void* stream);
 size_t merv_fused_backward_workspace(const merv_fused_bwd_desc* desc);
 int merv_fused_backward(const merv_fused_bwd_desc* desc, int dtype, void* stream);
 /* The same fused training step in front of the ScalarAdapter (one w [E] for every video, no query vector).  Per encoder,

@@ -119,6 +119,8 @@ _SIGNATURES = {
     "merv_wgrad_video_workspace": (c_size_t, [c_int, c_int, c_int]),
     "merv_wgrad_video": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p,
                                  c_int, c_int, c_int, c_int, c_void_p]),
+    "merv_wgrad_video_ex": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p,
+                                    c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "merv_pair_dot": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int64, c_int, c_void_p]),
     "merv_pair_dot_scale": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int, c_int64, c_int, c_void_p]),
     "merv_transpose_rowscale": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int64, c_int64, c_void_p, c_int64, c_int, c_int, c_void_p]),
@@ -134,13 +136,20 @@ _SIGNATURES = {
     "merv_mix_backward_ex": (c_int, [_PP, POINTER(c_int32), c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p,
                                      c_void_p, c_void_p, _PP, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int, c_int,
                                      c_int, c_int, c_int, c_int, c_void_p]),
+    "merv_mix_backward_strided": (c_int, [_PP, POINTER(c_int32), c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64,
+                                          c_void_p, c_void_p, c_void_p, c_void_p, _PP, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                          c_size_t, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "merv_scalar_mix_backward_workspace": (c_size_t, [c_int, c_int, c_int]),
     "merv_scalar_mix_backward": (c_int, [_PP, c_void_p, c_void_p, c_void_p, _PP, c_void_p, c_void_p, c_size_t, c_int, c_int, c_int, c_int, c_int,
                                          c_void_p]),
+    "merv_scalar_mix_backward_strided": (c_int, [_PP, c_void_p, c_int64, c_int64, c_void_p, c_void_p, _PP, c_void_p, c_void_p, c_size_t, c_int, c_int,
+                                                 c_int, c_int, c_int, c_void_p]),
     "merv_scalar_fused_backward_workspace": (c_size_t, [c_int, c_int]),
     "merv_scalar_fused_backward": (c_int, [c_void_p, c_void_p, c_void_p, _PP, _PP, _PP, c_void_p, c_void_p, c_size_t, c_int, c_int, c_int, c_int,
                                            c_void_p]),
     "merv_softmax_mix": (c_int, [_PP, POINTER(c_int32), c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "merv_softmax_mix_ex": (c_int, [_PP, POINTER(c_int32), c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_int, c_int, c_int,
+                                    c_void_p]),
     "merv_fused_linear_mix": (c_int, [_PP, POINTER(c_int64), _PP, POINTER(c_int64), POINTER(c_int32), c_int, c_void_p, c_void_p,
                                       c_void_p, c_int64, c_int64, c_int, c_int, c_int, c_int, c_void_p]),
 }

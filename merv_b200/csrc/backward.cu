@@ -91,8 +91,9 @@ struct BwdPtrs {
 // vbar = V_e[b,0], and are kept for its dV (written by the CTAs of encoder gsum_e, the first single-token one).
 constexpr int kMixRedCols = 8;  // 16-byte vectors per CTA
 template <typename T>
-__global__ void __launch_bounds__(256) mix_bwd_reduce_kernel(const __grid_constant__ BwdPtrs p, const T* __restrict__ dOut, float* __restrict__ dw_partial,
-                                                             float* __restrict__ vbar, float* __restrict__ gsum, int gsum_e, int E, int Ttok, int K) {
+__global__ void __launch_bounds__(256) mix_bwd_reduce_kernel(const __grid_constant__ BwdPtrs p, const T* __restrict__ dOut, long long ldg, long long gbs,
+                                                             float* __restrict__ dw_partial, float* __restrict__ vbar, float* __restrict__ gsum, int gsum_e,
+                                                             int E, int Ttok, int K) {
   constexpr int VEC = Vec16<T>::kN;
   __shared__ float part[32][kMixRedCols * VEC + 1];
   __shared__ float red[32];
@@ -104,12 +105,12 @@ __global__ void __launch_bounds__(256) mix_bwd_reduce_kernel(const __grid_consta
 #pragma unroll
     for (int c = 0; c < VEC; ++c) gs[c] = 0.f;
     if (k0 < K) {
-      const T* g = dOut + (long long)b * Ttok * K + k0;
+      const T* g = dOut + (long long)b * gbs + k0;
       int t = rg;
       for (; t + 96 < Ttok; t += 128) {
         uint4 rd[4];
 #pragma unroll
-        for (int i = 0; i < 4; ++i) rd[i] = ldg_nc_v4(g + (long long)(t + 32 * i) * K);
+        for (int i = 0; i < 4; ++i) rd[i] = ldg_nc_v4(g + (long long)(t + 32 * i) * ldg);
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
           float d[VEC];
@@ -120,7 +121,7 @@ __global__ void __launch_bounds__(256) mix_bwd_reduce_kernel(const __grid_consta
       }
       for (; t < Ttok; t += 32) {
         float d[VEC];
-        Vec16<T>::unpack(ldg_nc_v4(g + (long long)t * K), d);
+        Vec16<T>::unpack(ldg_nc_v4(g + (long long)t * ldg), d);
 #pragma unroll
         for (int c = 0; c < VEC; ++c) gs[c] += d[c];
       }
@@ -150,14 +151,14 @@ __global__ void __launch_bounds__(256) mix_bwd_reduce_kernel(const __grid_consta
   for (int c = 0; c < VEC; ++c) vs[c] = 0.f;
   if (k0 < K) {
     const T* v = static_cast<const T*>(p.V[e]) + (long long)b * Ttok * K + k0;
-    const T* g = dOut + (long long)b * Ttok * K + k0;
+    const T* g = dOut + (long long)b * gbs + k0;
     int t = rg;
     for (; t + 96 < Ttok; t += 128) {
       uint4 ra[4], rd[4];
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
         ra[i] = ldg_nc_v4(v + (long long)(t + 32 * i) * K);
-        rd[i] = ldg_nc_v4(g + (long long)(t + 32 * i) * K);
+        rd[i] = ldg_nc_v4(g + (long long)(t + 32 * i) * ldg);
       }
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
@@ -174,7 +175,7 @@ __global__ void __launch_bounds__(256) mix_bwd_reduce_kernel(const __grid_consta
     for (; t < Ttok; t += 32) {
       float a[VEC], d[VEC];
       Vec16<T>::unpack(ldg_nc_v4(v + (long long)t * K), a);
-      Vec16<T>::unpack(ldg_nc_v4(g + (long long)t * K), d);
+      Vec16<T>::unpack(ldg_nc_v4(g + (long long)t * ldg), d);
 #pragma unroll
       for (int c = 0; c < VEC; ++c) {
         vs[c] += a[c];
@@ -214,8 +215,9 @@ __global__ void __launch_bounds__(32) mix_bwd_scores_kernel(const float* __restr
 
 // ---- stage 3: dV_e[b,t,:] = w[b,e] dOut[b,t,:] + (ds[b,e] / T) u  for the encoders in full_mask (the T-token ones) --------------
 template <typename T, int E>
-__global__ void __launch_bounds__(256) mix_bwd_dv_kernel(const __grid_constant__ BwdPtrs p, const T* __restrict__ dOut, const float* __restrict__ weights,
-                                                         const float* __restrict__ ds, const float* __restrict__ u, int Ttok, int K, unsigned full_mask) {
+__global__ void __launch_bounds__(256) mix_bwd_dv_kernel(const __grid_constant__ BwdPtrs p, const T* __restrict__ dOut, long long ldg, long long gbs,
+                                                         const float* __restrict__ weights, const float* __restrict__ ds, const float* __restrict__ u,
+                                                         int Ttok, int K, unsigned full_mask) {
   constexpr int VEC = Vec16<T>::kN;
   const int b = blockIdx.y;
   float w[E], s[E];
@@ -226,11 +228,12 @@ __global__ void __launch_bounds__(256) mix_bwd_dv_kernel(const __grid_constant__
   }
   const int kvec = K / VEC;
   const long long nvec = (long long)Ttok * kvec;
-  const T* g = dOut + (long long)b * Ttok * K;
+  const T* g = dOut + (long long)b * gbs;
   for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < nvec; i += (long long)gridDim.x * 256) {
-    const int kc = int(i % kvec) * VEC;
+    const long long t = i / kvec;
+    const int kc = int(i - t * kvec) * VEC;
     float d[VEC], uu[VEC];
-    Vec16<T>::unpack(ldg_nc_v4(g + i * VEC), d);
+    Vec16<T>::unpack(ldg_nc_v4(g + t * ldg + kc), d);
 #pragma unroll
     for (int c = 0; c < VEC; c += 4) {
       const float4 u4 = __ldg(reinterpret_cast<const float4*>(u + kc + c));
@@ -253,15 +256,16 @@ __global__ void __launch_bounds__(256) mix_bwd_dv_kernel(const __grid_constant__
 // du needs ds, hence the second read of V; a thread owns one 16-byte column vector of one token for ALL videos, so du is summed in a fixed
 // order (videos, then encoders) in registers and written once: no atomics, no [B, T*K] partials.
 template <typename T, int E>
-__global__ void __launch_bounds__(256) mix_bwd_dv_flat_kernel(const __grid_constant__ BwdPtrs p, const T* __restrict__ dOut, const float* __restrict__ weights,
-                                                              const float* __restrict__ ds, const float* __restrict__ u, float* __restrict__ du, int B,
-                                                              int Ttok, int K, unsigned full_mask) {
+__global__ void __launch_bounds__(256) mix_bwd_dv_flat_kernel(const __grid_constant__ BwdPtrs p, const T* __restrict__ dOut, long long ldg, long long gbs,
+                                                              const float* __restrict__ weights, const float* __restrict__ ds, const float* __restrict__ u,
+                                                              float* __restrict__ du, int B, int Ttok, int K, unsigned full_mask) {
   constexpr int VEC = Vec16<T>::kN;
   const int kvec = K / VEC;
   const long long nvec = (long long)Ttok * kvec;
   const long long vstride = (long long)Ttok * K;
   for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < nvec; i += (long long)gridDim.x * 256) {
-    const int kc = int(i % kvec) * VEC;
+    const long long t = i / kvec;
+    const int kc = int(i - t * kvec) * VEC;
     float uu[VEC], acc[VEC];
 #pragma unroll
     for (int c = 0; c < VEC; c += 4) {
@@ -272,7 +276,7 @@ __global__ void __launch_bounds__(256) mix_bwd_dv_flat_kernel(const __grid_const
     for (int c = 0; c < VEC; ++c) acc[c] = 0.f;
     for (int b = 0; b < B; ++b) {
       float d[VEC];
-      Vec16<T>::unpack(ldg_nc_v4(dOut + b * vstride + i * VEC), d);
+      Vec16<T>::unpack(ldg_nc_v4(dOut + b * gbs + t * ldg + kc), d);
 #pragma unroll
       for (int e = 0; e < E; ++e) {
         const float w = __ldg(weights + (long long)b * E + e), s = __ldg(ds + (long long)b * E + e);
@@ -451,8 +455,8 @@ __global__ void __launch_bounds__(256) gelu_kernel(const T* __restrict__ z, cons
 }
 
 template <typename T>
-static int launch_mix_dv(const BwdPtrs& p, const void* dOut, const float* weights, const float* ds, const float* u, int B, int E, int Ttok, int K,
-                         unsigned full_mask, cudaStream_t s) {
+static int launch_mix_dv(const BwdPtrs& p, const void* dOut, long long ldg, long long gbs, const float* weights, const float* ds, const float* u, int B,
+                         int E, int Ttok, int K, unsigned full_mask, cudaStream_t s) {
   constexpr int VEC = Vec16<T>::kN;
   const long long nvec = (long long)Ttok * (K / VEC);
   long long gx = (nvec + 255) / 256;
@@ -461,7 +465,7 @@ static int launch_mix_dv(const BwdPtrs& p, const void* dOut, const float* weight
   dim3 grid((unsigned)gx, B);
   const T* g = static_cast<const T*>(dOut);
   switch (E) {
-#define MERV_DV_CASE(n) case n: mix_bwd_dv_kernel<T, n><<<grid, 256, 0, s>>>(p, g, weights, ds, u, Ttok, K, full_mask); break;
+#define MERV_DV_CASE(n) case n: mix_bwd_dv_kernel<T, n><<<grid, 256, 0, s>>>(p, g, ldg, gbs, weights, ds, u, Ttok, K, full_mask); break;
     MERV_DV_CASE(1) MERV_DV_CASE(2) MERV_DV_CASE(3) MERV_DV_CASE(4) MERV_DV_CASE(5) MERV_DV_CASE(6) MERV_DV_CASE(7) MERV_DV_CASE(8)
 #undef MERV_DV_CASE
     default: return fail(MERV_E_ARG, "merv_mix_backward: E=%d", E);
@@ -471,8 +475,8 @@ static int launch_mix_dv(const BwdPtrs& p, const void* dOut, const float* weight
 }
 
 template <typename T>
-static int launch_mix_dv_flat(const BwdPtrs& p, const void* dOut, const float* weights, const float* ds, const float* u, float* du, int B, int E,
-                              int Ttok, int K, unsigned full_mask, cudaStream_t s) {
+static int launch_mix_dv_flat(const BwdPtrs& p, const void* dOut, long long ldg, long long gbs, const float* weights, const float* ds, const float* u,
+                              float* du, int B, int E, int Ttok, int K, unsigned full_mask, cudaStream_t s) {
   constexpr int VEC = Vec16<T>::kN;
   const long long nvec = (long long)Ttok * (K / VEC);
   long long gx = (nvec + 255) / 256;
@@ -480,7 +484,7 @@ static int launch_mix_dv_flat(const BwdPtrs& p, const void* dOut, const float* w
   if (gx > cap) gx = cap;
   const T* g = static_cast<const T*>(dOut);
   switch (E) {
-#define MERV_DV_CASE(n) case n: mix_bwd_dv_flat_kernel<T, n><<<(unsigned)gx, 256, 0, s>>>(p, g, weights, ds, u, du, B, Ttok, K, full_mask); break;
+#define MERV_DV_CASE(n) case n: mix_bwd_dv_flat_kernel<T, n><<<(unsigned)gx, 256, 0, s>>>(p, g, ldg, gbs, weights, ds, u, du, B, Ttok, K, full_mask); break;
     MERV_DV_CASE(1) MERV_DV_CASE(2) MERV_DV_CASE(3) MERV_DV_CASE(4) MERV_DV_CASE(5) MERV_DV_CASE(6) MERV_DV_CASE(7) MERV_DV_CASE(8)
 #undef MERV_DV_CASE
     default: return fail(MERV_E_ARG, "merv_mix_backward_ex: E=%d", E);
@@ -502,8 +506,8 @@ static int launch_mix_dv_flat(const BwdPtrs& p, const void* dOut, const float* w
 //      every dV_e vector written once, (1 + 2E) B T K elements in all.  Two tokens per iteration keep 2 (1 + E) independent 16-byte loads
 //      in flight per thread.  The dots are reduced in a fixed order (warp butterfly, then the 8 warps in order) into partial[b, e, kb].
 template <typename T, int E>
-__global__ void __launch_bounds__(256) scalar_mix_bwd_kernel(const __grid_constant__ BwdPtrs p, const T* __restrict__ dOut, const float* __restrict__ weights,
-                                                             float* __restrict__ partial, int Ttok, int K) {
+__global__ void __launch_bounds__(256) scalar_mix_bwd_kernel(const __grid_constant__ BwdPtrs p, const T* __restrict__ dOut, long long ldg, long long gbs,
+                                                             const float* __restrict__ weights, float* __restrict__ partial, int Ttok, int K) {
   constexpr int VEC = Vec16<T>::kN;
   __shared__ float red[E][8];
   const int kb = blockIdx.x, b = blockIdx.y;
@@ -517,7 +521,7 @@ __global__ void __launch_bounds__(256) scalar_mix_bwd_kernel(const __grid_consta
   }
   if (k0 < K) {
     const long long base = (long long)b * Ttok * K + k0;
-    const T* g = dOut + base;
+    const T* g = dOut + (long long)b * gbs + k0;
     const T* vb[E];
     T* db[E];
 #pragma unroll
@@ -531,7 +535,7 @@ __global__ void __launch_bounds__(256) scalar_mix_bwd_kernel(const __grid_consta
 #pragma unroll
       for (int i = 0; i < 2; ++i) {
         const long long off = (long long)(t + 32 * i) * K;
-        rd[i] = ldg_nc_v4(g + off);
+        rd[i] = ldg_nc_v4(g + (long long)(t + 32 * i) * ldg);
 #pragma unroll
         for (int e = 0; e < E; ++e) rv[i][e] = ldg_nc_v4(vb[e] + off);
       }
@@ -557,7 +561,7 @@ __global__ void __launch_bounds__(256) scalar_mix_bwd_kernel(const __grid_consta
     for (; t < Ttok; t += 32) {
       const long long off = (long long)t * K;
       float d[VEC];
-      Vec16<T>::unpack(ldg_nc_v4(g + off), d);
+      Vec16<T>::unpack(ldg_nc_v4(g + (long long)t * ldg), d);
 #pragma unroll
       for (int e = 0; e < E; ++e) {
         float a[VEC], o[VEC];
@@ -631,12 +635,12 @@ __global__ void __launch_bounds__(256) scalar_mix_fold_kernel(const float* __res
 }
 
 template <typename T>
-static int launch_scalar_mix_bwd(const BwdPtrs& p, const void* dOut, const float* weights, float* partial, int B, int E, int Ttok, int K,
-                                 int kblocks, cudaStream_t s) {
+static int launch_scalar_mix_bwd(const BwdPtrs& p, const void* dOut, long long ldg, long long gbs, const float* weights, float* partial, int B, int E,
+                                 int Ttok, int K, int kblocks, cudaStream_t s) {
   dim3 grid(kblocks, B);
   const T* g = static_cast<const T*>(dOut);
   switch (E) {
-#define MERV_SCALAR_CASE(n) case n: scalar_mix_bwd_kernel<T, n><<<grid, 256, 0, s>>>(p, g, weights, partial, Ttok, K); break;
+#define MERV_SCALAR_CASE(n) case n: scalar_mix_bwd_kernel<T, n><<<grid, 256, 0, s>>>(p, g, ldg, gbs, weights, partial, Ttok, K); break;
     MERV_SCALAR_CASE(1) MERV_SCALAR_CASE(2) MERV_SCALAR_CASE(3) MERV_SCALAR_CASE(4) MERV_SCALAR_CASE(5) MERV_SCALAR_CASE(6) MERV_SCALAR_CASE(7)
     MERV_SCALAR_CASE(8)
 #undef MERV_SCALAR_CASE
@@ -1152,11 +1156,14 @@ extern "C" size_t merv_mix_backward_ex_workspace(int B, int E, int T, int K, int
 //   u_token_stride == 0 : averagetoken=True,  u fp32 [K],    s_e = u . (mean_t V_e + pe[e])     (pe [E, K] (ldpe) or NULL)
 //   u_token_stride == K : averagetoken=False, u fp32 [T*K],  s_e = sum_t u[t,:] . V_e[b,t,:]    (pe must be NULL; Wk is [embed, T*K])
 // Outputs: dV_e [B, T_e, K], dQ [embed], dWq [embed, embed], dWk [embed, T*K or K], dbias [3 * embed] and, with pe, dpe [E, K] (all `dtype`).
+// dOut video b's rows start at dOut + b * dout_batch_stride, rows lddo apart (the prefix slot of the multimodal embedding buffer's gradient, read
+// in place); dV stays contiguous.  lddo == K, dout_batch_stride == T * K is merv_mix_backward_ex: the same kernels, bit-identical gradients.
 // The T-token-only, stride-0, pe-less call is merv_mix_backward: the same kernels, bit-identical gradients.
-extern "C" int merv_mix_backward_ex(const void* const* V, const int32_t* tokens, const void* dOut, const float* weights, const float* dweights_out,
-                                    const float* u, int64_t u_token_stride, const void* pe, int64_t ldpe, const void* Q, const void* Wq, const void* Wk,
-                                    const void* in_proj_bias, void* const* dV, void* dQ, void* dWq, void* dWk, void* dbias, void* dpe, float* workspace,
-                                    size_t workspace_floats, int B, int E, int T, int K, int embed, int dtype, void* stream) {
+extern "C" int merv_mix_backward_strided(const void* const* V, const int32_t* tokens, const void* dOut, int64_t lddo, int64_t dout_batch_stride,
+                                         const float* weights, const float* dweights_out, const float* u, int64_t u_token_stride, const void* pe,
+                                         int64_t ldpe, const void* Q, const void* Wq, const void* Wk, const void* in_proj_bias, void* const* dV, void* dQ,
+                                         void* dWq, void* dWk, void* dbias, void* dpe, float* workspace, size_t workspace_floats, int B, int E, int T,
+                                         int K, int embed, int dtype, void* stream) {
   MERV_REQUIRE(dtype == MERV_F32 || dtype == MERV_BF16, MERV_E_DTYPE, "merv_mix_backward_ex: unknown dtype %d", dtype);
   MERV_REQUIRE(V && tokens && dOut && weights && u && Q && Wq && Wk && dV && dQ && dWq && dWk && dbias && workspace, MERV_E_ARG,
                "merv_mix_backward_ex: NULL pointer");
@@ -1164,6 +1171,12 @@ extern "C" int merv_mix_backward_ex(const void* const* V, const int32_t* tokens,
   MERV_REQUIRE(B > 0 && T > 0 && K > 0 && embed > 0, MERV_E_SHAPE, "merv_mix_backward_ex: B=%d T=%d K=%d embed=%d", B, T, K, embed);
   const int vec = dtype == MERV_BF16 ? 8 : 4;
   MERV_REQUIRE(K % vec == 0, MERV_E_SHAPE, "merv_mix_backward_ex: K=%d must be a multiple of %d", K, vec);
+  MERV_REQUIRE(aligned16(dOut) && lddo % vec == 0 && dout_batch_stride % vec == 0, MERV_E_ALIGN,
+               "merv_mix_backward_strided: dOut must be 16-byte aligned and lddo=%lld / dout_batch_stride=%lld whole 16-byte vectors",
+               (long long)lddo, (long long)dout_batch_stride);
+  MERV_REQUIRE(lddo >= K && dout_batch_stride >= (int64_t)T * lddo, MERV_E_SHAPE,
+               "merv_mix_backward_strided: lddo=%lld < K or dout_batch_stride=%lld < T * lddo (rows or videos would overlap)", (long long)lddo,
+               (long long)dout_batch_stride);
   const bool flat = u_token_stride != 0;
   MERV_REQUIRE(!flat || u_token_stride == K, MERV_E_SHAPE, "merv_mix_backward_ex: u_token_stride=%lld (0 or K=%d)", (long long)u_token_stride, K);
   MERV_REQUIRE(!flat || (long long)T * K <= 0x7fffffffLL, MERV_E_SHAPE, "merv_mix_backward_ex: T*K overflows");
@@ -1200,13 +1213,13 @@ extern "C" int merv_mix_backward_ex(const void* const* V, const int32_t* tokens,
   const float rs = 1.0f / sqrtf(float(embed));
   const long long nWk = (long long)embed * Ku, nWq = (long long)embed * embed;
 #define MERV_MIX_BWD_BODY(T_)                                                                                                                      \
-  mix_bwd_reduce_kernel<T_><<<dim3(kblocks, E, B), 256, 0, s>>>(p, (const T_*)dOut, dw_partial, vbar, gsum, gsum_e, E, T, K);                     \
+  mix_bwd_reduce_kernel<T_><<<dim3(kblocks, E, B), 256, 0, s>>>(p, (const T_*)dOut, lddo, dout_batch_stride, dw_partial, vbar, gsum, gsum_e, E, T, K); \
   mix_bwd_scores_kernel<<<B, 32, 0, s>>>(dw_partial, weights, dweights_out, ds, E, kblocks);                                                       \
   if (flat) {                                                                                                                                      \
-    if (int rc = launch_mix_dv_flat<T_>(p, dOut, weights, ds, u, du, B, E, T, K, full_mask, s)) return rc;                                         \
+    if (int rc = launch_mix_dv_flat<T_>(p, dOut, lddo, dout_batch_stride, weights, ds, u, du, B, E, T, K, full_mask, s)) return rc;                \
   } else {                                                                                                                                         \
     if (full_mask != 0) {                                                                                                                          \
-      if (int rc = launch_mix_dv<T_>(p, dOut, weights, ds, u, B, E, T, K, full_mask, s)) return rc;                                                \
+      if (int rc = launch_mix_dv<T_>(p, dOut, lddo, dout_batch_stride, weights, ds, u, B, E, T, K, full_mask, s)) return rc;                       \
     }                                                                                                                                              \
     if (pe != nullptr)                                                                                                                             \
       du_pe_kernel<T_><<<(K + 255) / 256, 256, 0, s>>>(ds, vbar, (const T_*)pe, ldpe, u, du, (T_*)dpe, B, E, K);                                   \
@@ -1229,6 +1242,14 @@ extern "C" int merv_mix_backward_ex(const void* const* V, const int32_t* tokens,
 #undef MERV_MIX_BWD_BODY
   MERV_CUDA_OK(cudaGetLastError());
   return MERV_OK;
+}
+
+extern "C" int merv_mix_backward_ex(const void* const* V, const int32_t* tokens, const void* dOut, const float* weights, const float* dweights_out,
+                                    const float* u, int64_t u_token_stride, const void* pe, int64_t ldpe, const void* Q, const void* Wq, const void* Wk,
+                                    const void* in_proj_bias, void* const* dV, void* dQ, void* dWq, void* dWk, void* dbias, void* dpe, float* workspace,
+                                    size_t workspace_floats, int B, int E, int T, int K, int embed, int dtype, void* stream) {
+  return merv_mix_backward_strided(V, tokens, dOut, K, (int64_t)T * K, weights, dweights_out, u, u_token_stride, pe, ldpe, Q, Wq, Wk, in_proj_bias, dV,
+                                   dQ, dWq, dWk, dbias, dpe, workspace, workspace_floats, B, E, T, K, embed, dtype, stream);
 }
 
 // V_e [B, T, K] (all encoders must have T tokens), dOut [B, T, K], weights fp32 [B, E] (forward output), u fp32 [K];
@@ -1258,11 +1279,12 @@ extern "C" size_t merv_scalar_mix_backward_workspace(int B, int E, int K) {
   return (size_t)B * E * ((K + kMixRedCols * 4 - 1) / (kMixRedCols * 4));
 }
 
-// V_e, dOut, dV_e [B, T, K] contiguous (`dtype`), weights = softmax(scalar) fp32 [E], dweights_out fp32 [E] or NULL, dscalar fp32 [E].
-// B == 0 (a rank without videos) reads no tensor and gives dscalar from dweights_out alone.
-extern "C" int merv_scalar_mix_backward(const void* const* V, const void* dOut, const float* weights, const float* dweights_out, void* const* dV,
-                                        float* dscalar, float* workspace, size_t workspace_floats, int B, int E, int T, int K, int dtype,
-                                        void* stream) {
+// V_e, dV_e [B, T, K] contiguous (`dtype`), dOut [B, T, K] with rows lddo apart and videos dout_batch_stride apart, weights = softmax(scalar)
+// fp32 [E], dweights_out fp32 [E] or NULL, dscalar fp32 [E].  B == 0 (a rank without videos) reads no tensor and gives dscalar from dweights_out
+// alone.  lddo == K, dout_batch_stride == T * K is merv_scalar_mix_backward (the same kernels, bit-identical).
+extern "C" int merv_scalar_mix_backward_strided(const void* const* V, const void* dOut, int64_t lddo, int64_t dout_batch_stride, const float* weights,
+                                                const float* dweights_out, void* const* dV, float* dscalar, float* workspace, size_t workspace_floats,
+                                                int B, int E, int T, int K, int dtype, void* stream) {
   MERV_REQUIRE(dtype == MERV_F32 || dtype == MERV_BF16, MERV_E_DTYPE, "merv_scalar_mix_backward: unknown dtype %d", dtype);
   MERV_REQUIRE(V && dV && weights && dscalar, MERV_E_ARG, "merv_scalar_mix_backward: NULL pointer");
   MERV_REQUIRE(E >= 1 && E <= MERV_MAX_ENCODERS, MERV_E_ARG, "merv_scalar_mix_backward: E=%d not in [1,%d]", E, MERV_MAX_ENCODERS);
@@ -1272,7 +1294,12 @@ extern "C" int merv_scalar_mix_backward(const void* const* V, const void* dOut, 
   BwdPtrs p = {};
   if (B > 0) {
     MERV_REQUIRE(dOut && workspace, MERV_E_ARG, "merv_scalar_mix_backward: NULL pointer");
-    MERV_REQUIRE(aligned16(dOut), MERV_E_ALIGN, "merv_scalar_mix_backward: dOut must be 16-byte aligned");
+    MERV_REQUIRE(aligned16(dOut) && lddo % vec == 0 && dout_batch_stride % vec == 0, MERV_E_ALIGN,
+                 "merv_scalar_mix_backward: dOut must be 16-byte aligned and lddo=%lld / dout_batch_stride=%lld whole 16-byte vectors", (long long)lddo,
+                 (long long)dout_batch_stride);
+    MERV_REQUIRE(lddo >= K && dout_batch_stride >= (int64_t)T * lddo, MERV_E_SHAPE,
+                 "merv_scalar_mix_backward_strided: lddo=%lld < K or dout_batch_stride=%lld < T * lddo (rows or videos would overlap)", (long long)lddo,
+                 (long long)dout_batch_stride);
     for (int e = 0; e < E; ++e) {
       MERV_REQUIRE(V[e] && dV[e], MERV_E_ARG, "merv_scalar_mix_backward: encoder %d: NULL pointer", e);
       MERV_REQUIRE(aligned16(V[e]) && aligned16(dV[e]), MERV_E_ALIGN, "merv_scalar_mix_backward: encoder %d: tensor not 16-byte aligned", e);
@@ -1287,13 +1314,20 @@ extern "C" int merv_scalar_mix_backward(const void* const* V, const void* dOut, 
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const int kblocks = (K / vec + kMixRedCols - 1) / kMixRedCols;
   if (B > 0) {
-    const int rc = dtype == MERV_BF16 ? launch_scalar_mix_bwd<__nv_bfloat16>(p, dOut, weights, workspace, B, E, T, K, kblocks, s)
-                                      : launch_scalar_mix_bwd<float>(p, dOut, weights, workspace, B, E, T, K, kblocks, s);
+    const int rc = dtype == MERV_BF16 ? launch_scalar_mix_bwd<__nv_bfloat16>(p, dOut, lddo, dout_batch_stride, weights, workspace, B, E, T, K, kblocks, s)
+                                      : launch_scalar_mix_bwd<float>(p, dOut, lddo, dout_batch_stride, weights, workspace, B, E, T, K, kblocks, s);
     if (rc) return rc;
   }
   scalar_mix_fold_kernel<<<1, 256, 0, s>>>(workspace, weights, dweights_out, dscalar, B, E, kblocks);
   MERV_CUDA_OK(cudaGetLastError());
   return MERV_OK;
+}
+
+extern "C" int merv_scalar_mix_backward(const void* const* V, const void* dOut, const float* weights, const float* dweights_out, void* const* dV,
+                                        float* dscalar, float* workspace, size_t workspace_floats, int B, int E, int T, int K, int dtype,
+                                        void* stream) {
+  return merv_scalar_mix_backward_strided(V, dOut, K, (int64_t)T * K, weights, dweights_out, dV, dscalar, workspace, workspace_floats, B, E, T, K, dtype,
+                                          stream);
 }
 
 extern "C" size_t merv_scalar_fused_backward_workspace(int E, int K) {
@@ -1416,10 +1450,18 @@ extern "C" size_t merv_wgrad_video_workspace(int videos, int N_out, int C) {
   return dots + (split > 1 ? (size_t)split * N_out * C : 0);
 }
 
-extern "C" int merv_wgrad_video(const void* dY, int64_t lddy, const void* X, int64_t ldx, const float* scale, int64_t scale_stride, const void* W,
-                                int64_t ldw, void* dW, int64_t lddw, float* dot_partial, float* workspace, int videos, int tokens_per_video,
-                                int N_out, int C, void* stream) {
+// dY video b's rows start at dY + b * dy_batch_stride (rows lddy apart): the gradient of the prefix slot of the [B, L + T, N_out] multimodal
+// embedding buffer is read in place.  dy_batch_stride == tokens_per_video * lddy is merv_wgrad_video (the same kernel, bit-identical).
+extern "C" int merv_wgrad_video_ex(const void* dY, int64_t lddy, int64_t dy_batch_stride, const void* X, int64_t ldx, const float* scale,
+                                   int64_t scale_stride, const void* W, int64_t ldw, void* dW, int64_t lddw, float* dot_partial, float* workspace,
+                                   int videos, int tokens_per_video, int N_out, int C, void* stream) {
   MERV_REQUIRE(dY && X && W && dW && dot_partial && workspace, MERV_E_ARG, "merv_wgrad_video: NULL pointer");
+  MERV_REQUIRE(aligned16(dY) && lddy % 8 == 0 && dy_batch_stride % 8 == 0, MERV_E_ALIGN,
+               "merv_wgrad_video_ex: dY must be 16-byte aligned and lddy=%lld / dy_batch_stride=%lld multiples of 8 elements", (long long)lddy,
+               (long long)dy_batch_stride);
+  MERV_REQUIRE(dy_batch_stride >= (int64_t)tokens_per_video * lddy, MERV_E_SHAPE,
+               "merv_wgrad_video_ex: dy_batch_stride=%lld < tokens_per_video * lddy = %lld (videos would overlap)", (long long)dy_batch_stride,
+               (long long)tokens_per_video * lddy);
   MERV_REQUIRE(videos >= 0 && tokens_per_video > 0 && N_out > 0 && C > 0, MERV_E_SHAPE, "merv_wgrad_video: videos=%d tokens=%d N_out=%d C=%d", videos,
                tokens_per_video, N_out, C);
   MERV_REQUIRE(tokens_per_video % 64 == 0, MERV_E_SHAPE, "merv_wgrad_video: tokens_per_video=%d must be a multiple of 64 (one k-block never spans two videos)",
@@ -1437,7 +1479,8 @@ extern "C" int merv_wgrad_video(const void* dY, int64_t lddy, const void* X, int
   dots = (dots + 3) / 4 * 4;
   float* partial = split > 1 ? workspace + dots : nullptr;
   MERV_REQUIRE(aligned16(workspace), MERV_E_ALIGN, "merv_wgrad_video: workspace must be 16-byte aligned");
-  WgradVideoArgs vid = {videos, tokens_per_video / 64, scale, scale_stride, W, ldw, workspace, split, partial};
+  const bool packed = dy_batch_stride == (int64_t)tokens_per_video * lddy;  // the 2-D map of the contiguous case
+  WgradVideoArgs vid = {videos, tokens_per_video / 64, scale, scale_stride, W, ldw, workspace, split, partial, packed ? 0 : (long long)dy_batch_stride};
   if (int rc = launch_gemm_tcgen05(&seg, 1, nullptr, nullptr, N_out, nullptr, MERV_ACT_NONE, nullptr, nullptr, dW, lddw, 0, N_out, C, 0, s, nullptr, 0,
                                    false, nullptr, nullptr, &vid))
     return rc;
@@ -1449,6 +1492,13 @@ extern "C" int merv_wgrad_video(const void* dY, int64_t lddy, const void* X, int
   fold_partials_kernel<<<videos, 32, 0, s>>>(workspace, dot_partial, wgrad_video_parts(N_out, C));
   MERV_CUDA_OK(cudaGetLastError());
   return MERV_OK;
+}
+
+extern "C" int merv_wgrad_video(const void* dY, int64_t lddy, const void* X, int64_t ldx, const float* scale, int64_t scale_stride, const void* W,
+                                int64_t ldw, void* dW, int64_t lddw, float* dot_partial, float* workspace, int videos, int tokens_per_video,
+                                int N_out, int C, void* stream) {
+  return merv_wgrad_video_ex(dY, lddy, (int64_t)tokens_per_video * lddy, X, ldx, scale, scale_stride, W, ldw, dW, lddw, dot_partial, workspace, videos,
+                             tokens_per_video, N_out, C, stream);
 }
 
 extern "C" int merv_pair_dot_scale(const void* x, const void* y, float* partial, const float* scale, int64_t scale_stride, void* y_scaled, int B,

@@ -42,6 +42,7 @@ struct WgradVideoArgs {
   float* dot_out;          // [videos, wgrad_video_parts(M, N)]
   int split;               // work items per tile: the videos in `split` contiguous ranges (1: no split, the result goes straight to Y)
   float* partial;          // [split, M, N] fp32 when split > 1
+  long long dy_batch_stride;  // 0: the videos' rows of dY (the A operand) follow each other; else video b's rows start at A + b * dy_batch_stride
 };
 int wgrad_video_parts(int M, int N);
 int wgrad_video_split(int M, int N, int videos);  // the split that fills the SMs best (1 if nothing is gained)

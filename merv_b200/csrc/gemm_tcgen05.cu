@@ -129,7 +129,9 @@ struct TensorMaps {
 // long; a lone thread sustains roughly one instruction per 4 cycles, a k-block lasts ~560, and the CTA PAIR (whose two producers feed
 // one MMA stream) ran 35 % SLOWER than the single CTA on MN-major operands — on K-major ones too when sent through that code
 // (scripts/gpu_mn_pair_lab.py).
-template <int kCtas, bool kWide, bool kGelu, int kMaj, bool kAssist, bool kVid = false>
+// kDy3 (kVid only): the A operand (dY, MN-major) is a 3-D map (N_out columns, token in video, video), so video b's rows may start at any
+// 16-byte aligned batch stride — the gradient of a prefix slot inside the [B, L + T, N] multimodal embedding buffer, read in place.
+template <int kCtas, bool kWide, bool kGelu, int kMaj, bool kAssist, bool kVid = false, bool kDy3 = false>
 __device__ __forceinline__ void gemm_body(const TensorMaps& maps, const GemmParams& p, const AssistArgs* ap) {
   using C = Cfg<kCtas, kWide, kAssist>;
   constexpr int STAGES = C::STAGES, STAGE_BYTES = C::STAGE_BYTES, RING_BYTES = C::RING_BYTES;
@@ -253,6 +255,13 @@ __device__ __forceinline__ void gemm_body(const TensorMaps& maps, const GemmPara
             // are kept in L2 preferentially (for the 4096 x 16384 second MLP layer they barely fit: 134 of 126 MB)
             if (!a_mn) {
               load(&maps.a[s], sa, kb * BK, m0, L2_EVICT_NORMAL);
+            } else if constexpr (kDy3) {  // video s0's k-block (a k-block never spans two videos) at its own batch stride
+              const int t0 = (kb - s0 * nkb) * BK;
+#pragma unroll
+              for (int j = 0; j < BM / 64; ++j) {
+                if constexpr (kCtas == 2) tma_load_3d_pair(&maps.a[s], bar, sa + j * MN_CHUNK_BYTES, m0 + 64 * j, t0, s0, L2_EVICT_NORMAL);
+                else tma_load_3d(&maps.a[s], bar, sa + j * MN_CHUNK_BYTES, m0 + 64 * j, t0, s0, L2_EVICT_NORMAL);
+              }
             } else {  // A given as [K, M]: one [64 m x BK k] box per 64 rows of the tile
 #pragma unroll
               for (int j = 0; j < BM / 64; ++j) load(&maps.a[s], sa + j * MN_CHUNK_BYTES, m0 + 64 * j, kb * BK, L2_EVICT_NORMAL);
@@ -543,6 +552,13 @@ gemm_wgrad_video_tcgen05_kernel(const __grid_constant__ TensorMaps maps, const _
   gemm_body<kCtas, false, false, 3, false, true>(maps, p, nullptr);
 }
 
+// the same with dY read through the 3-D (batch-strided) map: a separate kernel, so the contiguous one above keeps its code
+template <int kCtas>
+__global__ void __launch_bounds__(GEMM_THREADS, 1)
+gemm_wgrad_video_strided_tcgen05_kernel(const __grid_constant__ TensorMaps maps, const __grid_constant__ GemmParams p) {
+  gemm_body<kCtas, false, false, 3, false, true, true>(maps, p, nullptr);
+}
+
 // the fused forward GEMM (CTA pair, K-major operands) whose two spare warps pool the videos ahead of the tiles (pool_assist.cuh)
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_pool_assist_tcgen05_kernel(const __grid_constant__ TensorMaps maps, const __grid_constant__ GemmParams p,
@@ -744,6 +760,16 @@ int launch_gemm_tcgen05(const GemmSegment* seg, int nseg, const float* seg_scale
     MERV_REQUIRE(vid->split >= 1 && vid->split <= vid->videos && (vid->split == 1 || (vid->partial != nullptr && aligned16(vid->partial) && N % 4 == 0)), MERV_E_ARG,
                  "gemm: per-video weight gradient: split=%d of %d videos needs a 16-byte aligned partial buffer", vid->split, vid->videos);
     p.vid_parts = vid->split; p.vid_partial = vid->partial;
+    if (vid->dy_batch_stride != 0) {  // dY as (N_out columns, token in video, video); same [64 x BK] boxes and swizzle as the 2-D map
+      const long long tpv = (long long)vid->kblocks_per_video * BK;
+      MERV_REQUIRE(vid->dy_batch_stride % 8 == 0 && vid->dy_batch_stride >= tpv * seg[0].lda, MERV_E_SHAPE,
+                   "gemm: per-video weight gradient: dY batch stride %lld must be a multiple of 8 and >= %lld", vid->dy_batch_stride, tpv * seg[0].lda);
+      const unsigned long long dims[3] = {(unsigned long long)M, (unsigned long long)tpv, (unsigned long long)vid->videos};
+      const unsigned long long strides[2] = {(unsigned long long)seg[0].lda * 2, (unsigned long long)vid->dy_batch_stride * 2};
+      const unsigned box[3] = {64u, (unsigned)BK, 1u};
+      if (int rc = encode_tmap_cached(&maps.a[0], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, seg[0].A, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
+      for (int s = 1; s < MERV_MAX_SEGMENTS; ++s) maps.a[s] = maps.a[0];
+    }
   }
   const long long total = (long long)p.m_blocks * p.n_blocks * (vid != nullptr ? vid->split : 1);
   int sms = sm_count();
@@ -764,6 +790,23 @@ int launch_gemm_tcgen05(const GemmSegment* seg, int nseg, const float* seg_scale
   attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = pdl ? 2 : 1;
+  if (vid != nullptr && vid->dy_batch_stride != 0) {
+    if (ctas == 2) {
+      constexpr int smem = Cfg<2, false>::SMEM_BYTES;
+      static const cudaError_t attr_rc = cudaFuncSetAttribute(gemm_wgrad_video_strided_tcgen05_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+      MERV_REQUIRE(attr_rc == cudaSuccess, MERV_E_CUDA, "cudaFuncSetAttribute(max dynamic smem=%d) failed: %s", smem, cudaGetErrorString(attr_rc));
+      cfg.dynamicSmemBytes = smem;
+      MERV_CUDA_OK(cudaLaunchKernelEx(&cfg, gemm_wgrad_video_strided_tcgen05_kernel<2>, maps, p));
+    } else {
+      constexpr int smem = Cfg<1, false>::SMEM_BYTES;
+      static const cudaError_t attr_rc = cudaFuncSetAttribute(gemm_wgrad_video_strided_tcgen05_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+      MERV_REQUIRE(attr_rc == cudaSuccess, MERV_E_CUDA, "cudaFuncSetAttribute(max dynamic smem=%d) failed: %s", smem, cudaGetErrorString(attr_rc));
+      cfg.dynamicSmemBytes = smem;
+      MERV_CUDA_OK(cudaLaunchKernelEx(&cfg, gemm_wgrad_video_strided_tcgen05_kernel<1>, maps, p));
+    }
+    MERV_CUDA_OK(cudaGetLastError());
+    return MERV_OK;
+  }
   if (vid != nullptr) {
     if (ctas == 2) {
       constexpr int smem = Cfg<2, false>::SMEM_BYTES;

@@ -304,7 +304,8 @@ struct MixParams {
 
 template <typename T, int E>
 __global__ void __launch_bounds__(256) softmax_mix_kernel(const __grid_constant__ MixParams p, const float* __restrict__ scores,
-                                                          float* __restrict__ weights, T* __restrict__ out, int Ttok, int K) {
+                                                          float* __restrict__ weights, T* __restrict__ out, long long ldo, long long obs, int Ttok,
+                                                          int K) {
   constexpr int VEC = Vec16<T>::kN;
   const int b = blockIdx.y, lane = threadIdx.x & 31;
   float wl;
@@ -326,7 +327,7 @@ __global__ void __launch_bounds__(256) softmax_mix_kernel(const __grid_constant_
   }
   const int kvec = K / VEC;
   const long long nvec = (long long)Ttok * kvec;
-  T* ob = out + (long long)b * Ttok * K;
+  T* ob = out + (long long)b * obs;
   const long long stride = (long long)gridDim.x * 256;
   for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < nvec; i += 2 * stride) {
     const long long i2 = i + stride;
@@ -350,7 +351,7 @@ __global__ void __launch_bounds__(256) softmax_mix_kernel(const __grid_constant_
 #pragma unroll
       for (int c = 0; c < VEC; ++c) acc[c] = fmaf(w[e], x[c], acc[c]);
     }
-    stg_na_v4(ob + t1 * K + c1, Vec16<T>::pack(acc));
+    stg_na_v4(ob + t1 * ldo + c1, Vec16<T>::pack(acc));
     if (has2) {
 #pragma unroll
       for (int c = 0; c < VEC; ++c) acc[c] = 0.f;
@@ -361,14 +362,14 @@ __global__ void __launch_bounds__(256) softmax_mix_kernel(const __grid_constant_
 #pragma unroll
         for (int c = 0; c < VEC; ++c) acc[c] = fmaf(w[e], x[c], acc[c]);
       }
-      stg_na_v4(ob + t2 * K + c2, Vec16<T>::pack(acc));
+      stg_na_v4(ob + t2 * ldo + c2, Vec16<T>::pack(acc));
     }
   }
 }
 
 template <typename T>
-static int launch_mix(const MixParams& p, const float* scores, float* weights, void* out, int B, int E, int Ttok, int K,
-                      cudaStream_t s) {
+static int launch_mix(const MixParams& p, const float* scores, float* weights, void* out, long long ldo, long long obs, int B, int E, int Ttok,
+                      int K, cudaStream_t s) {
   constexpr int VEC = Vec16<T>::kN;
   const long long nvec = (long long)Ttok * (K / VEC);
   // ~8 waves of 256-thread CTAs in total across the batch, at least 1 and at most what the video needs
@@ -380,7 +381,7 @@ static int launch_mix(const MixParams& p, const float* scores, float* weights, v
   T* o = static_cast<T*>(out);
   switch (E) {
 #define MERV_MIX_CASE(n) \
-  case n: softmax_mix_kernel<T, n><<<grid, 256, 0, s>>>(p, scores, weights, o, Ttok, K); break;
+  case n: softmax_mix_kernel<T, n><<<grid, 256, 0, s>>>(p, scores, weights, o, ldo, obs, Ttok, K); break;
     MERV_MIX_CASE(1) MERV_MIX_CASE(2) MERV_MIX_CASE(3) MERV_MIX_CASE(4) MERV_MIX_CASE(5) MERV_MIX_CASE(6) MERV_MIX_CASE(7) MERV_MIX_CASE(8)
 #undef MERV_MIX_CASE
     default: return fail(MERV_E_ARG, "merv_softmax_mix: E=%d not in [1,%d]", E, MERV_MAX_ENCODERS);
@@ -564,8 +565,11 @@ extern "C" int merv_softmax_weights_ex(const float* scores, float* weights, void
   return MERV_OK;
 }
 
-extern "C" int merv_softmax_mix(const void* const* V, const int32_t* tokens, const float* scores, float* weights, void* out,
-                                int B, int E, int T, int K, int dtype, void* stream) {
+// out video b's rows start at out + b * out_batch_stride, rows ldo apart: the fused tokens go straight into the prefix slot of the
+// [B, L + T, K] multimodal embedding buffer.  Nothing outside the [B, T, K] block is written.  ldo == K, out_batch_stride == T * K is
+// merv_softmax_mix (the same kernel, bit-identical).
+extern "C" int merv_softmax_mix_ex(const void* const* V, const int32_t* tokens, const float* scores, float* weights, void* out, int64_t ldo,
+                                   int64_t out_batch_stride, int B, int E, int T, int K, int dtype, void* stream) {
   MERV_DTYPE_OK("merv_softmax_mix");
   MERV_REQUIRE(V && tokens && weights && out, MERV_E_ARG, "merv_softmax_mix: NULL pointer");
   MERV_REQUIRE(E >= 1 && E <= MERV_MAX_ENCODERS, MERV_E_ARG, "merv_softmax_mix: E=%d not in [1,%d]", E, MERV_MAX_ENCODERS);
@@ -573,6 +577,11 @@ extern "C" int merv_softmax_mix(const void* const* V, const int32_t* tokens, con
   const int vec = dtype == MERV_BF16 ? 8 : 4;
   MERV_REQUIRE(K % vec == 0, MERV_E_SHAPE, "merv_softmax_mix: K=%d must be a multiple of %d", K, vec);
   MERV_REQUIRE(aligned16(out), MERV_E_ALIGN, "merv_softmax_mix: out not 16-byte aligned");
+  MERV_REQUIRE(ldo % vec == 0 && out_batch_stride % vec == 0, MERV_E_ALIGN,
+               "merv_softmax_mix_ex: ldo=%lld / out_batch_stride=%lld must be whole 16-byte vectors", (long long)ldo, (long long)out_batch_stride);
+  MERV_REQUIRE(ldo >= K && out_batch_stride >= (int64_t)T * ldo, MERV_E_SHAPE,
+               "merv_softmax_mix_ex: ldo=%lld < K or out_batch_stride=%lld < T * ldo (rows or videos would overlap)", (long long)ldo,
+               (long long)out_batch_stride);
   if (int rc = require_sm100()) return rc;
   if (B == 0) return MERV_OK;
   MixParams p;
@@ -584,8 +593,13 @@ extern "C" int merv_softmax_mix(const void* const* V, const int32_t* tokens, con
     p.tokens[e] = tokens[e];
   }
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (dtype == MERV_BF16) return launch_mix<__nv_bfloat16>(p, scores, weights, out, B, E, T, K, s);
-  return launch_mix<float>(p, scores, weights, out, B, E, T, K, s);
+  if (dtype == MERV_BF16) return launch_mix<__nv_bfloat16>(p, scores, weights, out, ldo, out_batch_stride, B, E, T, K, s);
+  return launch_mix<float>(p, scores, weights, out, ldo, out_batch_stride, B, E, T, K, s);
+}
+
+extern "C" int merv_softmax_mix(const void* const* V, const int32_t* tokens, const float* scores, float* weights, void* out,
+                                int B, int E, int T, int K, int dtype, void* stream) {
+  return merv_softmax_mix_ex(V, tokens, scores, weights, out, K, (int64_t)T * K, B, E, T, K, dtype, stream);
 }
 
 // merv_scores_from_partials + merv_softmax_weights_ex in one launch (bf16 biases); used by merv_fused_forward

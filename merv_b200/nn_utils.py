@@ -231,30 +231,83 @@ class _ConvTapsFn(torch.autograd.Function):
         return None, None, None, dW, db
 
 
+class _Assembly:
+    """MERV.forward's ``[BOS | prefix | text]`` assembly (merv.py:622-720) done INSIDE a mixer's autograd Function, which then owns the whole
+    embedding buffer: the kernels write the prefix into its slot and its backward reads the prefix gradient from the buffer's gradient in place.
+    (An in-place write into a view of a buffer autograd tracks would make CopySlices clone the whole gradient: the copy this avoids.)
+
+    Rows ``idx`` (multimodal) come first as [BOS | prefix | text], then rows ``uni`` (text only) padded at the end with T zero rows.
+    ``emb`` [Bt, L, K] is the text embedding tensor; it is one more differentiable input of the Function."""
+
+    def __init__(self, emb: torch.Tensor, idx: torch.Tensor, uni: torch.Tensor, bos: int) -> None:
+        self.emb, self.idx, self.uni, self.bos = emb, idx, uni, bos
+
+    def buffer(self, T: int, K: int, dtype: torch.dtype) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(buf [Bm + Bu, L + T, K] in `dtype` with the text spliced in, its prefix slot buf[:Bm, bos:bos + T])."""
+        e, idx, uni, bos = self.emb.detach(), self.idx, self.uni, self.bos
+        Bm, Bu, L = idx.numel(), uni.numel(), e.shape[1]
+        assert e.shape[2] == K, f"input_embeddings have {e.shape[2]} channels, the prefix {K}"
+        buf = torch.empty((Bm + Bu, L + T, K), dtype=dtype, device=e.device)
+        buf[:Bm, :bos].copy_(e[idx, :bos])
+        buf[:Bm, bos + T:].copy_(e[idx, bos:])
+        if Bu:
+            buf[Bm:, :L].copy_(e[uni])
+            buf[Bm:, L:].zero_()
+        return buf, buf[:Bm, bos:bos + T]
+
+    def grads(self, dbuf: Optional[torch.Tensor], T: int, dtype: torch.dtype, need_emb: bool):
+        """(prefix-slot gradient [Bm, T, K], a view of dbuf unless dbuf had to be made contiguous in `dtype`; d input_embeddings or None).
+        The text parts of dbuf go back to rows idx / uni; rows in neither set get zeros."""
+        idx, uni, bos = self.idx, self.uni, self.bos
+        Bm, L = idx.numel(), self.emb.shape[1]
+        if dbuf is None:  # only the mixing weights were used downstream
+            return None, None
+        if dbuf.dtype != dtype or not dbuf.is_contiguous():
+            dbuf = dbuf.to(dtype).contiguous()
+        demb = None
+        if need_emb:
+            demb = torch.zeros(self.emb.shape, dtype=self.emb.dtype, device=dbuf.device)
+            demb.index_add_(0, idx, torch.cat([dbuf[:Bm, :bos], dbuf[:Bm, bos + T:]], 1).to(demb.dtype))
+            if uni.numel():
+                demb.index_add_(0, uni, dbuf[Bm:, :L].to(demb.dtype))
+        return dbuf[:Bm, bos:bos + T], demb
+
+
 class _MixFn(torch.autograd.Function):
     """CrossAttentionAdapterLearnableQuery.forward (nn_utils.py:487-521) with its hand-written backward, in every configuration:
     averagetoken=True / False, single-token (repeated) encoders, and positional_embedding=True, where ``pe`` is an input (None
-    otherwise: with averagetoken=False the reference never reads it, so it gets no gradient)."""
+    otherwise: with averagetoken=False the reference never reads it, so it gets no gradient).  With an assembly (``asm``, see _Assembly) the
+    fused tokens go into the prefix slot of the embedding buffer, which is returned instead, and ``emb`` gets its gradient."""
 
     @staticmethod
-    def forward(ctx, adapter, dtype, Q, Wq, Wk, bias, pe, *V):
+    def forward(ctx, adapter, dtype, asm, emb, Q, Wq, Wk, bias, pe, *V):
         c = adapter._cast_cache
         Vc = [v if v.dtype == dtype else v.to(dtype) for v in V]
         u = adapter.query_vector(dtype)  # [K], or [T*K] with averagetoken=False (the key is the flattened token block)
         per_token_u = not adapter.averagetoken
-        scores = ops.scores_from_tokens(Vc, u, adapter.token_length, per_token_u=per_token_u, consts=adapter._pe_consts(dtype),
-                                        mean=adapter.averagetoken)
-        out, weights = ops.softmax_mix(Vc, adapter.token_length, scores=scores)
+        T = adapter.token_length
+        scores = ops.scores_from_tokens(Vc, u, T, per_token_u=per_token_u, consts=adapter._pe_consts(dtype), mean=adapter.averagetoken)
+        buf, slot = (None, None) if asm is None else asm.buffer(T, Vc[0].shape[2], dtype)
+        if slot is None:
+            out, weights = ops.softmax_mix(Vc, T, scores=scores)
+        else:
+            _, weights = ops.softmax_mix(Vc, T, scores=scores, out=slot)
         params = (Q, Wq, Wk, bias) + (() if pe is None else (pe,))
         ctx.save_for_backward(weights, u, *[c.get(p, dtype) for p in params], *Vc)
         ctx.meta = (dtype, per_token_u, [p.dtype for p in params], [v.dtype for v in V])
-        return out, weights.to(dtype)
+        ctx.asm, ctx.T = asm, T
+        return (out if asm is None else buf), weights.to(dtype)
 
     @staticmethod
     def backward(ctx, dout, dweights):
         dtype, per_token_u, pdt, vdt = ctx.meta
         weights, u, Qc, Wqc, Wkc, bc, *rest = ctx.saved_tensors
         pec, Vc = (rest[0], rest[1:]) if len(pdt) == 5 else (None, rest)
+        demb = None
+        if ctx.asm is not None:  # the prefix slot of the buffer's gradient, read in place by the kernels
+            dout, demb = ctx.asm.grads(dout, ctx.T, dtype, ctx.needs_input_grad[3])
+        if dout is None:  # only the mixing weights were used downstream
+            dout = torch.zeros((weights.shape[0], ctx.T, Vc[0].shape[2]), dtype=dtype, device=weights.device)
         dw = None if dweights is None else dweights.float().contiguous()
         if per_token_u or pec is not None or any(v.shape[1] != dout.shape[1] for v in Vc):
             dVs, dQ, dWq, dWk, dbias, dpe = ops.mix_backward_ex(Vc, dout.to(dtype), weights, dw, u, Qc, Wqc, Wkc, bc, per_token_u=per_token_u, pe=pec)
@@ -263,39 +316,47 @@ class _MixFn(torch.autograd.Function):
         grads = [g.to(t) for g, t in zip((dQ, dWq, dWk, dbias, dpe), pdt)]
         if dpe is None:
             grads.append(None)
-        return (None, None, *grads, *[g.to(t) for g, t in zip(dVs, vdt)])
+        return (None, None, None, demb, *grads, *[g.to(t) for g, t in zip(dVs, vdt)])
 
 
 class _ScalarMixFn(torch.autograd.Function):
     """ScalarAdapter.forward (nn_utils.py:524-537) with its hand-written backward: w = softmax(scalar) [E] for every video,
     out = sum_e w_e V_e, returns (out, w[None]).  dV_e = w_e dOut and dscalar = w (.) (g - <w, g>) with
     g_e = sum_b <dOut[b], V_e[b]> + dW_out[e], in one pass over dOut and the V_e (merv_scalar_mix_backward).  Every V_e is [B, T, K]:
-    the reference stacks them.  The scalar gradient comes back in the parameter's dtype (fp32 master weights under autocast)."""
+    the reference stacks them.  The scalar gradient comes back in the parameter's dtype (fp32 master weights under autocast).  With an
+    assembly (``asm``, see _Assembly) the mix goes into the prefix slot of the embedding buffer, which is returned instead."""
 
     @staticmethod
-    def forward(ctx, scalar, dtype, *V):
+    def forward(ctx, scalar, dtype, asm, emb, *V):
         Vc = [v if v.dtype == dtype else v.to(dtype) for v in V]
         B, T, K = Vc[0].shape
         E = len(Vc)
         w, _ = ops.softmax_weights(scalar.detach().float().reshape(1, E))
-        if B > 0:
+        buf, slot = (None, None) if asm is None else asm.buffer(T, K, dtype)
+        if B > 0 and slot is not None:
+            ops.softmax_mix(Vc, T, weights=w.expand(B, E).contiguous(), out=slot)
+        elif B > 0:
             out, _ = ops.softmax_mix(Vc, T, weights=w.expand(B, E).contiguous())
         else:  # a rank that owns no videos (merv_b200/parallel.py): no mix to launch, the weights still carry a gradient
             out = torch.empty((0, T, K), dtype=dtype, device=Vc[0].device)
         ctx.save_for_backward(w, *Vc)
         ctx.meta = (scalar.dtype, [v.dtype for v in V])
-        return out, w.to(dtype)
+        ctx.asm = asm
+        return (out if asm is None else buf), w.to(dtype)
 
     @staticmethod
     def backward(ctx, dout, dweights):
         w, *Vc = ctx.saved_tensors
         sdt, vdt = ctx.meta
         dt = Vc[0].dtype
+        demb = None
+        if ctx.asm is not None:  # the prefix slot of the buffer's gradient, read in place by the kernel
+            dout, demb = ctx.asm.grads(dout, Vc[0].shape[1], dt, ctx.needs_input_grad[3])
         if dout is None:  # only the mixing weights were used downstream
             dout = torch.zeros_like(Vc[0])
         dw = None if dweights is None else dweights.float().reshape(-1).contiguous()
         dVs, dscalar = ops.scalar_mix_backward(Vc, dout.to(dt), w.reshape(-1), dw)
-        return (dscalar.to(sdt), None, *[g.to(t) for g, t in zip(dVs, vdt)])
+        return (dscalar.to(sdt), None, None, demb, *[g.to(t) for g, t in zip(dVs, vdt)])
 
 
 class _AttentivePoolFn(torch.autograd.Function):
@@ -410,6 +471,34 @@ class _CastCache:
         return hit[1]
 
 
+def _fused_mix_into(asm: Optional[_Assembly], pooled, Ws, weights, bias_mix, B: int, T: int, K: int):
+    """The fused GEMM's prefix [B, T, K] and the embedding buffer (None without an assembly).  The GEMM stores straight into the buffer's
+    prefix slot when T % 128 == 0 (its batch-strided store); otherwise the prefix is computed contiguous and copied in."""
+    if asm is None:
+        return ops.fused_linear_mix(pooled, Ws, weights, bias_mix, T).view(B, T, K), None
+    buf, slot = asm.buffer(T, K, torch.bfloat16)
+    if T % 128 == 0:
+        ops.fused_linear_mix(pooled, Ws, weights, bias_mix, T, out=slot)
+    else:
+        slot.copy_(ops.fused_linear_mix(pooled, Ws, weights, bias_mix, T).view(B, T, K))
+    return slot, buf
+
+
+def _fused_dout(asm: Optional[_Assembly], dout, B: int, T: int, K: int, dt: torch.dtype, device, need_emb: bool):
+    """(dOut [B, T, K] in `dt` — the prefix slot of the buffer's gradient, read in place — and d input_embeddings) for the fused backwards."""
+    demb = None
+    if asm is not None:
+        dout, demb = asm.grads(dout, T, dt, need_emb)
+    if dout is None:  # only the mixing weights were used downstream
+        return torch.zeros((B, T, K), dtype=dt, device=device), demb
+    if dout.dtype != dt:
+        dout = dout.to(dt)
+    if dout.stride(2) != 1:
+        dout = dout.contiguous()
+    # the videos' rows back to back: one [B * T, K] matrix, as the GEMMs took it before any embedding buffer existed
+    return (dout.view(B * T, K) if dout.is_contiguous() else dout), demb
+
+
 class _FusedLinearFn(torch.autograd.Function):
     """Training step of the shipped configuration (3d-avg pool + linear projectors + learnable-query mixer, merv.py:587-589,608)
     through the FUSED forward, with a backward that never materialises the per-encoder projections Y_e or their gradients.
@@ -421,29 +510,33 @@ class _FusedLinearFn(torch.autograd.Function):
               Token counts that are not a multiple of 64 take the two-GEMM form (Z_e = dOut W_e, dW_e = dOut^T (w_e (.) P_e)).
     Per video this moves ~100 MB less through HBM in the forward and ~130 MB less in the backward than the module-by-module
     path and keeps 7 MB instead of 41 MB of activations.  No gradient flows into the patch features (frozen backbones).
+    ``batch_index`` gathers the videos inside the pool kernel (``multimodal_indices``); with an assembly (``asm``, see _Assembly) the GEMM
+    writes the prefix into its slot of the embedding buffer (T % 128 == 0; otherwise it is computed contiguous and copied in), the buffer is
+    returned, and the backward reads dOut from the buffer's gradient in place.
     """
 
     @staticmethod
-    def forward(ctx, fusion, projs, xs, Q, Wq, Wk, in_proj_bias, *proj_params):
+    def forward(ctx, fusion, projs, xs, batch_index, asm, emb, Q, Wq, Wk, in_proj_bias, *proj_params):
         dtype = torch.bfloat16
         E = len(projs)
         T, K = fusion.token_length, fusion.llm_dim
-        B = xs[0].shape[0]
+        B = xs[0].shape[0] if batch_index is None else batch_index.numel()
         lasts = [p.layers()[-1][0] for p in projs]
         vcs = [fusion._affine_vec(lin, p._cast_cache, dtype) for lin, p in zip(lasts, projs)]
         Ws = [p._cast_cache.get(lin.weight, dtype) for lin, p in zip(lasts, projs)]
         biases = [p._cast_cache.get(lin.bias, dtype) for lin, p in zip(lasts, projs)]
-        pooled, partials = fusion._fused_stage1(projs, xs, vcs, dtype)
+        pooled, partials = fusion._fused_stage1(projs, xs, vcs, dtype, batch_index=batch_index)
         scores = ops.scores_from_partials(partials, [vc[1] for vc in vcs], B, T)
         weights, bias_mix = ops.softmax_weights(scores, biases, K)
-        out = ops.fused_linear_mix(pooled, Ws, weights, bias_mix, T)
+        out, buf = _fused_mix_into(asm, pooled, Ws, weights, bias_mix, B, T, K)
         c = fusion._cast_cache
         ctx.fusion_dims = (B, E, T, K)
+        ctx.asm = asm
         ctx.param_dtypes = [t.dtype for t in (Q, Wq, Wk, in_proj_bias, *proj_params)]
         ctx.save_for_backward(weights, fusion.query_vector(dtype), c.get(Q, dtype), c.get(Wq, dtype), c.get(Wk, dtype), c.get(in_proj_bias, dtype),
                               *pooled, *Ws, *biases)
         w_out = weights.to(dtype)
-        return out.view(B, T, K), w_out
+        return (out if asm is None else buf), w_out
 
     @staticmethod
     def backward(ctx, dout, dweights):
@@ -452,15 +545,11 @@ class _FusedLinearFn(torch.autograd.Function):
         weights, u, Qc, Wqc, Wkc, bc = saved[:6]
         pooled, Ws, biases = saved[6:6 + E], saved[6 + E:6 + 2 * E], saved[6 + 2 * E:6 + 3 * E]
         dt = Ws[0].dtype
-        if dout is None:  # only the mixing weights were used downstream
-            dout = torch.zeros((B, T, K), dtype=dt, device=weights.device)
-        g = dout.reshape(B * T, K)
-        if g.dtype != dt:
-            g = g.to(dt)
-        if g.stride(1) != 1 or g.stride(0) != K:
-            g = g.contiguous()
+        g, demb = _fused_dout(ctx.asm, dout, B, T, K, dt, weights.device, ctx.needs_input_grad[5])
         dwo = None if dweights is None else dweights.float().contiguous()
         gsum = ops.video_colsum(g.view(B, T, K))
+        if T % 64:  # the two-GEMM form below reads dOut as one [B * T, K] matrix
+            g = g.contiguous().view(B * T, K)
         dw_partials, pbars, dWs = [], [], []
         for e in range(E):  # dOut, P_e and W_e are all read in place: the tensor cores take them MN-major (no transposed copies)
             P = pooled[e].reshape(B * T, -1)
@@ -482,7 +571,7 @@ class _FusedLinearFn(torch.autograd.Function):
         for e in range(E):
             grads += [dWs[e], dbs[e]]
         grads = [gr.to(pd) if gr is not None else None for gr, pd in zip(grads, ctx.param_dtypes)]
-        return (None, None, None, *grads)
+        return (None, None, None, None, None, demb, *grads)
 
 
 class _FusedScalarLinearFn(torch.autograd.Function):
@@ -492,24 +581,26 @@ class _FusedScalarLinearFn(torch.autograd.Function):
     backward: per encoder ONE tcgen05 pass over dOut and the pooled tokens P_e (merv_wgrad_video, the same w_e for every video):
               dW_e = w_e dOut^T P_e and the partials of <dOut[b], Y_e[b] - b_e>;  gsum = colsum_t(dOut);  then merv_scalar_fused_backward:
               db_e = w_e sum_b gsum[b],  g_e = partials + b_e . sum_b gsum[b] + dW_out[e],  dscalar = w (.) (g - <w, g>).
-    Needs T % 64 == 0 (ScalarAdapter._can_fuse_training); no gradient flows into the patch features (frozen backbones)."""
+    Needs T % 64 == 0 (ScalarAdapter._can_fuse_training); no gradient flows into the patch features (frozen backbones).  ``batch_index`` and
+    an assembly (``asm``) as for _FusedLinearFn."""
 
     @staticmethod
-    def forward(ctx, adapter, projs, xs, scalar, *proj_params):
+    def forward(ctx, adapter, projs, xs, batch_index, asm, emb, scalar, *proj_params):
         dtype = torch.bfloat16
-        E, B = len(projs), xs[0].shape[0]
+        E, B = len(projs), (xs[0].shape[0] if batch_index is None else batch_index.numel())
         lasts = [p.layers()[0][0] for p in projs]
         Ws = [p._cast_cache.get(lin.weight, dtype) for lin, p in zip(lasts, projs)]
         biases = [p._cast_cache.get(lin.bias, dtype) for lin, p in zip(lasts, projs)]
-        pooled, _ = ops.pool3d(xs, [p.output_frames for p in projs], projs[0].output_size)
+        pooled, _ = ops.pool3d(xs, [p.output_frames for p in projs], projs[0].output_size, batch_index=batch_index)
         T, K = pooled[0].shape[1], lasts[0].out_features
         scores = scalar.detach().float().reshape(1, E).expand(B, E).contiguous()
         weights, bias_mix = ops.softmax_weights(scores, biases, K)
-        out = ops.fused_linear_mix(pooled, Ws, weights, bias_mix, T)
+        out, buf = _fused_mix_into(asm, pooled, Ws, weights, bias_mix, B, T, K)
         ctx.dims = (B, E, T, K)
+        ctx.asm = asm
         ctx.param_dtypes = [t.dtype for t in (scalar, *proj_params)]
         ctx.save_for_backward(weights[0], *pooled, *Ws, *biases)
-        return out.view(B, T, K), weights[:1].to(dtype)
+        return (out if asm is None else buf), weights[:1].to(dtype)
 
     @staticmethod
     def backward(ctx, dout, dweights):
@@ -517,13 +608,7 @@ class _FusedScalarLinearFn(torch.autograd.Function):
         w, *saved = ctx.saved_tensors
         pooled, Ws, biases = saved[:E], saved[E:2 * E], saved[2 * E:3 * E]
         dt = Ws[0].dtype
-        if dout is None:  # only the mixing weights were used downstream
-            dout = torch.zeros((B, T, K), dtype=dt, device=w.device)
-        g = dout.reshape(B * T, K)
-        if g.dtype != dt:
-            g = g.to(dt)
-        if g.stride(1) != 1 or g.stride(0) != K:
-            g = g.contiguous()
+        g, demb = _fused_dout(ctx.asm, dout, B, T, K, dt, w.device, ctx.needs_input_grad[5])
         gsum = ops.video_colsum(g.view(B, T, K))
         dWs, dw_partials = [], []
         for e in range(E):  # scale stride 0: w_e for every video
@@ -536,7 +621,7 @@ class _FusedScalarLinearFn(torch.autograd.Function):
         for e in range(E):
             grads += [dWs[e], dbs[e]]
         grads = [gr.to(pd) if gr is not None else None for gr, pd in zip(grads, ctx.param_dtypes)]
-        return (None, None, None, *grads)
+        return (None, None, None, None, None, demb, *grads)
 
 
 def _unwrap(module: nn.Module) -> nn.Module:
@@ -729,6 +814,19 @@ class DeferredProjection:
 
     def materialize(self) -> torch.Tensor:
         return self.projector._forward_unfused(self.features)
+
+
+def _materialize(V, batch_index: Optional[torch.Tensor]) -> List[torch.Tensor]:
+    """Projected tokens of the videos `batch_index` selects (all when None).  A DeferredProjection still holds the whole batch's features:
+    they are gathered with index_select before the projector runs, as the reference indexes the inputs before the backbones (merv.py:576-585);
+    tensors are the outputs of projectors that already saw the gathered features (MervFusion._project)."""
+    out = []
+    for v in V:
+        if isinstance(v, DeferredProjection):
+            x = v.features if batch_index is None else v.features.index_select(0, batch_index.to(device=v.features.device, dtype=torch.long))
+            v = v.projector._forward_unfused(x)
+        out.append(v)
+    return out
 
 
 class AveragePooling3DProjector(TokenResampler):
@@ -1194,8 +1292,21 @@ class CrossAttentionAdapterLearnableQuery(_LinkedMixer):
         if _needs_grad(self, *V):
             att = self.attention
             pe = self.pe if self.positional_embedding and self.averagetoken else None
-            return _MixFn.apply(self, _compute_dtype(V[0]), self.Q, att.q_proj_weight, att.k_proj_weight, att.in_proj_bias, pe, *V)
+            return _MixFn.apply(self, _compute_dtype(V[0]), None, None, self.Q, att.q_proj_weight, att.k_proj_weight, att.in_proj_bias, pe, *V)
         return self._forward_tokens(V)
+
+    def _forward_assembled(self, V, asm: "_Assembly", batch_index: Optional[torch.Tensor]) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(embedding buffer with the prefix in its slot, weights) through the autograd Functions (MervFusion.forward_multimodal): the fused
+        training step when it covers the configuration, module by module otherwise (bf16 or fp32, any averagetoken / pe / token layout)."""
+        deferred = all(isinstance(v, DeferredProjection) for v in V)
+        train = _needs_grad(self, asm.emb, *[t for v in V for t in ((v.features,) if isinstance(v, DeferredProjection) else (v,))],
+                            *[t for v in V if isinstance(v, DeferredProjection) for t in v.projector.parameters()])
+        if deferred and train and self._can_fuse_training(V):
+            return self._forward_fused_train(V, batch_index=batch_index, asm=asm)
+        V = _materialize(V, batch_index)
+        att = self.attention
+        pe = self.pe if self.positional_embedding and self.averagetoken else None
+        return _MixFn.apply(self, _compute_dtype(V[0]), asm, asm.emb, self.Q, att.q_proj_weight, att.k_proj_weight, att.in_proj_bias, pe, *V)
 
     def _forward_tokens(self, V: Sequence[torch.Tensor], rowdots=None) -> Tuple[torch.Tensor, torch.Tensor]:
         dtype = _compute_dtype(V[0])
@@ -1231,7 +1342,7 @@ class CrossAttentionAdapterLearnableQuery(_LinkedMixer):
                 return False
         return self.attention.in_proj_bias is not None
 
-    def _forward_fused_train(self, V: Sequence[DeferredProjection]) -> Tuple[torch.Tensor, torch.Tensor]:
+    def _forward_fused_train(self, V: Sequence[DeferredProjection], batch_index=None, asm=None) -> Tuple[torch.Tensor, torch.Tensor]:
         dtype = torch.bfloat16
         projs = [v.projector for v in V]
         xs = [v.features.detach() for v in V]
@@ -1239,7 +1350,8 @@ class CrossAttentionAdapterLearnableQuery(_LinkedMixer):
         xs = [x if _tma_readable(x) else x.contiguous() for x in xs]
         att = self.attention
         params = [t for p in projs for t in (p.layers()[0][0].weight, p.layers()[0][0].bias)]
-        return _FusedLinearFn.apply(self, projs, xs, self.Q, att.q_proj_weight, att.k_proj_weight, att.in_proj_bias, *params)
+        return _FusedLinearFn.apply(self, projs, xs, batch_index, asm, None if asm is None else asm.emb, self.Q, att.q_proj_weight,
+                                    att.k_proj_weight, att.in_proj_bias, *params)
 
     # ---- fused pipeline ------------------------------------------------------------------------------------
     def _fused_stage1(self, projs, xs, vcs, dtype, max_ctas: int = 0, batch_index=None):
@@ -1383,6 +1495,19 @@ class ScalarAdapter(_LinkedMixer):
         out, weights = ops.softmax_mix(V, V[0].shape[1], scores=scores)
         return out, weights[:1].to(dtype)
 
+    def _forward_assembled(self, V, asm: "_Assembly", batch_index: Optional[torch.Tensor]) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(embedding buffer with the prefix in its slot, weights), as CrossAttentionAdapterLearnableQuery._forward_assembled."""
+        E = len(V)
+        assert E == self.scalar.numel(), f"ScalarAdapter holds {self.scalar.numel()} scalars, got {E} encoders (nn_utils.py:527,535)"
+        proj_params = [t for v in V if isinstance(v, DeferredProjection) for t in v.projector.parameters()]
+        if _needs_grad(self, asm.emb, *[v for v in V if isinstance(v, torch.Tensor)], *proj_params) and asm.idx.numel() and self._can_fuse_training(V):
+            return self._forward_train(V, batch_index=batch_index, asm=asm)
+        V = _materialize(V, batch_index)
+        if len({tuple(v.shape) for v in V}) != 1:
+            raise ValueError("the ScalarAdapter needs every encoder at one [B, T, K] shape to mix into the embedding buffer (the reference "
+                             f"stacks them, nn_utils.py:535), got {[tuple(v.shape) for v in V]}")
+        return _ScalarMixFn.apply(self.scalar, _compute_dtype(V[0]), asm, asm.emb, *V)
+
     def _can_fuse_training(self, V) -> bool:
         """The fused backward (_FusedScalarLinearFn) covers single-Linear projectors with bias on one pooled grid, bf16 compute, token
         counts that are a multiple of 64 (a k-block of merv_wgrad_video never spans two videos), frozen features, at least one video."""
@@ -1396,7 +1521,7 @@ class ScalarAdapter(_LinkedMixer):
                 return False
         return True
 
-    def _forward_train(self, V) -> Tuple[torch.Tensor, torch.Tensor]:
+    def _forward_train(self, V, batch_index=None, asm=None) -> Tuple[torch.Tensor, torch.Tensor]:
         if self._can_fuse_training(V):
             dtype = torch.bfloat16
             projs = [v.projector for v in V]
@@ -1404,12 +1529,12 @@ class ScalarAdapter(_LinkedMixer):
             xs = [x if x.dtype == dtype else x.to(dtype) for x in xs]
             xs = [x if _tma_readable(x) else x.contiguous() for x in xs]
             params = [t for p in projs for t in (p.layers()[0][0].weight, p.layers()[0][0].bias)]
-            return _FusedScalarLinearFn.apply(self, projs, xs, self.scalar, *params)
+            return _FusedScalarLinearFn.apply(self, projs, xs, batch_index, asm, None if asm is None else asm.emb, self.scalar, *params)
         V = [v.materialize() if isinstance(v, DeferredProjection) else v for v in V]
         if len({tuple(v.shape) for v in V}) != 1:
             raise ValueError("training the ScalarAdapter needs every encoder at one [B, T, K] shape (the reference stacks them, "
                              f"nn_utils.py:535), got {[tuple(v.shape) for v in V]}")
-        return _ScalarMixFn.apply(self.scalar, _compute_dtype(V[0]), *V)
+        return _ScalarMixFn.apply(self.scalar, _compute_dtype(V[0]), None, None, *V)
 
 
 class ConcatChannelFusion(LinearProjector):
@@ -1760,12 +1885,55 @@ class MervFusion(nn.Module):
             return self.feature_fusion(projected)
         return self.feature_fusion(projected, out=out, batch_index=batch_index)
 
+    def _slot_inference(self, patch_features: Sequence[torch.Tensor], input_embeddings: torch.Tensor) -> bool:
+        """Whether the linked bf16 inference path (the cached single-call plan, _forward_fused with ``out=``) writes the prefix: autograd
+        records nothing, the learnable-query mixer fuses these inputs.  Everything else assembles the embeddings inside the mixer's autograd
+        Function (_Assembly): training, fp32, and the module-by-module path."""
+        ff = self.feature_fusion
+        if not isinstance(ff, CrossAttentionAdapterLearnableQuery) or _needs_grad(self, input_embeddings, *patch_features):
+            return False
+        if ff.token_length % 128:  # the GEMM's batch-strided slot store works in 128-row tiles
+            return False
+        if any(getattr(p, "_linked_fusion", None) is None or not ff._may_defer(p) for p in self.projectors):
+            return False
+        return ff._can_fuse([DeferredProjection(p, x) for p, x in zip(self.projectors, patch_features)])
+
+    def _project(self, patch_features: Sequence[torch.Tensor], batch_index: Optional[torch.Tensor]) -> list:
+        """The projectors' outputs for the videos `batch_index` selects: a linked projector that hands its input over keeps the whole batch
+        (the fused pool gathers in-kernel, _materialize otherwise); every other projector sees the gathered features."""
+        ff = self.feature_fusion
+        out = []
+        for p, x in zip(self.projectors, patch_features):
+            defers = getattr(p, "_linked_fusion", None) is not None and ff._may_defer(p)
+            if batch_index is not None and not defers:
+                x = x.index_select(0, batch_index.to(device=x.device, dtype=torch.long))
+            out.append(p(x))
+        return out
+
+    def _assemble(self, patch_features: Sequence[torch.Tensor], input_embeddings: torch.Tensor, idx: Optional[torch.Tensor],
+                  uni: torch.Tensor, bos: int) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(embedding buffer, weights) with the assembly inside the mixer's autograd Function; `idx` None = every row is multimodal."""
+        ff = self.feature_fusion
+        if not isinstance(ff, (CrossAttentionAdapterLearnableQuery, ScalarAdapter)):
+            raise NotImplementedError("the embedding assembly covers the learnable-query and scalar mixers")
+        dev = input_embeddings.device
+        bi = None if idx is None else _as_batch_index(idx, patch_features[0])
+        asm = _Assembly(input_embeddings, torch.arange(input_embeddings.shape[0], device=dev) if idx is None else idx.to(dev), uni, bos)
+        return ff._forward_assembled(self._project(patch_features, bi), asm, bi)
+
     def forward_into_embeddings(self, patch_features: Sequence[torch.Tensor], input_embeddings: torch.Tensor,
                                 bos_token_length: int = 1, multimodal_indices: Optional[torch.Tensor] = None):
         """Build `[BOS | visual prefix | text]` embeddings as MERV.forward does (merv.py:572,633-640) without the
         concat copy of the prefix: the buffer is allocated once, the text embeddings are copied around the prefix slot
-        and the fused GEMM writes the prefix straight into it.  Returns (multimodal_embeddings, weights)."""
+        and the fused GEMM writes the prefix straight into it.  Returns (multimodal_embeddings, weights).
+        In grad mode, in fp32 and on the module-by-module path the buffer belongs to the mixer's autograd Function: the prefix gradient is
+        read from the buffer's gradient in place, and ``input_embeddings`` get theirs (rows outside ``multimodal_indices``: zeros)."""
         ff = self.feature_fusion
+        if not self._slot_inference(patch_features, input_embeddings):
+            idx = multimodal_indices
+            uni = torch.zeros(0, dtype=torch.long, device=input_embeddings.device)
+            return self._assemble(patch_features, input_embeddings, None if idx is None else idx.to(input_embeddings.device), uni,
+                                  bos_token_length)
         idx = multimodal_indices
         emb = input_embeddings if idx is None else input_embeddings[idx]
         B, L, K = emb.shape
@@ -1789,11 +1957,12 @@ class MervFusion(nn.Module):
 
         ``patch_features[e]`` is the backbone output for the WHOLE batch (it is gathered inside the pool kernel).
         ``unimodal_indices`` may be passed to avoid the host sync the reference's Python loop (merv.py:668-672) implies.
+        In grad mode, in fp32, with the scalar mixer and on the module-by-module path the buffer belongs to the mixer's autograd Function
+        (_Assembly): the kernels read the prefix gradient from the buffer's gradient in place and ``input_embeddings`` get theirs.
         Returns (fused_embeddings, fused_attention_mask | None, fused_labels | None, weights)."""
         ff = self.feature_fusion
         emb = input_embeddings
         Bt, L, K = emb.shape
-        T = ff.token_length
         dev = emb.device
         idx = torch.arange(Bt, device=dev) if multimodal_indices is None else multimodal_indices.to(dev)
         if unimodal_indices is None:
@@ -1803,14 +1972,19 @@ class MervFusion(nn.Module):
         uni = unimodal_indices.to(dev)
         Bm, Bu = idx.numel(), uni.numel()
         bos = bos_token_length
-        buf = torch.empty((Bm + Bu, L + T, K), dtype=torch.bfloat16, device=dev)
-        buf[:Bm, :bos].copy_(emb[idx, :bos])
-        buf[:Bm, bos + T:].copy_(emb[idx, bos:])
-        if Bu:
-            buf[Bm:, :L].copy_(emb[uni])
-            buf[Bm:, L:].zero_()
         whole = multimodal_indices is None
-        _, weights = self.forward(patch_features, out=buf[:Bm, bos:bos + T], batch_index=None if whole else idx.to(torch.int32))
+        if self._slot_inference(patch_features, emb):
+            T = ff.token_length
+            buf = torch.empty((Bm + Bu, L + T, K), dtype=torch.bfloat16, device=dev)
+            buf[:Bm, :bos].copy_(emb[idx, :bos])
+            buf[:Bm, bos + T:].copy_(emb[idx, bos:])
+            if Bu:
+                buf[Bm:, :L].copy_(emb[uni])
+                buf[Bm:, L:].zero_()
+            _, weights = self.forward(patch_features, out=buf[:Bm, bos:bos + T], batch_index=None if whole else idx.to(torch.int32))
+        else:
+            buf, weights = self._assemble(patch_features, emb, None if whole else idx, uni, bos)
+            T = buf.shape[1] - L
 
         def splice(t, fill_mm, fill_uni):
             if t is None:

@@ -50,6 +50,18 @@ def _p(t: Optional[torch.Tensor]) -> Optional[int]:
     return None if t is None else t.data_ptr()
 
 
+def _rows_in_place(x: torch.Tensor) -> torch.Tensor:
+    """x [B, T, K] as the kernels read or write it in place — channels contiguous, row and batch strides whole 16-byte vectors that keep
+    rows and videos apart, 16-byte aligned base (e.g. the prefix slot ``buf[:, bos:bos + T]`` of the multimodal embedding buffer or its
+    gradient) — or else a contiguous copy."""
+    vec = 8 if x.dtype == torch.bfloat16 else 4
+    B, T, K = x.shape
+    if (x.stride(2) != 1 or x.stride(1) % vec or x.stride(0) % vec or x.data_ptr() % 16
+            or (T > 1 and x.stride(1) < K) or (B > 1 and x.stride(0) < T * x.stride(1))):
+        x = x.contiguous()
+    return x
+
+
 # ---- launch accounting ----------------------------------------------------------------------------------------
 # kernels launched by one call of each entry point (used for bench.py's `gpu_launches` and per-kernel timing)
 KERNELS_PER_CALL = {
@@ -422,25 +434,32 @@ def softmax_weights(
 
 
 def softmax_mix(
-    Vs: Sequence[torch.Tensor], token_length: int, scores: Optional[torch.Tensor] = None, weights: Optional[torch.Tensor] = None
+    Vs: Sequence[torch.Tensor], token_length: int, scores: Optional[torch.Tensor] = None, weights: Optional[torch.Tensor] = None,
+    out: Optional[torch.Tensor] = None,
 ) -> Tuple[torch.Tensor, torch.Tensor]:
     """out[b,t,:] = sum_e w[b,e] V_e[b,t,:] with w = softmax(scores) computed in-kernel (or given `weights`).
 
     Reference: torch.stack + torch.bmm at merv/util/nn_utils.py:503,521.  Returns (out [B,T,K], weights fp32 [B,E]).
+    `out`: optional [B, T, K] destination (any row / batch stride), e.g. the prefix slot of the multimodal embedding buffer; written in
+    place when the kernel can address it (include/merv_fusion.h: merv_softmax_mix_ex), otherwise through a contiguous copy.
     """
     lib = _lib.load()
-    dev = _require_cuda(*Vs, scores, weights)
+    dev = _require_cuda(*Vs, scores, weights, out)
     assert (scores is None) != (weights is None)
     B, _, K = Vs[0].shape
     E = len(Vs)
     Vs = [v.contiguous() for v in Vs]
     with torch.cuda.device(dev):
-        out = torch.empty((B, token_length, K), dtype=Vs[0].dtype, device=dev)
+        dst = torch.empty((B, token_length, K), dtype=Vs[0].dtype, device=dev) if out is None else _rows_in_place(out)
+        assert dst.shape == (B, token_length, K) and dst.dtype == Vs[0].dtype, f"out must be {Vs[0].dtype} [{B}, {token_length}, {K}]"
         if weights is None:
             weights = torch.empty((B, E), dtype=torch.float32, device=dev)
-        _call('merv_softmax_mix', lib.merv_softmax_mix, ptr_array([v.data_ptr() for v in Vs]), i32_array([v.shape[1] for v in Vs]), _p(scores),
-                                   weights.data_ptr(), out.data_ptr(), B, E, token_length, K, dtype_code(Vs[0].dtype), _stream())
-    return out, weights
+        _call('merv_softmax_mix', lib.merv_softmax_mix_ex, ptr_array([v.data_ptr() for v in Vs]), i32_array([v.shape[1] for v in Vs]), _p(scores),
+              weights.data_ptr(), dst.data_ptr(), dst.stride(1), dst.stride(0), B, E, token_length, K, dtype_code(Vs[0].dtype), _stream())
+    if out is not None and dst is not out:
+        out.copy_(dst)
+        dst = out
+    return dst, weights
 
 
 def fused_linear_mix(
@@ -702,9 +721,7 @@ def video_colsum(x: torch.Tensor, scale: float = 1.0) -> torch.Tensor:
     lib = _lib.load()
     dev = _require_cuda(x)
     assert x.dim() == 3
-    vec = 8 if x.dtype == torch.bfloat16 else 4
-    if x.stride(2) != 1 or x.stride(1) % vec or x.stride(0) % vec or x.data_ptr() % 16:
-        x = x.contiguous()
+    x = _rows_in_place(x)
     B, T, K = x.shape
     with torch.cuda.device(dev):
         out = torch.empty((B, K), dtype=torch.float32, device=dev)
@@ -739,19 +756,29 @@ def pair_dot(x: torch.Tensor, y: torch.Tensor, scale: Optional[torch.Tensor] = N
 def wgrad_video(dy: torch.Tensor, x: torch.Tensor, scale: torch.Tensor, w: torch.Tensor, videos: int) -> Tuple[torch.Tensor, torch.Tensor]:
     """(dW [N_out, C] = sum_b scale[b] dy[b]^T x[b],  partials [videos, pair_dot_chunks] of <w, dy[b]^T x[b]>) in ONE tcgen05 pass over
     dy [videos * T, N_out] and x [videos * T, C], both read in place (include/merv_fusion.h: merv_wgrad_video).  `scale` fp32 [videos] (any
-    stride), w [N_out, C] bf16.  T % 64 == 0."""
+    stride), w [N_out, C] bf16.  T % 64 == 0.  dy may also be a [videos, T, N_out] view with any row / batch stride (the gradient of the prefix
+    slot of the multimodal embedding buffer): read in place when TMA can address it (merv_wgrad_video_ex), otherwise copied."""
     lib = _lib.load()
     dev = _require_cuda(dy, x, scale, w)
     assert dy.dtype == x.dtype == w.dtype == torch.bfloat16 and scale.dtype == torch.float32 and scale.dim() == 1 and scale.numel() == videos
-    assert dy.dim() == 2 and x.dim() == 2 and dy.shape[0] == x.shape[0] and dy.shape[0] % videos == 0
-    assert dy.stride(1) == 1 and x.stride(1) == 1 and w.stride(1) == 1 and w.shape == (dy.shape[1], x.shape[1])
-    T = dy.shape[0] // videos
+    if dy.dim() == 3:
+        assert dy.shape[0] == videos
+        dy = _rows_in_place(dy)
+        lddy, dy_bs = dy.stride(1), dy.stride(0)
+        dy2 = dy.shape[1] * videos, dy.shape[2]
+    else:
+        assert dy.dim() == 2 and dy.stride(1) == 1 and dy.shape[0] % videos == 0
+        lddy, dy_bs = dy.stride(0), (dy.shape[0] // videos) * dy.stride(0)
+        dy2 = tuple(dy.shape)
+    assert x.dim() == 2 and dy2[0] == x.shape[0]
+    assert x.stride(1) == 1 and w.stride(1) == 1 and w.shape == (dy2[1], x.shape[1])
+    T = dy2[0] // videos
     N_out, Cc = w.shape
     with torch.cuda.device(dev):
         dW = torch.empty((N_out, Cc), dtype=torch.bfloat16, device=dev)
         partial = torch.empty((videos, lib.merv_pair_dot_chunks()), dtype=torch.float32, device=dev)
         ws = torch.empty(max(int(lib.merv_wgrad_video_workspace(videos, N_out, Cc)), 4), dtype=torch.float32, device=dev)
-        _call('merv_wgrad_video', lib.merv_wgrad_video, dy.data_ptr(), dy.stride(0), x.data_ptr(), x.stride(0), scale.data_ptr(), scale.stride(0),
+        _call('merv_wgrad_video', lib.merv_wgrad_video_ex, dy.data_ptr(), lddy, dy_bs, x.data_ptr(), x.stride(0), scale.data_ptr(), scale.stride(0),
               w.data_ptr(), w.stride(0), dW.data_ptr(), dW.stride(0), partial.data_ptr(), ws.data_ptr(), videos, T, N_out, Cc, _stream())
     return dW, partial
 
@@ -833,7 +860,7 @@ def mix_backward(Vs: Sequence[torch.Tensor], dout: torch.Tensor, weights: torch.
     E, embed = len(Vs), Wk.shape[0]
     dt = Vs[0].dtype
     Vs = [v.contiguous() for v in Vs]
-    dout = dout.contiguous()
+    dout = _rows_in_place(dout)
     assert all(v.shape == (B, T, K) and v.dtype == dt for v in Vs) and dout.shape == (B, T, K) and dout.dtype == dt
     assert weights.dtype == torch.float32 and weights.is_contiguous() and (dweights is None or (dweights.dtype == torch.float32 and dweights.is_contiguous()))
     with torch.cuda.device(dev):
@@ -842,11 +869,12 @@ def mix_backward(Vs: Sequence[torch.Tensor], dout: torch.Tensor, weights: torch.
         dWq = torch.empty((embed, embed), dtype=dt, device=dev)
         dWk = torch.empty((embed, K), dtype=dt, device=dev)
         dbias = torch.empty(3 * embed, dtype=dt, device=dev)
-        n = lib.merv_mix_backward_workspace(B, E, T, K, embed)
+        n = lib.merv_mix_backward_workspace(B, E, T, K, embed)  # every encoder at T tokens: no single-token column sums
         ws = torch.empty(n, dtype=torch.float32, device=dev)
-        _call('merv_mix_backward', lib.merv_mix_backward, ptr_array([v.data_ptr() for v in Vs]), dout.data_ptr(), weights.data_ptr(), _p(dweights),
-              u.data_ptr(), Q.contiguous().data_ptr(), Wq.contiguous().data_ptr(), Wk.contiguous().data_ptr(), in_proj_bias.data_ptr(),
-              ptr_array([d.data_ptr() for d in dVs]), dQ.data_ptr(), dWq.data_ptr(), dWk.data_ptr(), dbias.data_ptr(), ws.data_ptr(), n,
+        _call('merv_mix_backward', lib.merv_mix_backward_strided, ptr_array([v.data_ptr() for v in Vs]), i32_array([T] * E), dout.data_ptr(),
+              dout.stride(1), dout.stride(0), weights.data_ptr(), _p(dweights), u.data_ptr(), 0, None, 0, Q.contiguous().data_ptr(),
+              Wq.contiguous().data_ptr(), Wk.contiguous().data_ptr(), in_proj_bias.data_ptr(),
+              ptr_array([d.data_ptr() for d in dVs]), dQ.data_ptr(), dWq.data_ptr(), dWk.data_ptr(), dbias.data_ptr(), None, ws.data_ptr(), n,
               B, E, T, K, embed, dtype_code(dt), _stream())
     return dVs, dQ, dWq, dWk, dbias
 
@@ -864,7 +892,7 @@ def mix_backward_ex(Vs: Sequence[torch.Tensor], dout: torch.Tensor, weights: tor
     dt = Vs[0].dtype
     Ku = T * K if per_token_u else K
     Vs = [v.contiguous() for v in Vs]
-    dout = dout.contiguous()
+    dout = _rows_in_place(dout)
     assert all(v.shape in ((B, T, K), (B, 1, K)) and v.dtype == dt for v in Vs) and dout.dtype == dt
     assert u.dtype == torch.float32 and u.is_contiguous() and u.numel() == Ku and Wk.shape[1] == Ku
     assert weights.dtype == torch.float32 and weights.is_contiguous() and (dweights is None or (dweights.dtype == torch.float32 and dweights.is_contiguous()))
@@ -880,8 +908,8 @@ def mix_backward_ex(Vs: Sequence[torch.Tensor], dout: torch.Tensor, weights: tor
         dpe = None if pe is None else torch.empty((E, K), dtype=dt, device=dev)
         n = lib.merv_mix_backward_ex_workspace(B, E, T, K, embed, K if per_token_u else 0)
         ws = torch.empty(n, dtype=torch.float32, device=dev)
-        _call('merv_mix_backward_ex', lib.merv_mix_backward_ex, ptr_array([v.data_ptr() for v in Vs]), i32_array([v.shape[1] for v in Vs]),
-              dout.data_ptr(), weights.data_ptr(), _p(dweights), u.data_ptr(), K if per_token_u else 0, _p(pe), 0 if pe is None else pe.stride(0),
+        _call('merv_mix_backward_ex', lib.merv_mix_backward_strided, ptr_array([v.data_ptr() for v in Vs]), i32_array([v.shape[1] for v in Vs]),
+              dout.data_ptr(), dout.stride(1), dout.stride(0), weights.data_ptr(), _p(dweights), u.data_ptr(), K if per_token_u else 0, _p(pe), 0 if pe is None else pe.stride(0),
               Q.contiguous().data_ptr(), Wq.contiguous().data_ptr(), Wk.contiguous().data_ptr(), in_proj_bias.data_ptr(),
               ptr_array([d.data_ptr() for d in dVs]), dQ.data_ptr(), dWq.data_ptr(), dWk.data_ptr(), dbias.data_ptr(), _p(dpe), ws.data_ptr(), n,
               B, E, T, K, embed, dtype_code(dt), _stream())
@@ -897,7 +925,7 @@ def scalar_mix_backward(Vs: Sequence[torch.Tensor], dout: torch.Tensor, weights:
     B, T, K = dout.shape
     E, dt = len(Vs), dout.dtype
     Vs = [v.contiguous() for v in Vs]
-    dout = dout.contiguous()
+    dout = _rows_in_place(dout)
     assert all(v.shape == (B, T, K) and v.dtype == dt for v in Vs), "every encoder must have the [B, T, K] shape and dtype of dout"
     assert weights.dtype == torch.float32 and weights.is_contiguous() and weights.numel() == E
     assert dweights is None or (dweights.dtype == torch.float32 and dweights.is_contiguous() and dweights.numel() == E)
@@ -906,7 +934,8 @@ def scalar_mix_backward(Vs: Sequence[torch.Tensor], dout: torch.Tensor, weights:
         dscalar = torch.empty(E, dtype=torch.float32, device=dev)
         n = lib.merv_scalar_mix_backward_workspace(B, E, K)
         ws = torch.empty(max(n, 1), dtype=torch.float32, device=dev)
-        _call('merv_scalar_mix_backward', lib.merv_scalar_mix_backward, ptr_array([v.data_ptr() for v in Vs]), dout.data_ptr(), weights.data_ptr(),
+        _call('merv_scalar_mix_backward', lib.merv_scalar_mix_backward_strided, ptr_array([v.data_ptr() for v in Vs]), dout.data_ptr(), dout.stride(1),
+              dout.stride(0), weights.data_ptr(),
               _p(dweights), ptr_array([d.data_ptr() for d in dVs]), dscalar.data_ptr(), ws.data_ptr(), n, B, E, T, K, dtype_code(dt), _stream())
     return dVs, dscalar
 
