@@ -161,7 +161,8 @@ __device__ __forceinline__ void gemm_body(const TensorMaps& maps, const GemmPara
   auto seg_first = [&](int q) { return kVid ? int(((long long)q * p.nseg) / p.vid_parts) : (q == 0 ? 0 : p.nseg); };
 
   if (warp == 0 && lane == 0) {
-    for (int s = 0; s < p.nseg; ++s) {
+    // kVid: p.nseg counts videos, but every video reads the one map pair a[0] / b[0] (a and b hold only MERV_MAX_SEGMENTS maps)
+    for (int s = 0; s < (kVid ? 1 : p.nseg); ++s) {
       prefetch_tmap(&maps.a[s]);
       prefetch_tmap(&maps.b[s]);
     }
