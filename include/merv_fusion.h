@@ -249,13 +249,6 @@ int merv_fused_linear_mix_multicast(const void* const* A, const int64_t* lda, co
  *   W, ldw, bias, c: last-layer weights [N, C_e], biases [N] (bf16) and score constants c_e (fp32 [1]) per encoder
  *   scores, weights: workspaces fp32 [B, E]; bias_mix fp32 [B, N]; weights_bf16 (optional) bf16 [B, E] copy of weights
  *   out            : bf16 [B, rows_per_video, N] with row stride ldo and batch stride out_batch_stride (0 = contiguous)
- * Pool assist (large batches of the shipped encoder shapes: square 16 x 16 / 14 x 14 patch grids -> 8 x 8, one input frame per output
- * frame, sync_ws given, B > assist_head): the pool is HBM-bound with an idle tensor pipe and the GEMM tensor-bound with idle HBM, so
- * only the first assist_head videos go through the standalone pool + scores kernels; the rest are pooled, scored and soft-maxed by two
- * spare warps of every GEMM CTA while the tensor cores multiply the videos before them (per-video ready flags, release / acquire).
- * Pooled tokens, scores, weights and the prefix are bit-identical to the three-launch path.  Opt-in: MERV_POOL_ASSIST=1 in the
- * environment (read per call; measured neutral-to-slower on B200 under the power cap, see DESIGN.md section 10); MERV_ASSIST_HEAD=n
- * overrides the head.
  * ------------------------------------------------------------------------------------------------------- */
 typedef struct {
   int32_t num_encoders, B, N, rows_per_video;
@@ -271,11 +264,9 @@ typedef struct {
   void* weights_bf16; /* may be NULL */
   void* out;
   int64_t ldo, out_batch_stride;
-  /* ABI v5: workspace of the in-GEMM pooling ("pool assist", see below), int32 [sync_ws_ints] on the device with
-   * sync_ws_ints >= 4 + 2 * B, or NULL (then the three-launch path always runs).  Contents need no initialisation. */
-  int32_t* sync_ws;
-  int32_t sync_ws_ints;
-  int32_t assist_head; /* videos pooled by the standalone kernel before the GEMM starts; 0 = library default */
+  /* reserved: ignored by the library; they keep the ABI v5 layout, so any value a v5 caller stores here is harmless */
+  int32_t* reserved_ptr_;
+  int32_t reserved_[2];
 } merv_fused_desc;
 
 int merv_fused_forward(const merv_fused_desc* d, void* stream);

@@ -49,7 +49,7 @@ class FusedDesc(C.Structure):
         ("W", c_void_p * 4), ("ldw", c_int64 * 4), ("bias", c_void_p * 4), ("c", c_void_p * 4),
         ("scores", c_void_p), ("weights", c_void_p), ("bias_mix", c_void_p), ("weights_bf16", c_void_p),
         ("out", c_void_p), ("ldo", c_int64), ("out_batch_stride", c_int64),
-        ("sync_ws", c_void_p), ("sync_ws_ints", c_int32), ("assist_head", c_int32),
+        ("reserved_ptr_", c_void_p), ("reserved_", c_int32 * 2),
     ]
 
 

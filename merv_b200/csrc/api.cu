@@ -4,7 +4,6 @@
 #include <mutex>
 
 #include "common.cuh"
-#include "pool_assist.cuh"
 #include "tmap.cuh"
 
 namespace merv {
@@ -229,12 +228,9 @@ extern "C" int merv_concat_linear(const void* const* A, const int64_t* lda, cons
                              static_cast<cudaStream_t>(stream));
 }
 
-// Pool assist policy.  OFF unless MERV_POOL_ASSIST=1: measured on B200 (profiles/r2_assist_lab*.json, DESIGN.md §10) it is bit-identical
-// to the three-launch path but not faster — two 64-register warps per SM pool one video per ~35 us (a single warp issues one instruction
-// per ~4 cycles whatever the instruction), the tensor cores need one per 20 us, and under the power cap the GEMM slows down by what the
-// pooling draws.  Batches below kAssistMinVideos always keep the three-launch path; the first kAssistDefaultHead videos are pooled up
-// front (at the measured rates the pooling warps keep up with the tensor cores for roughly the last 24 of 64 videos).
-static constexpr int kAssistMinVideos = 16, kAssistDefaultHead = 40;
+// callers built against ABI v5 lay the descriptor out this way (LP64)
+static_assert(sizeof(merv_fused_desc) == 744 && offsetof(merv_fused_desc, reserved_ptr_) == 728 && offsetof(merv_fused_desc, reserved_) == 736,
+              "merv_fused_desc must keep its ABI v5 layout");
 
 extern "C" int merv_fused_forward(const merv_fused_desc* d, void* stream) {
   MERV_REQUIRE(d != nullptr, MERV_E_ARG, "merv_fused_forward: desc is NULL");
@@ -259,34 +255,13 @@ extern "C" int merv_fused_forward(const merv_fused_desc* d, void* stream) {
   // scores kernel is resident (blocked in griddepcontrol.wait) when the pool's last CTA retires, and the GEMM's CTAs run their
   // prologue (barriers, TMEM allocation, tensor-map prefetch) on every SM the pool has left — no launch gap between the stages.
   const bool pdl = pdl_enabled();
-  // Pool assist (pool_assist.cuh): only the first `head` videos take the standalone pool + scores kernels; the GEMM's spare warps pool,
-  // score and soft-max the others while the tensor cores work on the videos before them.
-  AssistArgs assist_args;
-  const AssistArgs* assist = nullptr;
-  int pool_B = d->B;
-  {
-    const char* on = getenv("MERV_POOL_ASSIST");
-    int head = d->assist_head > 0 ? d->assist_head : kAssistDefaultHead;
-    if (const char* h = getenv("MERV_ASSIST_HEAD")) head = atoi(h);
-    if (on != nullptr && on[0] == '1' && d->sync_ws != nullptr && d->B >= kAssistMinVideos && head >= 1 && head < d->B) {
-      int rc = MERV_OK;
-      if (build_pool_assist(d, head, &assist_args, &rc)) {
-        assist = &assist_args;
-        pool_B = head;
-      } else if (rc != MERV_OK) {
-        return rc;
-      }
-    }
-  }
-  if (int rc = merv_pool3d(d->pool, E, pool_B, MERV_BF16, 0, stream)) return rc;
-  if (int rc = launch_scores_softmax_weights(partial, d->parts, d->c, d->bias, d->scores, d->weights, d->weights_bf16, d->bias_mix, pool_B, E,
-                                             d->rows_per_video, d->N, static_cast<cudaStream_t>(stream), pdl, assist ? d->sync_ws : nullptr,
-                                             assist ? ASSIST_SYNC_HEADER + 2 * d->B : 0))
+  if (int rc = merv_pool3d(d->pool, E, d->B, MERV_BF16, 0, stream)) return rc;
+  if (int rc = launch_scores_softmax_weights(partial, d->parts, d->c, d->bias, d->scores, d->weights, d->weights_bf16, d->bias_mix, d->B, E,
+                                             d->rows_per_video, d->N, static_cast<cudaStream_t>(stream), pdl))
     return rc;
   MERV_REQUIRE(d->B * (long long)d->rows_per_video <= 0x7fffffffLL, MERV_E_SHAPE, "merv_fused_forward: B * rows_per_video overflows");
   GemmSegment seg[MERV_MAX_SEGMENTS];
   for (int e = 0; e < E; ++e) seg[e] = GemmSegment{A[e], lda[e], d->W[e], d->ldw[e], K[e]};
   return launch_gemm_tcgen05(seg, E, d->weights, d->bias_mix, d->rows_per_video, nullptr, MERV_ACT_NONE, nullptr, nullptr, d->out, d->ldo,
-                             d->out_batch_stride, d->B * d->rows_per_video, d->N, 0, static_cast<cudaStream_t>(stream), nullptr, 0, pdl, nullptr,
-                             assist);
+                             d->out_batch_stride, d->B * d->rows_per_video, d->N, 0, static_cast<cudaStream_t>(stream), nullptr, 0, pdl);
 }

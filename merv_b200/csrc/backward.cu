@@ -1482,7 +1482,7 @@ extern "C" int merv_wgrad_video_ex(const void* dY, int64_t lddy, int64_t dy_batc
   const bool packed = dy_batch_stride == (int64_t)tokens_per_video * lddy;  // the 2-D map of the contiguous case
   WgradVideoArgs vid = {videos, tokens_per_video / 64, scale, scale_stride, W, ldw, workspace, split, partial, packed ? 0 : (long long)dy_batch_stride};
   if (int rc = launch_gemm_tcgen05(&seg, 1, nullptr, nullptr, N_out, nullptr, MERV_ACT_NONE, nullptr, nullptr, dW, lddw, 0, N_out, C, 0, s, nullptr, 0,
-                                   false, nullptr, nullptr, &vid))
+                                   false, nullptr, &vid))
     return rc;
   if (split > 1) {
     const long long vecs = (long long)N_out * (C / 4);

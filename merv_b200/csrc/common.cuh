@@ -30,7 +30,6 @@ inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 
 int require_sm100();   // MERV_OK or MERV_E_ARCH for the current device (cached per device)
 int sm_count();        // SM count of the current device
 
-struct AssistArgs;  // pool_assist.cuh
 // Weight gradient over per-video segments (gemm_tcgen05.cu, kVid): the single (A, W) segment handed to launch_gemm_tcgen05 covers all
 // `videos` x kblocks_per_video k-blocks; the kernel drains the accumulator once per video.
 struct WgradVideoArgs {
@@ -64,10 +63,10 @@ struct GemmSegment {
 int launch_gemm_tcgen05(const GemmSegment* seg, int nseg, const float* seg_scale, const float* bias_rows, int rows_per_video,
                         const void* bias, int act, const float* rowdot_vec, float* rowdot_out, void* Y, long long ldy, long long y_batch_stride,
                         int M, int N, int max_ctas, cudaStream_t stream, void* const* extra_out = nullptr, int num_extra = 0, bool pdl = false,
-                        void* mc_out = nullptr, const struct AssistArgs* assist = nullptr, const WgradVideoArgs* vid = nullptr);
+                        void* mc_out = nullptr, const WgradVideoArgs* vid = nullptr);
 int launch_scores_softmax_weights(const float* const* partial, const int32_t* count, const float* const* c, const void* const* bias,
                                   float* scores, float* weights, void* weights_bf16, float* bias_mix, int B, int E, int T, int N,
-                                  cudaStream_t stream, bool pdl, int* sync_ws = nullptr, int sync_ints = 0);
+                                  cudaStream_t stream, bool pdl);
 // tcgen05 cross attention (attention_tcgen05.cu): bf16, at most 128 queries and 256 keys per frame, head_dim % 32 == 0 and <= 128
 bool attention_tcgen05_supported(int n_q, int n_kv, int heads, int hd, long long ldq, long long q_batch_stride, long long ldkv, long long ldo);
 int launch_attention_tcgen05(const void* q, long long ldq, long long q_batch_stride, const void* kv, long long ldkv, void* out, long long ldo,

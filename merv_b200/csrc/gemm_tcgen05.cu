@@ -8,7 +8,6 @@
 //                           nn_utils.py:31-32,503,521, without ever writing the per-encoder projections to HBM)
 //   merv_gemm_ex           the same with either operand stored transposed (MN-major: the backward's dX = dY W, dW = dY^T X)
 //   merv_wgrad_video       dW = sum_b w[b] dY[b]^T X[b] and <W, dY[b]^T X[b]> per video: the accumulator is drained once per video
-//   (opt-in) the fused forward with the pooling of the following videos done by its two spare warps (pool_assist.cuh)
 //
 // Tile 128 x 256 x 64 per CTA, as a CTA pair (cluster 2 x 1, cta_group::2, UMMA 256x256x16: each CTA loads its 128 rows of A and HALF of
 // the W tile, 6-stage ring of 32 KB) or as a single CTA (UMMA 128x256x16, 4 stages of 48 KB); TMA -> shared memory with 128-byte swizzle;
@@ -19,17 +18,16 @@
 //
 //   warp 0      TMA producer   \  warp-uniform loops; one lane issues under elect.sync (lane-0 guards made the compiler wrap every
 //   warp 1      tcgen05.mma issuer /  UTMALDG / UTCHMMA in an ELECT / R2UR waterfall loop: tensor pipe 84 % -> 95 % of elapsed without them)
-//   warp 2      TMEM allocator (+ pooling warp of the opt-in pool assist)
-//   warp 3      idle           (+ pooling warp of the opt-in pool assist)
+//   warp 2      TMEM allocator
+//   warp 3      idle
 //   warps 4-19  epilogue: warp w owns TMEM lanes 32*(w%4)..+31 and columns 64*((w-4)/4)..+63 of the tile
 // Template parameters: kCtas (1 | 2), kWide (128-byte-row output boxes: NVLink peer stores, short contractions), kGelu, kMaj (operand
-// majorness, compile-time), kAssist, kVid.  Measured: fused forward 1614 TFLOP/s in the bench = 0.98 of the burst cuBLAS peak (DESIGN.md 5.2).
+// majorness, compile-time), kVid, kDy3.  Measured: fused forward 1614 TFLOP/s in the bench = 0.98 of the burst cuBLAS peak (DESIGN.md 5.2).
 #include <cuda.h>
 
 #include <cstdlib>
 
 #include "common.cuh"
-#include "pool_assist.cuh"
 #include "tcgen05_util.cuh"
 #include "tmap.cuh"
 
@@ -42,19 +40,15 @@ constexpr int EPI_WARPS = 16;                          // 4 per scheduler: the e
 constexpr int OUT_GROUPS = EPI_WARPS / 4;              // 4 groups of 4 warps, one staging box each
 // kWide (the fused all-gather variant): output boxes of 128-byte rows instead of 64-byte rows — NVLink peer writes are
 // packetised per box row, and 64-byte payloads only reach ~380 GB/s of egress — paid for with one ring stage.
-// kAssist (pool_assist.cuh): one ring stage becomes the quarter-slab buffers of the two pooling warps.
-template <int kCtas, bool kWide, bool kAssist = false> struct Cfg {
-  static_assert(!kAssist || (kCtas == 2 && !kWide), "the pooling warps ride on the CTA-pair forward kernel");
-  static constexpr int STAGES = (kCtas == 1 ? 4 : 6) - (kWide ? 1 : 0) - (kAssist ? 1 : 0);
+template <int kCtas, bool kWide> struct Cfg {
+  static constexpr int STAGES = (kCtas == 1 ? 4 : 6) - (kWide ? 1 : 0);
   static constexpr int B_ROWS = BN / kCtas;
   static constexpr int B_BYTES = B_ROWS * BK * 2;
   static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
   static constexpr int RING_BYTES = STAGES * STAGE_BYTES;  // 192 KB (144 / 160 KB when wide)
   static constexpr int OUT_BOX_COLS = kWide ? 64 : 32;      // one staged output box: 128 rows x 32 (64) bf16, 64B (128B) swizzle
   static constexpr int OUT_BOX_BYTES = BM * OUT_BOX_COLS * 2;
-  static constexpr int ASSIST_BYTES = kAssist ? ASSIST_SMEM_BYTES : 0;
-  static_assert(!kAssist || ASSIST_SMEM_BYTES == STAGE_BYTES, "the pooling buffers take exactly the ring stage given up");
-  static constexpr int SMEM_BYTES = 1024 /*align slack*/ + RING_BYTES + OUT_GROUPS * OUT_BOX_BYTES + ASSIST_BYTES + 256 /*barriers*/;
+  static constexpr int SMEM_BYTES = 1024 /*align slack*/ + RING_BYTES + OUT_GROUPS * OUT_BOX_BYTES + 256 /*barriers*/;
   static_assert(RING_BYTES % 1024 == 0 && OUT_BOX_BYTES % 1024 == 0, "swizzle atoms need 1024-byte aligned boxes");
   static_assert(SMEM_BYTES <= 232448, "227 KB of shared memory per CTA");
 };
@@ -131,9 +125,9 @@ struct TensorMaps {
 // (scripts/gpu_mn_pair_lab.py).
 // kDy3 (kVid only): the A operand (dY, MN-major) is a 3-D map (N_out columns, token in video, video), so video b's rows may start at any
 // 16-byte aligned batch stride — the gradient of a prefix slot inside the [B, L + T, N] multimodal embedding buffer, read in place.
-template <int kCtas, bool kWide, bool kGelu, int kMaj, bool kAssist, bool kVid = false, bool kDy3 = false>
-__device__ __forceinline__ void gemm_body(const TensorMaps& maps, const GemmParams& p, const AssistArgs* ap) {
-  using C = Cfg<kCtas, kWide, kAssist>;
+template <int kCtas, bool kWide, bool kGelu, int kMaj, bool kVid = false, bool kDy3 = false>
+__device__ __forceinline__ void gemm_body(const TensorMaps& maps, const GemmParams& p) {
+  using C = Cfg<kCtas, kWide>;
   constexpr int STAGES = C::STAGES, STAGE_BYTES = C::STAGE_BYTES, RING_BYTES = C::RING_BYTES;
   constexpr int OUT_BOX_COLS = C::OUT_BOX_COLS, OUT_BOX_BYTES = C::OUT_BOX_BYTES;
   extern __shared__ uint8_t smem_raw[];
@@ -141,15 +135,12 @@ __device__ __forceinline__ void gemm_body(const TensorMaps& maps, const GemmPara
   const uint32_t tiles_addr = (raw_addr + 1023u) & ~1023u;  // SWIZZLE_128B atoms need 1024-byte alignment
   uint8_t* tiles = smem_raw + (tiles_addr - raw_addr);
   const uint32_t stage_out_addr = tiles_addr + RING_BYTES;  // 4 x 8 KB, 1024-byte aligned
-  const uint32_t assist_addr = stage_out_addr + OUT_GROUPS * OUT_BOX_BYTES;  // kAssist: 2 warps x 2 quarter slabs
-  uint64_t* bars = reinterpret_cast<uint64_t*>(tiles + RING_BYTES + OUT_GROUPS * OUT_BOX_BYTES + C::ASSIST_BYTES);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(tiles + RING_BYTES + OUT_GROUPS * OUT_BOX_BYTES);
   const uint32_t full_bar = smem_u32(bars);                  // [STAGES]
   const uint32_t empty_bar = full_bar + 8 * STAGES;          // [STAGES]
   const uint32_t tfull_bar = empty_bar + 8 * STAGES;         // [2]
   const uint32_t tempty_bar = tfull_bar + 16;                // [2]
   uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 2 * STAGES + 4);
-  const uint32_t assist_bar = full_bar + 8 * (2 * STAGES + 4) + 16;  // [ASSIST_WARPS][2], behind the TMEM pointer
-  static_assert(8 * (2 * 6 + 4) + 16 + 8 * 2 * ASSIST_WARPS <= 256, "barrier block");
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t rank = kCtas == 2 ? cluster_ctarank() : 0u;  // 0 = leader of the pair
@@ -177,8 +168,6 @@ __device__ __forceinline__ void gemm_body(const TensorMaps& maps, const GemmPara
       mbar_init(tfull_bar + 8 * i, 1);
       mbar_init(tempty_bar + 8 * i, EPI_WARPS * kCtas);  // in a pair, both CTAs' epilogue warps arrive on the leader's barrier
     }
-    if constexpr (kAssist)
-      for (int i = 0; i < 2 * ASSIST_WARPS; ++i) mbar_init(assist_bar + 8 * i, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
   }
@@ -206,34 +195,9 @@ __device__ __forceinline__ void gemm_body(const TensorMaps& maps, const GemmPara
       // ===== TMA producer (one elected lane issues; the loop itself is warp-uniform) =====
       uint32_t it = 0;
       const uint32_t leader_full = kCtas == 2 ? mapa_rank(full_bar, 0) : full_bar;
-      int ready_video = -1;  // kAssist: last video whose ready flag this thread has acquired
       for (int item = unit; item < total_items; item += num_units) {
         const int tile = kVid ? item % total_tiles : item, part = kVid ? item / total_tiles : 0;
         const int m_blk = tile / p.n_blocks, n_blk = tile % p.n_blocks;
-        if constexpr (kAssist) {
-          // the pooled rows of this CTA's half of the tile (and the video's mixing weights / bias row the epilogue will read) are
-          // produced inside this launch by the pooling warps of whatever CTAs are resident: acquire the video's flag first
-          const int video = ((m_blk * kCtas + int(rank)) * BM) / p.rows_per_video;
-          if (video != ready_video) {
-            // (every lane of the warp-uniform producer acquires and fences: whichever lane elect.sync picks has done both itself)
-            if (video >= ap->head && !(MERV_ASSIST_PROFILE && (ap->dbg & 8))) {
-              const int* flag = ap->sync + ASSIST_SYNC_HEADER + ap->B + video;
-              if (ld_acquire_gpu(flag) == 0) {
-                const unsigned long long t0 = globaltimer_ns();
-                while (ld_acquire_gpu(flag) == 0) {
-                  __nanosleep(128);
-                  if (globaltimer_ns() - t0 > 4000000000ull) {
-                    printf("merv gemm: pool assist never published video %d (block %d)\n", video, blockIdx.x);
-                    __trap();
-                  }
-                }
-              }
-              fence_proxy_async_all();  // generic-proxy stores of the pooling warps -> this thread's async-proxy (TMA) reads
-            }
-            __syncwarp();
-            ready_video = video;
-          }
-        }
         for (int s0 = seg_first(part); s0 < seg_first(part + 1); ++s0) {
           const int s = kVid ? 0 : s0;                       // kVid: every video reads the same pair of tensors ...
           const int nkb = kVid ? p.vid_kblocks : p.kblocks[s];
@@ -318,12 +282,6 @@ __device__ __forceinline__ void gemm_body(const TensorMaps& maps, const GemmPara
           }
         }
       }
-    } else if (kAssist && warp >= 2) {
-      // ===== pooling warps (pool_assist.cuh): pool, score and soft-max the videos ahead of the tiles being multiplied =====
-      if constexpr (kAssist)
-        if (!(MERV_ASSIST_PROFILE && (ap->dbg & 16)))
-        assist_warp_loop(*ap, assist_addr + uint32_t(warp - 2) * 2u * ASSIST_QUARTER_BYTES, assist_bar + 16u * uint32_t(warp - 2), lane,
-                         int(blockIdx.x) * ASSIST_WARPS + (warp - 2));
     }
   } else {
     // Register redistribution happens INSIDE the CTA's launch-time allocation (640 threads x 96 = 61440): warps 0-3 give
@@ -366,7 +324,7 @@ __device__ __forceinline__ void gemm_body(const TensorMaps& maps, const GemmPara
               Vec16<__nv_bfloat16>::unpack(__ldg(reinterpret_cast<const uint4*>(p.bias + n)), b);
             } else if (p.bias_rows != nullptr) {
               const float4* br = reinterpret_cast<const float4*>(p.bias_rows + (long long)video * p.N + n);
-              const float4 b0 = kAssist ? __ldcg(br) : __ldg(br), b1 = kAssist ? __ldcg(br + 1) : __ldg(br + 1);
+              const float4 b0 = __ldg(br), b1 = __ldg(br + 1);
               b[0] = b0.x; b[1] = b0.y; b[2] = b0.z; b[3] = b0.w; b[4] = b1.x; b[5] = b1.y; b[6] = b1.z; b[7] = b1.w;
             } else {
 #pragma unroll
@@ -457,11 +415,8 @@ __device__ __forceinline__ void gemm_body(const TensorMaps& maps, const GemmPara
           const uint32_t buf = acc_it & 1u, aph = (acc_it >> 1) & 1u;
           float scale = 1.0f;
           if constexpr (kVid) scale = p.seg_scale ? __ldg(p.seg_scale + (long long)s * p.seg_scale_stride) : 1.0f;
-          else if constexpr (!kAssist) scale = p.seg_scale ? __ldg(p.seg_scale + (long long)video * p.nseg + s) : 1.0f;
+          else scale = p.seg_scale ? __ldg(p.seg_scale + (long long)video * p.nseg + s) : 1.0f;
           mbar_wait(tfull_bar + 8 * buf, aph);
-          // pool assist: the video's mixing weights are written inside this launch; the full accumulator implies (mbarrier chain from
-          // the producer's acquire) that they are published — read them from L2
-          if constexpr (kAssist) scale = __ldcg(p.seg_scale + (long long)video * p.nseg + s);
           tc_fence_after();
           const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + buf * BN + h * EPI_COLS;
           if constexpr (kVid) {
@@ -543,28 +498,21 @@ __device__ __forceinline__ void gemm_body(const TensorMaps& maps, const GemmPara
 template <int kCtas, bool kWide, bool kGelu, int kMaj = 0>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_bf16_tcgen05_kernel(const __grid_constant__ TensorMaps maps, const __grid_constant__ GemmParams p) {
-  gemm_body<kCtas, kWide, kGelu, kMaj, false>(maps, p, nullptr);
+  gemm_body<kCtas, kWide, kGelu, kMaj>(maps, p);
 }
 
 // weight gradient over per-video segments (single CTA, MN-major operands): dW = sum_b scale[b] dY[b]^T X[b] and <W, dY[b]^T X[b]> per video
 template <int kCtas>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_wgrad_video_tcgen05_kernel(const __grid_constant__ TensorMaps maps, const __grid_constant__ GemmParams p) {
-  gemm_body<kCtas, false, false, 3, false, true>(maps, p, nullptr);
+  gemm_body<kCtas, false, false, 3, true>(maps, p);
 }
 
 // the same with dY read through the 3-D (batch-strided) map: a separate kernel, so the contiguous one above keeps its code
 template <int kCtas>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_wgrad_video_strided_tcgen05_kernel(const __grid_constant__ TensorMaps maps, const __grid_constant__ GemmParams p) {
-  gemm_body<kCtas, false, false, 3, false, true, true>(maps, p, nullptr);
-}
-
-// the fused forward GEMM (CTA pair, K-major operands) whose two spare warps pool the videos ahead of the tiles (pool_assist.cuh)
-__global__ void __launch_bounds__(GEMM_THREADS, 1)
-gemm_pool_assist_tcgen05_kernel(const __grid_constant__ TensorMaps maps, const __grid_constant__ GemmParams p,
-                                const __grid_constant__ AssistArgs assist) {
-  gemm_body<2, false, false, 0, true>(maps, p, &assist);
+  gemm_body<kCtas, false, false, 3, true, true>(maps, p);
 }
 
 // ---- host side ---------------------------------------------------------------------------------------------
@@ -594,16 +542,20 @@ static int make_tmap(CUtensorMap* map, const void* base, long long rows, long lo
   return encode_tmap_cached(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, base, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
-template <int kCtas, bool kWide, bool kGelu, int kMaj = 0>
-static int launch_variant(cudaLaunchConfig_t& cfg, const TensorMaps& maps, const GemmParams& p) {
-  constexpr int smem = Cfg<kCtas, kWide>::SMEM_BYTES;
-  static const cudaError_t attr_rc =  // once per variant (thread-safe static init)
-      cudaFuncSetAttribute(gemm_bf16_tcgen05_kernel<kCtas, kWide, kGelu, kMaj>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  MERV_REQUIRE(attr_rc == cudaSuccess, MERV_E_CUDA, "cudaFuncSetAttribute(max dynamic smem=%d) failed: %s", smem, cudaGetErrorString(attr_rc));
-  cfg.dynamicSmemBytes = smem;
-  MERV_CUDA_OK(cudaLaunchKernelEx(&cfg, gemm_bf16_tcgen05_kernel<kCtas, kWide, kGelu, kMaj>, maps, p));
+template <auto kKernel, int kSmem>
+static int launch_kernel(cudaLaunchConfig_t& cfg, const TensorMaps& maps, const GemmParams& p) {
+  static const cudaError_t attr_rc =  // once per kernel (thread-safe static init)
+      cudaFuncSetAttribute(kKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
+  MERV_REQUIRE(attr_rc == cudaSuccess, MERV_E_CUDA, "cudaFuncSetAttribute(max dynamic smem=%d) failed: %s", kSmem, cudaGetErrorString(attr_rc));
+  cfg.dynamicSmemBytes = kSmem;
+  MERV_CUDA_OK(cudaLaunchKernelEx(&cfg, kKernel, maps, p));
   MERV_CUDA_OK(cudaGetLastError());
   return MERV_OK;
+}
+
+template <int kCtas, bool kWide, bool kGelu, int kMaj = 0>
+static int launch_variant(cudaLaunchConfig_t& cfg, const TensorMaps& maps, const GemmParams& p) {
+  return launch_kernel<gemm_bf16_tcgen05_kernel<kCtas, kWide, kGelu, kMaj>, Cfg<kCtas, kWide>::SMEM_BYTES>(cfg, maps, p);
 }
 
 static int wgrad_video_ctas(int M) { return gemm_cta_group(M, true); }
@@ -641,7 +593,7 @@ int wgrad_video_split(int M, int N, int videos) {
 int launch_gemm_tcgen05(const GemmSegment* seg, int nseg, const float* seg_scale, const float* bias_rows, int rows_per_video,
                         const void* bias, int act, const float* rowdot_vec, float* rowdot_out, void* Y, long long ldy, long long y_batch_stride,
                         int M, int N, int max_ctas, cudaStream_t stream, void* const* extra_out, int num_extra, bool pdl, void* mc_out,
-                        const AssistArgs* assist, const WgradVideoArgs* vid) {
+                        const WgradVideoArgs* vid) {
   MERV_REQUIRE(nseg >= 1 && nseg <= MERV_MAX_SEGMENTS, MERV_E_ARG, "gemm: nseg=%d not in [1,%d]", nseg, MERV_MAX_SEGMENTS);
   MERV_REQUIRE(M > 0 && N > 0, MERV_E_SHAPE, "gemm: M=%d N=%d", M, N);
   MERV_REQUIRE(N % 8 == 0 && ldy % 8 == 0 && ldy >= N, MERV_E_ALIGN, "gemm: N=%d and ldy=%lld must be multiples of 8 (16-byte rows)", N, ldy);
@@ -657,21 +609,18 @@ int launch_gemm_tcgen05(const GemmSegment* seg, int nseg, const float* seg_scale
     any_mn = any_mn || seg[i].a_mn || seg[i].b_mn;
     a_mn_any = a_mn_any || seg[i].a_mn;
   }
-  const int ctas = assist != nullptr ? 2 : vid != nullptr ? wgrad_video_ctas(M) : gemm_cta_group(M, a_mn_any);
+  const int ctas = vid != nullptr ? wgrad_video_ctas(M) : gemm_cta_group(M, a_mn_any);
   // majorness is compiled into the kernel (kMaj): one choice per launch
   for (int i = 1; i < nseg; ++i)
     MERV_REQUIRE(seg[i].a_mn == seg[0].a_mn && seg[i].b_mn == seg[0].b_mn, MERV_E_ARG, "gemm: all segments of a launch share the operand majorness");
   if (vid != nullptr) {
-    MERV_REQUIRE(nseg == 1 && seg[0].a_mn && seg[0].b_mn && act == MERV_ACT_NONE && num_extra == 0 && mc_out == nullptr && assist == nullptr &&
+    MERV_REQUIRE(nseg == 1 && seg[0].a_mn && seg[0].b_mn && act == MERV_ACT_NONE && num_extra == 0 && mc_out == nullptr &&
                      bias == nullptr && bias_rows == nullptr && rowdot_vec == nullptr && seg_scale == nullptr,
                  MERV_E_ARG, "gemm: the per-video weight gradient takes one MN-major segment and no epilogue options");
     MERV_REQUIRE(vid->videos >= 1 && vid->kblocks_per_video >= 1 && (long long)vid->videos * vid->kblocks_per_video * BK == seg[0].K, MERV_E_SHAPE,
                  "gemm: %d videos x %d k-blocks of %d do not cover K=%d", vid->videos, vid->kblocks_per_video, BK, seg[0].K);
     MERV_REQUIRE(vid->W && vid->dot_out && vid->ldw >= N && vid->ldw % 8 == 0 && aligned16(vid->W), MERV_E_ARG, "gemm: per-video weight gradient: W / dot_out");
   }
-  MERV_REQUIRE(assist == nullptr || (!any_mn && M > BM && num_extra == 0 && mc_out == nullptr && act == MERV_ACT_NONE && seg_scale && bias_rows &&
-                                     rowdot_vec == nullptr),
-               MERV_E_ARG, "gemm: pool assist rides on the plain fused forward GEMM only");
   // wide output boxes only pay when the kernel is NVLink-bound: with one peer (2 GPUs) it still is tensor-bound and the
   // ring stage given up for the staging costs more (2.05 vs 1.95 ms); from 2 peers on the link decides (3.15 vs 4.36 ms
   // at 4 GPUs).  MERV_GEMM_WIDE_OUT=0|1 overrides, for the tests.
@@ -682,9 +631,8 @@ int launch_gemm_tcgen05(const GemmSegment* seg, int nseg, const float* seg_scale
   // the single staging box (the second pass waits for the first pass's TMA store to have read it).  One 128-byte-row pass per tile
   // instead: M = 262144, K = 768 (SigLIP single) on the pair 1199 -> 1283 TFLOP/s; at K = 1024 the ring stage given up costs more
   // (1374 -> 1350), at K = 3584 too (profiles/r2b_gemm_lab_wide.json)
-  if (ctas == 2 && total_k <= 832 && !any_mn && vid == nullptr && assist == nullptr) wide = true;
+  if (ctas == 2 && total_k <= 832 && !any_mn && vid == nullptr) wide = true;
   if (const char* e = getenv("MERV_GEMM_WIDE_OUT")) wide = e[0] == '1';
-  if (assist != nullptr) wide = false;
   MERV_REQUIRE(act == MERV_ACT_NONE || act == MERV_ACT_GELU_ERF, MERV_E_ARG, "gemm: unknown activation %d", act);
   if (act != MERV_ACT_NONE) {
     MERV_REQUIRE(nseg == 1 && seg_scale == nullptr, MERV_E_ARG, "gemm: an activation needs a single segment without per-video scales");
@@ -791,48 +739,13 @@ int launch_gemm_tcgen05(const GemmSegment* seg, int nseg, const float* seg_scale
   attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = pdl ? 2 : 1;
-  if (vid != nullptr && vid->dy_batch_stride != 0) {
-    if (ctas == 2) {
-      constexpr int smem = Cfg<2, false>::SMEM_BYTES;
-      static const cudaError_t attr_rc = cudaFuncSetAttribute(gemm_wgrad_video_strided_tcgen05_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-      MERV_REQUIRE(attr_rc == cudaSuccess, MERV_E_CUDA, "cudaFuncSetAttribute(max dynamic smem=%d) failed: %s", smem, cudaGetErrorString(attr_rc));
-      cfg.dynamicSmemBytes = smem;
-      MERV_CUDA_OK(cudaLaunchKernelEx(&cfg, gemm_wgrad_video_strided_tcgen05_kernel<2>, maps, p));
-    } else {
-      constexpr int smem = Cfg<1, false>::SMEM_BYTES;
-      static const cudaError_t attr_rc = cudaFuncSetAttribute(gemm_wgrad_video_strided_tcgen05_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-      MERV_REQUIRE(attr_rc == cudaSuccess, MERV_E_CUDA, "cudaFuncSetAttribute(max dynamic smem=%d) failed: %s", smem, cudaGetErrorString(attr_rc));
-      cfg.dynamicSmemBytes = smem;
-      MERV_CUDA_OK(cudaLaunchKernelEx(&cfg, gemm_wgrad_video_strided_tcgen05_kernel<1>, maps, p));
-    }
-    MERV_CUDA_OK(cudaGetLastError());
-    return MERV_OK;
-  }
   if (vid != nullptr) {
-    if (ctas == 2) {
-      constexpr int smem = Cfg<2, false>::SMEM_BYTES;
-      static const cudaError_t attr_rc = cudaFuncSetAttribute(gemm_wgrad_video_tcgen05_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-      MERV_REQUIRE(attr_rc == cudaSuccess, MERV_E_CUDA, "cudaFuncSetAttribute(max dynamic smem=%d) failed: %s", smem, cudaGetErrorString(attr_rc));
-      cfg.dynamicSmemBytes = smem;
-      MERV_CUDA_OK(cudaLaunchKernelEx(&cfg, gemm_wgrad_video_tcgen05_kernel<2>, maps, p));
-    } else {
-      constexpr int smem = Cfg<1, false>::SMEM_BYTES;
-      static const cudaError_t attr_rc = cudaFuncSetAttribute(gemm_wgrad_video_tcgen05_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-      MERV_REQUIRE(attr_rc == cudaSuccess, MERV_E_CUDA, "cudaFuncSetAttribute(max dynamic smem=%d) failed: %s", smem, cudaGetErrorString(attr_rc));
-      cfg.dynamicSmemBytes = smem;
-      MERV_CUDA_OK(cudaLaunchKernelEx(&cfg, gemm_wgrad_video_tcgen05_kernel<1>, maps, p));
-    }
-    MERV_CUDA_OK(cudaGetLastError());
-    return MERV_OK;
-  }
-  if (assist != nullptr) {
-    constexpr int smem = Cfg<2, false, true>::SMEM_BYTES;
-    static const cudaError_t attr_rc = cudaFuncSetAttribute(gemm_pool_assist_tcgen05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    MERV_REQUIRE(attr_rc == cudaSuccess, MERV_E_CUDA, "cudaFuncSetAttribute(max dynamic smem=%d) failed: %s", smem, cudaGetErrorString(attr_rc));
-    cfg.dynamicSmemBytes = smem;
-    MERV_CUDA_OK(cudaLaunchKernelEx(&cfg, gemm_pool_assist_tcgen05_kernel, maps, p, *assist));
-    MERV_CUDA_OK(cudaGetLastError());
-    return MERV_OK;
+    constexpr int smem1 = Cfg<1, false>::SMEM_BYTES, smem2 = Cfg<2, false>::SMEM_BYTES;
+    if (vid->dy_batch_stride != 0)
+      return ctas == 2 ? launch_kernel<gemm_wgrad_video_strided_tcgen05_kernel<2>, smem2>(cfg, maps, p)
+                       : launch_kernel<gemm_wgrad_video_strided_tcgen05_kernel<1>, smem1>(cfg, maps, p);
+    return ctas == 2 ? launch_kernel<gemm_wgrad_video_tcgen05_kernel<2>, smem2>(cfg, maps, p)
+                     : launch_kernel<gemm_wgrad_video_tcgen05_kernel<1>, smem1>(cfg, maps, p);
   }
   if (p.a_mn_mask | p.b_mn_mask) {
     MERV_REQUIRE(act == MERV_ACT_NONE && !wide, MERV_E_ARG, "gemm: MN-major operands are supported without an activation and without extra output destinations");

@@ -5,7 +5,6 @@
 // All reductions use a fixed order (no float atomics) so results are bit-reproducible per video, independent
 // of batch size and of how the batch is sharded across GPUs.
 #include "common.cuh"
-#include "pool_assist.cuh"
 
 namespace merv {
 
@@ -226,7 +225,16 @@ __global__ void __launch_bounds__(256) partial_score_kernel(const __grid_constan
   if (threadIdx.x == 0) scores[(long long)b * E + e] = acc / float(T) + (p.c[e] ? *p.c[e] : 0.f);
 }
 
-// ---- softmax over the E encoders with warp shuffles: warp_softmax_over_encoders (pool_assist.cuh, shared with the in-GEMM pooling) ----
+// ---- softmax over the E encoders with warp shuffles ----
+// lane e (< E) passes its score; every lane gets the weight of lane e back in the same lane
+__device__ __forceinline__ float warp_softmax_over_encoders(float score, int lane, int E) {
+  const float s = lane < E ? score : -INFINITY;
+  const float m = warp_max(s);
+  const float ex = lane < E ? expf(s - m) : 0.f;
+  const float den = warp_sum(ex);
+  return ex / den;
+}
+
 struct BiasParams {
   const void* bias[MERV_MAX_ENCODERS];
 };
@@ -261,16 +269,12 @@ template <typename T>
 __global__ void __launch_bounds__(256) scores_softmax_kernel(const __grid_constant__ PartialParams pp, const __grid_constant__ BiasParams bp,
                                                              float* __restrict__ scores, float* __restrict__ weights,
                                                              __nv_bfloat16* __restrict__ weights_bf16, float* __restrict__ bias_mix, int E,
-                                                             int Ttok, int N, int* __restrict__ sync_ws, int sync_ints) {
+                                                             int Ttok, int N) {
   __shared__ float red[32];
   __shared__ float sc[MERV_MAX_ENCODERS];
   const int b = blockIdx.y, lane = threadIdx.x & 31;
   pdl_launch_dependents();  // the GEMM behind this kernel may start its prologue now
   pdl_wait();               // the pool kernel's score partials are complete and visible
-  // pool assist: the work counter, completion counters and ready flags of the GEMM behind this kernel start from zero (the GEMM's
-  // griddepcontrol.wait orders these stores before its first read; the previous call's GEMM completed before the pool kernel started)
-  if (sync_ws != nullptr && blockIdx.x == 0 && blockIdx.y == 0)
-    for (int i = threadIdx.x; i < sync_ints; i += 256) sync_ws[i] = 0;
   for (int e = 0; e < E; ++e) {
     const int n = pp.count[e];
     const float* src = pp.p[e] + (long long)b * n;
@@ -606,7 +610,7 @@ extern "C" int merv_softmax_mix(const void* const* V, const int32_t* tokens, con
 namespace merv {
 int launch_scores_softmax_weights(const float* const* partial, const int32_t* count, const float* const* c, const void* const* bias,
                                   float* scores, float* weights, void* weights_bf16, float* bias_mix, int B, int E, int T, int N,
-                                  cudaStream_t stream, bool pdl, int* sync_ws, int sync_ints) {
+                                  cudaStream_t stream, bool pdl) {
   MERV_REQUIRE(partial && count && bias && scores && weights && bias_mix, MERV_E_ARG, "merv_scores_softmax_weights: NULL pointer");
   MERV_REQUIRE(E >= 1 && E <= MERV_MAX_ENCODERS, MERV_E_ARG, "merv_scores_softmax_weights: E=%d", E);
   MERV_REQUIRE(B >= 0 && T > 0 && N > 0, MERV_E_SHAPE, "merv_scores_softmax_weights: B=%d T=%d N=%d", B, T, N);
@@ -631,7 +635,7 @@ int launch_scores_softmax_weights(const float* const* partial, const int32_t* co
   cfg.attrs = attr;
   cfg.numAttrs = pdl ? 1 : 0;
   MERV_CUDA_OK(cudaLaunchKernelEx(&cfg, scores_softmax_kernel<__nv_bfloat16>, pp, bp, scores, weights, static_cast<__nv_bfloat16*>(weights_bf16),
-                                  bias_mix, E, T, N, sync_ws, sync_ints));
+                                  bias_mix, E, T, N));
   MERV_CUDA_OK(cudaGetLastError());
   return MERV_OK;
 }

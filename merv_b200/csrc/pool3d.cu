@@ -29,7 +29,7 @@
 #include <cstring>
 
 #include "common.cuh"
-#include "pool_assist.cuh"
+#include "tcgen05_util.cuh"
 #include "tmap.cuh"
 
 namespace merv {
@@ -156,6 +156,29 @@ __device__ __forceinline__ int pt_find_encoder(const PoolTmaParams& p, int item)
 #pragma unroll 1
   while (e + 1 < p.n_enc && item >= p.enc[e + 1].item_begin) ++e;
   return e;
+}
+
+template <int N_IN, int N_OUT>
+struct PoolWin {  // adaptive pooling window k of an axis N_IN -> N_OUT: [floor(k N_IN / N_OUT), ceil((k + 1) N_IN / N_OUT))
+  __host__ __device__ static constexpr int lo(int i) { return (i * N_IN) / N_OUT; }
+  __host__ __device__ static constexpr int hi(int i) { return ((i + 1) * N_IN + N_OUT - 1) / N_OUT; }
+};
+
+__device__ __forceinline__ uint4 lds_v4(uint32_t addr) {
+  uint4 r;
+  asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "r"(addr));
+  return r;
+}
+// predicated 128-bit shared load: zeros when !ok, no branch
+__device__ __forceinline__ uint4 lds_v4_if(uint32_t addr, bool ok) {
+  uint4 r;
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.u32 p, %5, 0;\n\t"
+      "mov.u32 %0, 0;\n\tmov.u32 %1, 0;\n\tmov.u32 %2, 0;\n\tmov.u32 %3, 0;\n\t"
+      "@p ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];\n\t}"
+      : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "r"(addr), "r"(uint32_t(ok)));
+  return r;
 }
 
 // ---- specialised consumer for the square grids of the shipped encoders (16 x 16 and 14 x 14 patches -> 8 x 8), 128-byte rows ----
@@ -667,63 +690,6 @@ static int launch_direct(const merv_pool_desc* enc, int n, int B, int dtype, cud
     pool3d_direct_kernel<float><<<grid, threads, 0, s>>>(p);
   MERV_CUDA_OK(cudaGetLastError());
   return MERV_OK;
-}
-
-// ---- pool assist (pool_assist.cuh): argument block of the in-GEMM pooling for merv_fused_forward ----
-bool build_pool_assist(const merv_fused_desc* d, int head, AssistArgs* args, int* rc) {
-  *rc = MERV_OK;
-  const int E = d->num_encoders;
-  if (E < 1 || E > MERV_MAX_SEGMENTS || d->sync_ws == nullptr || head < 1 || head >= d->B) return false;
-  if (d->sync_ws_ints < ASSIST_SYNC_HEADER + 2 * d->B) return false;
-  if (!use_tma(d->pool, E, MERV_BF16)) return false;
-  AssistArgs a;
-  memset(&a, 0, sizeof(a));
-  int begin = 0;
-  for (int e = 0; e < E; ++e) {
-    const merv_pool_desc& p = d->pool[e];
-    const TmaPlan pl = plan_tma(p, MERV_BF16);
-    // the shipped encoders: square 16 x 16 / 14 x 14 patch grids pooled to 8 x 8, one input frame per output frame, 128-byte channel chunks
-    if (p.shift_f != 0 || p.shift_h != 0 || p.shift_w != 0) return false;
-    if (!(pl.ok && pl.vpr == 8 && pl.nf_max == 1 && p.F == p.T && p.S == ASSIST_S && p.H == p.W && (p.H == 16 || p.H == 14) && pl.nchunks <= 511 &&
-          p.T < (1 << 18)))
-      return false;
-    AssistEnc& en = a.enc[e];
-    en.y = static_cast<__nv_bfloat16*>(p.y); en.score_vec = p.score_vec; en.score_partial = p.score_partial; en.batch_index = p.batch_index;
-    en.c = d->c[e]; en.bias = static_cast<const __nv_bfloat16*>(d->bias[e]);
-    en.ybs = p.y_batch_stride; en.yrs = p.y_row_stride;
-    en.H = p.H; en.C = p.C; en.T = p.T; en.nchunks = pl.nchunks;
-    en.item_begin = begin;
-    en.parts = p.T * pl.nchunks * PT_GROUP_WARPS;
-    if (en.parts != d->parts[e]) return false;  // the caller sized the partials for another kernel plan
-    begin += p.T * pl.nchunks * 2;
-    const unsigned long long dims[5] = {(unsigned long long)p.C, (unsigned long long)p.W, (unsigned long long)p.H, (unsigned long long)p.F,
-                                        (unsigned long long)(p.batch_index && p.src_batch > 0 ? p.src_batch : d->B)};
-    const unsigned long long strides[4] = {(unsigned long long)p.x_token_stride * 2, (unsigned long long)p.x_token_stride * p.W * 2,
-                                           (unsigned long long)p.x_frame_stride * 2, (unsigned long long)p.x_batch_stride * 2};
-    const unsigned box[5] = {ASSIST_CB, (unsigned)p.W, ASSIST_ROWS, 1, 1};
-    if ((*rc = encode_tmap_cached(&a.m[e], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, p.x, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE)) != MERV_OK) return false;
-  }
-  for (int e = E; e < MERV_MAX_SEGMENTS; ++e) a.m[e] = a.m[0];
-  const long long total = (long long)begin * (d->B - head);
-  if (total > 0x7fffffffLL - 4096) return false;
-  a.n_enc = E; a.head = head; a.B = d->B; a.items_per_video = begin; a.total_items = int(total); a.N = d->N; a.rows_per_video = d->rows_per_video;
-  // items per fetch: amortises the release fence + completion atomic; must divide a video's item count (always even: two halves)
-  a.group = 2;
-  for (int g = 8; g > 2; g >>= 1)
-    if (begin % g == 0) { a.group = g; break; }
-  if (const char* e = getenv("MERV_ASSIST_GROUP")) {
-    const int g = atoi(e);
-    if (g >= 1 && begin % g == 0) a.group = g;
-  }
-  a.prof = nullptr;
-  a.dbg = 0;
-  if (const char* e = getenv("MERV_ASSIST_DBG")) a.dbg = atoi(e);
-  if (const char* e = getenv("MERV_ASSIST_PROFILE"))
-    if (e[0] == '1' && d->sync_ws_ints >= ASSIST_SYNC_HEADER + 2 * d->B + 8 * ASSIST_WARPS * sm_count()) a.prof = d->sync_ws + ASSIST_SYNC_HEADER + 2 * d->B;
-  a.sync = d->sync_ws; a.scores = d->scores; a.weights = d->weights; a.weights_bf16 = static_cast<__nv_bfloat16*>(d->weights_bf16);
-  a.bias_mix = d->bias_mix;
-  *args = a;
-  return true;
 }
 
 }  // namespace merv

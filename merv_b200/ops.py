@@ -578,9 +578,6 @@ class FusedLinearPlan:
             self.weights = torch.empty((B, E), dtype=torch.float32, device=dev)
             self.bias_mix = torch.empty((B, N), dtype=torch.float32, device=dev)
             d.scores, d.weights, d.bias_mix = self.scores.data_ptr(), self.weights.data_ptr(), self.bias_mix.data_ptr()
-            # counters / ready flags of the in-GEMM pooling (merv_fusion.h: pool assist); the library decides per call whether it runs
-            self.sync_ws = torch.zeros(4 + 2 * B + 8 * 2 * 160, dtype=torch.int32, device=dev)  # + per-warp profile slots (MERV_ASSIST_PROFILE=1)
-            d.sync_ws, d.sync_ws_ints, d.assist_head = self.sync_ws.data_ptr(), self.sync_ws.numel(), 0
         self.N, self.T_tok = N, T_tok
         self.x_meta = [(tuple(x.shape), tuple(x.stride())) for x in xs]
         self.fn = lib.merv_fused_forward

@@ -7,7 +7,4 @@ echo "rc=$?"
 echo "=== full capture: per-video weight gradient (64 videos, C = 1024) ==="
 TRAIN_STEP_ONLY=fused_training timeout 900 ncu --set full --clock-control none --import-source on -k regex:gemm_wgrad_video -s 8 -c 1 -f -o gpurun_out/r2b_prof_wgrad_video python scripts/gpu_train_step.py 64 > gpurun_out/r2b_prof_wgrad_video.log 2>&1
 echo "rc=$?"
-echo "=== full capture: GEMM with pool assist (64 videos, head 32) ==="
-MERV_POOL_ASSIST=1 MERV_ASSIST_HEAD=32 timeout 900 ncu --set full --clock-control none --import-source on -k regex:gemm_pool_assist -s 3 -c 1 -f -o gpurun_out/r2b_prof_pool_assist python bench.py --steps 3 --warmup 3 --no-e2e --no-cpu-baseline --no-configs --no-torch-eager --no-sustained > gpurun_out/r2b_prof_pool_assist.log 2>&1
-echo "rc=$?"
 ls -la gpurun_out/*.ncu-rep

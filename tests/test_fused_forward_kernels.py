@@ -570,7 +570,6 @@ def test_fused_forward_matches_its_three_launches(name, pdl, monkeypatch):
     from merv_b200 import ops
 
     monkeypatch.setenv("MERV_PDL", pdl)
-    monkeypatch.delenv("MERV_POOL_ASSIST", raising=False)
     for var in ("MERV_GEMM_CTA_GROUP", "MERV_GEMM_WIDE_OUT"):
         monkeypatch.delenv(var, raising=False)
     B, T, S, N, xs, vs, cs, Ws, biases = _fwd_inputs(name)

@@ -1117,35 +1117,6 @@ def test_attentive_pooler_training_matches_reference_autograd(C_, llm, n, heads,
     assert O.rel_err(_np(out_inf), _np(out)) < 1e-2
 
 
-@pytest.mark.parametrize("B,head", [(48, None), (24, 1), (24, 23)])  # None: the library's default head (40 videos)
-def test_pool_assist_is_bit_identical_to_the_three_launch_path(B, head, monkeypatch):
-    """Pool assist (merv_b200/csrc/pool_assist.cuh, opt-in with MERV_POOL_ASSIST=1): the GEMM's spare warps pool, score and soft-max the
-    videos behind the head inside the GEMM launch, handing them to the tensor cores through per-video release / acquire flags.  Same
-    arithmetic and summation order as the standalone kernels -> prefix and weights must be BIT-identical, on the plain call, on re-runs
-    of the cached plan (the flags are reset by the scores kernel), with the gather by multimodal_indices and with the prefix written
-    into a strided slot of the embedding buffer."""
-    m = _full_module(True)
-    feats = _full_features(B)
-    idx = torch.tensor([3, 0, 7, 23, 11, 5, 19, 2, 14, 9, 21, 1, 16, 8, 22, 4, 13, 6], dtype=torch.int32, device=DEV)
-    emb = torch.zeros((B, 1 + 1024 + 7, 4096), dtype=torch.bfloat16, device=DEV)
-    with torch.inference_mode():
-        monkeypatch.setenv("MERV_POOL_ASSIST", "0")
-        want, want_w = m(feats)
-        want_g, want_gw = m(feats, batch_index=idx)
-        torch.cuda.synchronize()
-        monkeypatch.setenv("MERV_POOL_ASSIST", "1")
-        if head is not None:
-            monkeypatch.setenv("MERV_ASSIST_HEAD", str(head))
-        for _ in range(3):
-            out, w = m(feats)
-            assert torch.equal(out, want) and torch.equal(w, want_w)
-        out_g, w_g = m(feats, batch_index=idx)
-        assert torch.equal(out_g, want_g) and torch.equal(w_g, want_gw)
-        m(feats, out=emb[:, 1:1025])
-        torch.cuda.synchronize()
-        assert torch.equal(emb[:, 1:1025], want) and not emb[:, 0].any() and not emb[:, 1025:].any()
-
-
 @pytest.mark.parametrize("F,H,T,S,Cc", [(5, 7, 2, 3, 24), (2, 16, 2, 8, 128), (3, 14, 3, 8, 64), (4, 6, 2, 2, 8)])
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
 @pytest.mark.parametrize("impl", ["tma", "direct"])
